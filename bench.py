@@ -8,7 +8,8 @@ quadrotor OCPs, n_grid 50).
 
 One "step" = one CPDP gradient iteration for every OCP of the batch: forward solve from the zero seed, auxiliary
 system (backward Riccati + forward sweep), loss and dL/dtheta, and the fixed-order cross-problem reduction.
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  The inputs are seeded, so with the same arguments every run solves the same problems;
+--dump-outputs DIR saves what the last timed step returned (see dump_outputs) to compare two builds output for output.
 """
 import argparse
 import json
@@ -46,7 +47,12 @@ def parse():
     ap.add_argument("--cpu-sample", type=int, default=0, help="problems in the CPU baseline sample (0 = one per core)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-deadline", type=float, default=200.0, help="stop starting new CPU-baseline steps after this many seconds")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float64), to compare two builds output for output")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return a
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -216,6 +222,32 @@ def flop_model(info, n, m, r, N, S, iters_sum, B, cnt, mode):
     return dict(solve=float(solve), aux_backward=float(back), aux_forward=float(fwdf), total=float(solve + back + fwdf))
 
 
+DUMP_BYTES = 32 << 20          # what --dump-outputs writes at most
+
+
+def dump_outputs(path, red, sol, aux, first):
+    """Writes what one step returned to its caller as path/<name>.npy, all float64: the reduced row `reduced` [sum loss |
+    sum dL/dtheta | failed OCPs], every OCP's status / iters / kkt / cost / loss / dtheta / aux_status / counters, and the
+    trajectories X, U, Lam, Xa, Ua of a fixed seeded sample of the OCPs, as many as DUMP_BYTES leaves room for; `sample_index`
+    holds the sample's global problem indices (`first` = index of this shard's first OCP)."""
+    import torch
+    B = int(aux["loss"].shape[0])
+    whole = {"reduced": red, **{k: sol[k] for k in ("status", "iters", "kkt", "cost")},
+             **{k: aux[k] for k in ("loss", "dtheta", "aux_status", "counters")}}
+    traj = {**{k: sol[k] for k in ("X", "U", "Lam")}, **{k: aux[k] for k in ("Xa", "Ua")}}
+    per_ocp = 8 * (1 + sum(v[0].numel() for v in traj.values()))
+    k = min(B, (DUMP_BYTES - 8 * sum(v.numel() for v in whole.values())) // per_ocp)
+    assert k > 0, "--dump-outputs: the per-OCP results of %d OCPs alone exceed %d bytes" % (B, DUMP_BYTES)
+    idx = np.sort(np.random.default_rng(0).choice(B, k, replace=False))
+    sel = torch.from_numpy(idx).to(red.device)
+    out = {name: v.cpu().numpy() for name, v in whole.items()}
+    out.update({name: v.index_select(0, sel).cpu().numpy() for name, v in traj.items()})
+    out["sample_index"] = first + idx
+    os.makedirs(path, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(v, dtype=np.float64))
+
+
 def run_ours(a):
     import torch
     import torch.distributed as dist
@@ -307,7 +339,7 @@ def run_ours(a):
     sync_all()
     ms = ev[0].elapsed_time(ev[1])
     clocks = sampler.stop() if rank == 0 else None
-    sol_t, aux_t = sol, aux
+    red_t, sol_t, aux_t = red, sol, aux
     # ---- phase times (single stream, each phase alone; explains `value`, is not part of it) -------------------------
     for _ in range(3):                                    # untimed: allocates the single-stream workspace, warms the caches
         s0 = oc.cocSolverBatch(resident["x0"], 1.0, resident["theta"], pdata=resident["goal"])
@@ -448,6 +480,8 @@ def run_ours(a):
     # a step that averaged failed problems into its gradient is not a valid measurement (fixed Newton rounds that are too few
     # would leave problems `running`; the count travels with the reduced row, see cpdp_pack_rows)
     out["valid"] = (int(loc[1]) == 0 and int(loc[2]) == 0 and out["stats"]["failed_ocps_in_reduced_row"] == 0)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, red_t, sol_t, aux_t, lo)
     if world == 1 and not a.no_cpu_baseline:
         cb, _, _ = cpu_baseline(a.n_grid, a.cpu_sample, deadline_s=a.cpu_deadline)
         out["cpu_baseline"] = cb
