@@ -60,6 +60,10 @@ int cpdp_last_rounds(void);
  *   mode 0: backward Riccati sweep by RK45 with (rtol_b, atol_b)   [what COCSys_TimeVarying does, CPDP.py:740]
  *   mode 1: backward sweep by the BDF scheme of the as-shipped COCSys (CPDP.py:335), scipy defaults in rtol_b/atol_b
  *   forward sweep: RK45 with (rtol_f, atol_f) (CPDP.py:368; scipy defaults 1e-3 / 1e-6).
+ *   mode 2 ("discrete"): no integrator -- Xa, Ua, loss and dtheta are the exact derivative of the discretised problem cpdp_solve
+ *   solves, from the KKT system of the RK4 multiple-shooting NLP differentiated at (X, U, Lam) (a Riccati recursion over the
+ *   stage derivatives; the tolerances are ignored, S must be > 0, counters stay 0).  aux_status 4 here: some Quu block of the
+ *   recursion is not positive definite (the reduced Hessian at the point is not positive definite).
  *   Loss: W waypoints of D observed state components sel[D] (host ints); taus[B][W] (taus_stride = W) or shared
  *   taus[W] (stride 0); wp[B][W][D].  W = 0 skips the loss.
  * Outputs Xa[B][N+1][n*r] (dx/dtheta nodes), Ua[B][N+1][m*r], loss[B], dtheta[B][r] (reference convention:
@@ -76,7 +80,8 @@ int cpdp_aux(void* ws, size_t ws_bytes, int B, int N, int S, double T,
              double* Xa, double* Ua, double* loss, double* dtheta, int* aux_status, int* counters, void* stream);
 
 /* cpdp_aux with the two sweeps selectable: phases 1 = backward Riccati sweep only (node table left in ws),
- * 2 = forward sweep + loss only (needs the table of a previous phase-1 call on the same ws), 3 = both. */
+ * 2 = forward sweep + loss only (needs the table of a previous phase-1 call on the same ws), 3 = both.
+ * Mode 2: phase 1 = stage derivatives + backward recursion (gains left in ws), phase 2 = rollout + loss. */
 int cpdp_aux_phases(void* ws, size_t ws_bytes, int B, int N, int S, double T,
              const double* theta, int theta_stride, const double* pdata,
              const double* X, const double* U, const double* Lam, const int* solve_status,

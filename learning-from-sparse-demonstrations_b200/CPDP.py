@@ -74,6 +74,7 @@ class COCSys:
     # modes of the backward Riccati sweep
     MODE_RK45 = 0     # explicit Dormand-Prince with tolerance knobs (what COCSys_TimeVarying uses, CPDP.py:740)
     MODE_BDF = 1      # scheme of the as-shipped COCSys (CPDP.py:335): scipy-style BDF at default tolerances
+    MODE_DISCRETE = 2  # exact derivative of the discretised problem the solver solves (DESIGN.md §3.7); tolerances unused
 
     def __init__(self, project_name="myOc"):
         self.sys_name = project_name

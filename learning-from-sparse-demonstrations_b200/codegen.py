@@ -15,6 +15,8 @@ Emitted members (n states, m controls, r parameters, nz = n+m):
                                              (the caller zero-fills the buffer once)
   term(x,th, &h, hx[n])                      final cost and gradient                   (CPDP.py:77-79,242)
   term2(x,th, hxx[n*n], hxe[n*r])            CPDP.py:245-248
+  dir_th(x,u,th,mu,w,dx,du,dth, df[n], hz[nz])   df = fx dx + fu du + fth dth ; hz = Hess_z(Ham) [dx;du] + Hess_ztheta(Ham) dth
+                                             (discrete auxiliary mode: theta-sensitivities of the RK4 stages)
 plus static sparsity tables (CSR and CSC) of fx and fu used by the Riccati / auxiliary right-hand sides.
 """
 import hashlib
@@ -160,6 +162,19 @@ def generate_model_header(name, state, control, auxvar, dyn, path_cost, final_co
                  "const double* __restrict__ dx, const double* __restrict__ du, "
                  "double* __restrict__ df, double* __restrict__ hz) {\n%s\n    }" % body)
 
+    # the same directional derivatives with a parameter tangent dth (forward theta-sensitivities of the RK4 stages and the
+    # mixed z-theta Hessian of the interval Lagrangian, used by the discrete auxiliary mode)
+    dths = [sp.Symbol("dth[%d]" % i, real=True) for i in range(r)]
+    dth = sp.Matrix(dths)
+    df_th = fz * dz + f.jacobian(ts) * dth
+    hz_th = Hzz * dz + Hz.T.jacobian(ts) * dth
+    body, info["ops_dir_th"] = _emit_body([("df[%d]" % i, df_th[i]) for i in range(n)] +
+                                          [("hz[%d]" % i, hz_th[i]) for i in range(nz)])
+    part_dir_th = ("    CPDP_HD static void dir_th(const double* __restrict__ x, const double* __restrict__ u, "
+                   "const double* __restrict__ th, const double* __restrict__ pd, const double* __restrict__ mu, const double w, "
+                   "const double* __restrict__ dx, const double* __restrict__ du, const double* __restrict__ dth, "
+                   "double* __restrict__ df, double* __restrict__ hz) {\n%s\n    }" % body)
+
     # PMP set, H = c + lam' f  (lam takes the role of mu, w = 1)
     Hp = c + sum(mus[i] * f[i] for i in range(n))
     Hx = sp.Matrix([Hp]).jacobian(xs)
@@ -218,6 +233,7 @@ def generate_model_header(name, state, control, auxvar, dyn, path_cost, final_co
                                          [("hxe[%d]" % (i * r + j), hxe[i, j]) for i in range(n) for j in range(r)])
     parts.append("    CPDP_HD static void term2(const double* __restrict__ x, const double* __restrict__ th, const double* __restrict__ pd, "
                  "double* __restrict__ hxx, double* __restrict__ hxe) {\n%s\n    }" % body)
+    parts.append(part_dir_th)
 
     tables = "\n".join([_sparse_tables("FX", mats[0][1]), _sparse_tables("FU", mats[1][1]),
                         _sparse_tables("FE", mats[2][1])])

@@ -10,6 +10,7 @@
 #include "cpdp_aux.cuh"
 #include "cpdp_bdf.cuh"
 #include "cpdp_fwd.cuh"
+#include "cpdp_disc.cuh"
 #include "cpdp_optim.cuh"
 
 // The only host-side state of the library: the first launch error of the call in progress.  Thread-local, cleared by every
