@@ -55,6 +55,12 @@ constexpr int BDF_WS_DOUBLES = BDF_NROWS * NX * NC;      // differences array of
 #ifndef CPDP_BDF_STENCIL_UNROLL
 #define CPDP_BDF_STENCIL_UNROLL 1
 #endif
+// Newton solves in the eigenbasis of L (bdf_eig_basis): taken for a Jacobian whose real eigenvector basis V has
+// ||V||_F ||V^{-1}||_F <= CPDP_BDF_EIG_KAPPA; 0 compiles the eigen path out (every solve runs the Bartels-Stewart sweep).
+#ifndef CPDP_BDF_EIG_KAPPA
+#define CPDP_BDF_EIG_KAPPA 1e4
+#endif
+constexpr double BDF_EIG_KAPPA = CPDP_BDF_EIG_KAPPA;
 #ifdef __CUDACC__
 #define BDF_SYNC() __syncwarp()
 #define BDF_UNROLL _Pragma("unroll")
@@ -106,7 +112,7 @@ constexpr int GHM = XB + NX * NCS;               // fu Huu^{-1}, [NX][NU]
 constexpr int YPM = GHM + NX * NU;               // Huu^{-1} Y, [NU][NX]
 constexpr int ROT = YPM + NU * NX;               // block rotations G: ga | gbr | gbi | partner   (4 x NX)
 constexpr int RU = (ROT + 4 * NX + 1) & ~1;                 // change_D: RU | R | U, 6 x 6 each (also Householder vector scratch, sweep store dump: 128)
-constexpr int FLAG = RU + 128;                   // 3 ints: prepare ok | Schur ok | first node row held in NODE
+constexpr int FLAG = RU + 128;                   // 4 ints: prepare ok | Schur ok | first node row held in NODE | eigen path
 constexpr int NODE = FLAG + 2;                   // the two node rows (x, u, lambda) bracketing the current grid interval
 constexpr int NODE_W = 2 * NX + NU;
 #ifdef CPDP_BDF_TIMING
@@ -116,6 +122,9 @@ constexpr int END = TS + 8;
 constexpr int END = NODE + ((2 * NODE_W + 1) & ~1);
 #endif
 static_assert(Y2 % 2 == 0 && T2S % 2 == 0 && TD % 2 == 0 && PV % 2 == 0 && RU % 2 == 0, "complex arrays are read with 128-bit loads");
+// eigen path (flag 3): Y2 holds V | Im x while the basis is built, then the coefficients k3 | k4 of the block solve; T2S holds
+// V^{-1} while the basis is built, then the block solution Z (row stride QS); PV the coefficients k1 | k2; TD (a, b) per index
+static_assert(2 * NX * NX <= T2S - Y2 && NX * NX <= 2 * NX * TW && NX * QS <= 2 * NX * TW, "eigen path scratch");
 }  // namespace bo
 constexpr int BDF_SMEM_DOUBLES = bo::END;
 constexpr size_t BDF_SMEM_BYTES = (size_t)BDF_SMEM_DOUBLES * sizeof(double);
@@ -175,6 +184,16 @@ CPDP_D double bdf_rcp(double x) {
 #define BDF_TP_ARG
 #define BDF_TS0()
 #define BDF_TS(i)
+#endif
+// Developer path counts (-DCPDP_BDF_PATH_COUNTS, implied by the timing build): Newton solves on the eigen path | on the
+// sweep, Jacobians on the eigen path | on the sweep, written over Ua[24..27] of the problem at kernel end.
+#ifdef CPDP_BDF_TIMING
+#define CPDP_BDF_PATH_COUNTS
+#endif
+#ifdef CPDP_BDF_PATH_COUNTS
+#define BDF_PATH(sm, k) do { cnt[4 + (k) + ((BDF_EIG_KAPPA > 0.0 && ((const int*)((sm) + bo::FLAG))[3]) ? 0 : 1)] += 1; } while (0)
+#else
+#define BDF_PATH(sm, k) do { } while (0)
 #endif
 
 // THE product of the hot loop, one out-of-line instance:  dst[(i0 + i) * ds] = sum_k AT[k][i0 + i] x[k * xs],  i < NH.
@@ -614,6 +633,120 @@ CPDP_D bool schur_real_w0(double* sm, double* H, double* Z, double* vb) {
     return true;
 }
 
+// Real eigenvector basis of the quasi-triangular T of L = Q T Q' (row stride NX):  T = V D V^{-1}, D block diagonal with
+// 1 x 1 blocks [lambda] and 2 x 2 blocks [[a, b], [-b, a]] on the columns [Re x, Im x] of the eigenvector x of a + ib (b > 0);
+// a 2 x 2 block of T with real eigenvalues gives two 1 x 1 blocks.  V is block upper triangular on T's blocks, so V (complex
+// back-substitution per eigenvalue, columns normalised) and V^{-1} (real back-substitution) take one column per lane, as
+// LAPACK's dtrevc does.  Nothing is perturbed: a defective or nearly defective T shows as a non-finite or large
+// ||V||_F ||V^{-1}||_F, and then nothing the sweep path reads is touched and the result is false (uniformly).  Otherwise
+// G = Q V and H = V^{-1} Q' replace Q and Q' in the product slots (k-major H' in Q, G' in QT), TD holds (a, b) per index
+// (b = 0 for a real eigenvalue) and ROT's partner row the other index of each complex pair.  The Q / QT slots hold Q on entry.
+CPDP_D bool bdf_eig_basis(double* sm, const double* T) {
+    constexpr int n = NX;
+    const int lane = threadIdx.x;
+    const bool own = lane < n;
+    const int j = own ? lane : 0;
+    double* Vr = sm + bo::Y2; double* Vi = Vr + n * n; double* W = sm + bo::T2S;        // row stride n
+    const bool up = j + 1 < n && T[(j + 1) * n + j] != 0.0, dn = j >= 1 && T[j * n + j - 1] != 0.0;
+    const int bs = dn ? j - 1 : j, be = up ? j + 1 : j;                // my block of T
+    double lr = T[j * n + j], li = 0.0;                                // my eigenvalue lr + i li
+    double x0r = 1.0, x0i = 0.0, x1r = 0.0;                            // x on rows bs, be (x1 is real)
+    bool cpx = false;
+    if (bs != be) {
+        const double p = T[bs * n + bs], q = T[bs * n + be], r = T[be * n + bs], s = T[be * n + be];
+        const double hd = 0.5 * (p - s), disc = hd * hd + q * r;
+        if (disc < 0.0) { cpx = true; li = sqrt(-disc); lr = s + hd; x0r = hd; x0i = li; x1r = r; }      // (lambda - s, r)
+        else {
+            const double sq = (hd >= 0.0) ? sqrt(disc) : -sqrt(disc);
+            if (j == bs) { lr = s + (hd + sq); x0r = hd + sq; x1r = r; }                                 // (lambda - s, r)
+            else { lr = p - (hd + sq); x0r = q; x1r = -(hd + sq); }                                        // (q, lambda - p)
+        }
+    }
+    if (own) {
+        CPDP_LOOP for (int i = 0; i < n; ++i) { Vr[i * n + j] = 0.0; Vi[i * n + j] = 0.0; }
+        Vr[bs * n + j] = x0r; Vi[bs * n + j] = x0i;
+        if (be != bs) Vr[be * n + j] = x1r;
+    }
+    // rows above my block, row blocks of T bottom-up: (T_II - lambda) x_I = -sum_{m > I} T_Im x_m
+    for (int i = n - 1; i >= 0;) {
+        const bool two = i >= 1 && T[i * n + i - 1] != 0.0;
+        const int i0 = two ? i - 1 : i;
+        if (own && i < bs) {
+            double ar = 0.0, ai = 0.0, br = 0.0, bi = 0.0;
+            CPDP_LOOP for (int m = i + 1; m < n; ++m) {
+                const double xr = Vr[m * n + j], xi = Vi[m * n + j], ta = T[i0 * n + m], tb = T[i * n + m];
+                ar -= ta * xr; ai -= ta * xi; br -= tb * xr; bi -= tb * xi;
+            }
+            const double dr = T[i0 * n + i0] - lr, di = -li;
+            double yr, yi;
+            if (two) {                                                 // 2 x 2 complex system by Cramer's rule
+                const double er = T[i * n + i] - lr, t01 = T[i0 * n + i], t10 = T[i * n + i0];
+                const double gr = (dr * er - di * di) - t01 * t10, gi = dr * di + di * er;          // det
+                const double ig = 1.0 / (gr * gr + gi * gi);
+                const double ur = (ar * er - ai * di) - t01 * br, ui = (ar * di + ai * er) - t01 * bi;
+                const double wr = (dr * br - di * bi) - t10 * ar, wi = (dr * bi + di * br) - t10 * ai;
+                Vr[i0 * n + j] = (ur * gr + ui * gi) * ig; Vi[i0 * n + j] = (ui * gr - ur * gi) * ig;
+                yr = (wr * gr + wi * gi) * ig; yi = (wi * gr - wr * gi) * ig;
+            } else {
+                const double ig = 1.0 / (dr * dr + di * di);
+                yr = (ar * dr + ai * di) * ig; yi = (ai * dr - ar * di) * ig;
+            }
+            Vr[i * n + j] = yr; Vi[i * n + j] = yi;
+        }
+        i = i0 - 1;
+    }
+    if (own) {                                                         // column j of V: Re x, or Im x for the second of a pair
+        double s2 = 0.0;
+        CPDP_LOOP for (int m = 0; m < n; ++m) s2 += Vr[m * n + j] * Vr[m * n + j] + Vi[m * n + j] * Vi[m * n + j];
+        const double sc = 1.0 / sqrt(s2);
+        const double* src = (cpx && j == be) ? Vi : Vr;
+        CPDP_LOOP for (int m = 0; m < n; ++m) Vr[m * n + j] = src[m * n + j] * sc;
+    }
+    BDF_SYNC();
+    // column j of V^{-1}: V w = e_j, row blocks bottom-up
+    for (int i = n - 1; i >= 0;) {
+        const bool two = i >= 1 && T[i * n + i - 1] != 0.0;
+        const int i0 = two ? i - 1 : i;
+        if (own) {
+            double a = (i0 == j) ? 1.0 : 0.0, b = (i == j) ? 1.0 : 0.0;
+            CPDP_LOOP for (int m = i + 1; m < n; ++m) { const double w = W[m * n + j]; a -= Vr[i0 * n + m] * w; b -= Vr[i * n + m] * w; }
+            if (two) {
+                const double v00 = Vr[i0 * n + i0], v01 = Vr[i0 * n + i], v10 = Vr[i * n + i0], v11 = Vr[i * n + i];
+                const double ig = 1.0 / (v00 * v11 - v01 * v10);
+                W[i0 * n + j] = (a * v11 - v01 * b) * ig;
+                W[i * n + j] = (v00 * b - v10 * a) * ig;
+            } else {
+                W[i * n + j] = a / Vr[i * n + i];
+            }
+        }
+        i = i0 - 1;
+    }
+    double nv = 0.0, nw = 0.0;
+    if (own) { CPDP_LOOP for (int m = 0; m < n; ++m) { nv += Vr[m * n + j] * Vr[m * n + j]; nw += W[m * n + j] * W[m * n + j]; } }
+    nv = bdf_reduce(nv, false);
+    nw = bdf_reduce(nw, false);
+    if (!(nv * nw <= BDF_EIG_KAPPA * BDF_EIG_KAPPA)) return false;     // (NaN / inf fail the test too)
+    // G = Q V -> XA[i][c];  H' = Q (V^{-1})' -> XB[k][i] = H[i][k]
+    double* XA = sm + bo::XA; double* XB = sm + bo::XB;
+    int hc, hi0;
+    if (bdf_half(lane, hc, hi0)) {
+        bdf_lmul_to(sm + bo::QT, QS, Vr + hc, n, XA + hc, NCS, hi0);
+        bdf_lmul_to(sm + bo::QT, QS, W + hc * n, 1, XB + hc, NCS, hi0);
+    }
+    BDF_SYNC();
+    CPDP_LOOP for (int e = lane; e < n * n; e += BDF_THREADS) {
+        const int k = e / n, i = e % n;
+        sm[bo::Q + k * QS + i] = XB[k * NCS + i];
+        sm[bo::QT + k * QS + i] = XA[i * NCS + k];
+    }
+    if (own) {
+        BDF_ST2(sm + bo::TD + 2 * j, lr, li);
+        sm[bo::ROT + 3 * n + j] = (double)(cpx ? (j == bs ? be : bs) : j);
+    }
+    BDF_SYNC();
+    return true;
+}
+
 // Complex Schur form L = Z T Z^H of the matrix in TR; result: T in (TR, TI), the real Schur vectors Q (and Q'), the block
 // rotations G (Z = Q G^H) as per-row coefficients.  Returns false (uniformly) if the QR iteration did not converge.
 CPDP_D_NOINLINE bool bdf_schur() {
@@ -630,8 +763,24 @@ CPDP_D_NOINLINE bool bdf_schur() {
     BDF_SYNC();
     const bool ok = schur_real_w0(sm, Tr, Zm, sm + bo::RU);
     BDF_SYNC();
-    BDF_TS0();
     if (!ok && lane == 0) flag[1] = 0;
+    // k-major product operands Q[k][i] (for Q' x) and QT[k][i] = Q[i][k] (for Q x)
+    CPDP_LOOP for (int e = lane; e < n * n; e += BDF_THREADS) {
+        const int r_ = e / n, c_ = e % n;
+        const double v = Zm[e];
+        sm[bo::Q + r_ * QS + c_] = v;
+        sm[bo::QT + c_ * QS + r_] = v;
+    }
+    BDF_SYNC();
+    if (BDF_EIG_KAPPA > 0.0) {
+        BDF_TS0();
+        const bool eig = ok && bdf_eig_basis(sm, Tr);
+        if (lane == 0) flag[3] = eig ? 1 : 0;
+        BDF_SYNC();
+        BDF_TS(5);
+        if (eig) return true;
+    }
+    BDF_TS0();
     // ---- one unitary rotation per 2 x 2 block:  G = [[c, s], [-conj(s), c]],  T <- G T G^H.  The Schur vectors stay REAL;
     //      the block-diagonal unitary factor is kept as per-index coefficients (Z = Q G^H):
     //      G[i][i] = ga[i] (real), G[i][pi[i]] = gb[i] (complex), pi[i] = the other index of i's block (or i).
@@ -677,13 +826,7 @@ CPDP_D_NOINLINE bool bdf_schur() {
     }
     BDF_SYNC();
     BDF_TS(3);
-    // k-major product operands Q[k][i] (for Q' x) and QT[k][i] = Q[i][k] (for Q x); T packed for the sweep
-    CPDP_LOOP for (int e = lane; e < n * n; e += BDF_THREADS) {
-        const int r_ = e / n, c_ = e % n;
-        const double v = Zm[e];
-        sm[bo::Q + r_ * QS + c_] = v;
-        sm[bo::QT + c_ * QS + r_] = v;
-    }
+    // T packed for the sweep
     CPDP_LOOP for (int e = lane; e < n * TW; e += BDF_THREADS) {
         const int r_ = e / TW, k = r_ + 1 + e % TW;
         BDF_ST2(sm + bo::T2S + 2 * e, k < n ? Tr[r_ * n + k] : 0.0, k < n ? Ti[r_ * n + k] : 0.0);
@@ -721,6 +864,54 @@ CPDP_D double bdf_stencil_GhYG(const double* rot, const double* Y, const int i, 
     return tjr * bj_r + (hj ? (tpr * bp_r - tpi * bp_i) : 0.0);
 }
 
+// scipy's "LU" event on the eigen path.  In the eigenbasis the Lyapunov operator Z + c (D Z + Z D') splits into the blocks of
+// D: for the index blocks I, J with eigenvalues a_I + i b_I (b = 0 for a real one) the parts of Z_IJ that commute and
+// anticommute with the rotation generator are scaled by  w+ = 1 / (1 + c (l_I + conj l_J))  and  w- = 1 / (1 + c conj(l_I + l_J)),
+// which gives every entry as  Z_ij = k1 B_ij + k2 B_pi,j + k3 B_i,pj + k4 B_pi,pj  (p: partner index, s = +1 / -1 for the
+// first / second index of a pair, 0 for a real eigenvalue):
+//   k1 = Re(w+ + w-) / 2,  k2 = s_i Im(w+ - w-) / 2,  k3 = -s_j Im(w+ + w-) / 2,  k4 = s_i s_j Re(w+ - w-) / 2.
+// (I + c L)^{-1} = G (I + c D)^{-1} H: H's rows scaled block by block, one product with G.  Zero pivots: false, as below.
+CPDP_D bool bdf_factor_eig(double* sm, const double c) {
+    constexpr int n = NX;
+    const int lane = threadIdx.x;
+    const bool own = lane < n;
+    const int j = own ? lane : 0;
+    const double* TD = sm + bo::TD; const double* part = sm + bo::ROT + 3 * n;
+    double* s1 = sm + bo::ROT; double* s2 = s1 + n;                    // row scaling of (I + cD)^{-1}: own row | partner row
+    double* XA = sm + bo::XA;
+    BDF_SYNC();
+    double bad = 0.0;
+    if (own) {
+        const auto lj = BDF_LD2(TD + 2 * j);
+        const int pj = (int)part[j];
+        const double sj = (pj > j) ? 1.0 : ((pj < j) ? -1.0 : 0.0);
+        CPDP_LOOP for (int i = 0; i < n; ++i) {
+            const auto li = BDF_LD2(TD + 2 * i);
+            const int pi = (int)part[i];
+            const double si = (pi > i) ? 1.0 : ((pi < i) ? -1.0 : 0.0);
+            const double er = 1.0 + c * (li.x + lj.x), ep = c * (li.y - lj.y), em = -c * (li.y + lj.y);
+            const double mp = er * er + ep * ep, mm = er * er + em * em;
+            if (!(mp > 0.0) || !(mm > 0.0)) bad = 1.0;
+            const double ip = 1.0 / mp, im = 1.0 / mm;
+            const double u = er * ip, v = -ep * ip, w = er * im, t = -em * im;       // w+ = u + iv, w- = w + it
+            BDF_ST2(sm + bo::PV + 2 * (i * n + j), 0.5 * (u + w), si * (0.5 * (v - t)));
+            BDF_ST2(sm + bo::Y2 + 2 * (i * n + j), -sj * (0.5 * (v + t)), (si * sj) * (0.5 * (u - w)));
+        }
+        const double dr = 1.0 + c * lj.x, di = c * lj.y, md = dr * dr + di * di;      // 1 / (1 + c (a + ib))
+        if (!(md > 0.0)) bad = 1.0;
+        s1[j] = dr / md; s2[j] = sj * (-di / md);
+    }
+    BDF_SYNC();
+    if (own) {                                                         // XA[i][k] = ((I + cD)^{-1} H)[i][k], my column k
+        CPDP_LOOP for (int i = 0; i < n; ++i) XA[i * NCS + j] = s1[i] * sm[bo::Q + j * QS + i] + s2[i] * sm[bo::Q + j * QS + (int)part[i]];
+    }
+    BDF_SYNC();
+    int hc, hi0;
+    if (bdf_half(lane, hc, hi0)) bdf_lmul_to(sm + bo::QT, QS, XA + hc, NCS, sm + bo::WT + hc * QS, 1, hi0);     // WT[k][i] = Winv[i][k]
+    BDF_SYNC();
+    return !bdf_ballot(sm, bad != 0.0);
+}
+
 // scipy's "LU" event for a new c: the Lyapunov pivots of the sweep and (I + c L)^{-1} by Gauss-Jordan elimination with partial
 // pivoting on [I + cL | I]: lane c < n owns column c of the left half, lane 16 + c column c of the right half.
 CPDP_D_NOINLINE bool bdf_factor(const double c) {
@@ -730,6 +921,7 @@ CPDP_D_NOINLINE bool bdf_factor(const double c) {
     const bool isP = lane < n, isB = (lane >= 16) && (lane < 16 + n);
     const double* TD = sm + bo::TD;
     double* XA = sm + bo::XA; double* XB = sm + bo::XB;
+    if (BDF_EIG_KAPPA > 0.0 && ((const int*)(sm + bo::FLAG))[3]) return bdf_factor_eig(sm, c);
     BDF_SYNC();
     double bad = 0.0;
     if (isP) {
@@ -882,6 +1074,8 @@ CPDP_D void bdf_solve_cols(double* sm, const double c, double (&r)[NX] BDF_TP_PA
     double* XA = sm + bo::XA; double* XB = sm + bo::XB;
     int hc, hi0;
     const bool hact = bdf_half(lane, hc, hi0);                   // products: lanes c and 16 + c share column c
+    const bool eig = BDF_EIG_KAPPA > 0.0 && ((const int*)(sm + bo::FLAG))[3];     // (uniform)
+    double* ZB = sm + bo::T2S;                                   // eigen path: Z, row stride QS
     BDF_T(10, {
     if (isP) bdf_put(XA, j, r);
     BDF_SYNC();
@@ -890,6 +1084,20 @@ CPDP_D void bdf_solve_cols(double* sm, const double c, double (&r)[NX] BDF_TP_PA
     if (hact) bdf_lmul_to(sm + bo::Q, QS, XB + hc * NCS, 1, XA + hc, NCS, hi0);    // Q'(row c of Q'B)' = row c (= column c) of E = Q'BQ
     BDF_SYNC();
     });
+    if (eig) {
+    BDF_T(9, {
+    if (isP) {                                                   // Z = block-diagonal solve of E = H B' H' (bdf_factor_eig), my column
+        const double* part = rot + 3 * n;
+        const int pj = (int)part[j];
+        CPDP_LOOP for (int i = 0; i < n; ++i) {
+            const int pi = (int)part[i];
+            const auto k12 = BDF_LD2(sm + bo::PV + 2 * (i * n + j)), k34 = BDF_LD2(sm + bo::Y2 + 2 * (i * n + j));
+            ZB[i * QS + j] = ((k12.x * XA[i * NCS + j] + k12.y * XA[pi * NCS + j]) + k34.x * XA[i * NCS + pj]) + k34.y * XA[pi * NCS + pj];
+        }
+    }
+    BDF_SYNC();
+    });
+    } else {
     BDF_T(11, {
     if (isP) {                                                   // C = G E G^H, upper triangle of my column -> sweep array
         BDF_PRAGMA_UNROLL(CPDP_BDF_STENCIL_UNROLL) for (int i = 0; i <= j; ++i) {
@@ -907,8 +1115,9 @@ CPDP_D void bdf_solve_cols(double* sm, const double c, double (&r)[NX] BDF_TP_PA
     }
     BDF_SYNC();
     });
+    }
     BDF_T(14, {
-    if (hact) bdf_lmul_to(sm + bo::QT, QS, XA + hc, NCS, XB + hc, NCS, hi0);       // (Q Yr)[:, c]
+    if (hact) bdf_lmul_to(sm + bo::QT, QS, (eig ? ZB : XA) + hc, eig ? QS : NCS, XB + hc, NCS, hi0);     // (Q Yr)[:, c] | (G Z)[:, c]
     BDF_SYNC();
     if (hact) bdf_lmul_to(sm + bo::QT, QS, XB + hc * NCS, 1, XA + hc, NCS, hi0);   // row c of X = Q Yr Q':  XA[i][c] = X[c][i]
     BDF_SYNC();
@@ -1027,6 +1236,7 @@ CPDP_D int bdf_interval(double* sm, double* D, const AuxProblem& p, const double
     bdf_get_col(sm + bo::XB, lc, f0);
     BDF_SYNC();
     { bool oks__; BDF_TB(3, oks__, bdf_schur()); if (!oks__) return 4; }
+    BDF_PATH(sm, 2);
     double h_abs;
     {
         const double interval_length = fabs(t1 - t0);
@@ -1134,6 +1344,7 @@ CPDP_D int bdf_interval(double* sm, double* D, const AuxProblem& p, const double
                     }
                     if (bdf_ballot(sm, fin)) break;
                     BDF_T(5, bdf_solve_cols(sm, c_lu, r BDF_TP_ARG));
+                    BDF_PATH(sm, 0);
                     double dy_norm; BDF_TB(6, dy_norm, bdf_norm_cols(r, isc, 1.0, act));
                     const bool have_rate = dy_norm_old >= 0.0;
                     const double rate = have_rate ? dy_norm / dy_norm_old : 0.0;
@@ -1158,6 +1369,7 @@ CPDP_D int bdf_interval(double* sm, double* D, const AuxProblem& p, const double
                     BDF_SYNC();
                     BDF_T(2, bdf_jacobian()); ++cnt[3];
                     { bool oks__; BDF_TB(3, oks__, bdf_schur()); if (!oks__) return 4; }
+                    BDF_PATH(sm, 2);
                     lu_valid = false;
                     current_jac = true;
                 }
@@ -1265,7 +1477,7 @@ CPDP_GLOBAL void __launch_bounds__(BDF_THREADS, CPDP_BDF_MINB) k_riccati_bdf(Aux
         }                                                                                               \
     }
     BDF_STORE_NODE(N)
-    int cnt[4] = {0, 0, 0, 0};
+    int cnt[8] = {0, 0, 0, 0, 0, 0, 0, 0};                          // (4..7: CPDP_BDF_PATH_COUNTS)
     int st = 0;
 #ifdef CPDP_BDF_TIMING
     long long tp[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
@@ -1285,6 +1497,9 @@ CPDP_GLOBAL void __launch_bounds__(BDF_THREADS, CPDP_BDF_MINB) k_riccati_bdf(Aux
         for (int i = 0; i < 16; ++i) dst[i] = (double)tp[i];
         for (int i = 0; i < 8; ++i) dst[16 + i] = sm[bo::TS + i];
     }
+#endif
+#ifdef CPDP_BDF_PATH_COUNTS
+    if (lane == 0) { for (int i = 0; i < 4; ++i) a.Ua[(size_t)b * (N + 1) * NU * NP + 24 + i] = (double)cnt[4 + i]; }
 #endif
     if (lane == 0) {
         a.aux_status[b] = st;

@@ -18,6 +18,8 @@ sys.path.insert(0, ROOT)
 VARIANTS = {
     "base": [],
     "time": ["-DCPDP_BDF_TIMING"],
+    "eig_off": ["-DCPDP_BDF_EIG_KAPPA=0"],                    # every Newton solve on the Bartels-Stewart sweep
+    "time_eig_off": ["-DCPDP_BDF_TIMING", "-DCPDP_BDF_EIG_KAPPA=0"],
     "l2s1": ["-DCPDP_BDF_LMUL_UNROLL=2", "-DCPDP_BDF_STENCIL_UNROLL=1"],
     "l1s1": ["-DCPDP_BDF_LMUL_UNROLL=1", "-DCPDP_BDF_STENCIL_UNROLL=1"],
     "l4s2": ["-DCPDP_BDF_LMUL_UNROLL=4", "-DCPDP_BDF_STENCIL_UNROLL=2"],
@@ -78,7 +80,7 @@ def main():
             out = {"variant": v, "batch": B, "ms": [round(t, 3) for t in times],
                    "failed": int((aux["aux_status"] != 0).sum().item())}
             if "time" in v:
-                tp = aux["Ua"].reshape(B, -1)[:, :24].cpu().numpy()
+                tp = aux["Ua"].reshape(B, -1)[:, :28].cpu().numpy()
                 tot = tp[:, 8].mean()
                 out["cycles_total_mean"] = float(tot)
                 out["phase_share"] = {PHASES[i]: round(float(tp[:, i].mean() / tot), 4) for i in range(8)}
@@ -93,11 +95,17 @@ def main():
                     "solve": float(tp[:, 5].mean() / (cnt[:, 0].mean() - 2 * a.n_grid)),
                 }
                 nsol = cnt[:, 0].mean() - 2 * a.n_grid
-                out["solve_cycles_per_call"] = {nm: float(tp[:, 10 + i].mean() / nsol) for i, nm in enumerate(
-                    ["QtBQ", "stencil_in", "sweep", "stencil_out", "QYQt", "sym_W"])}
+                # Newton solves / Jacobians on the eigen path and on the sweep (path counts of the timing build)
+                n_eig, n_sweep, j_eig, j_sweep = (float(tp[:, 24 + i].mean()) for i in range(4))
+                out["paths"] = {"solves_eig": n_eig, "solves_sweep": n_sweep, "jac_eig": j_eig, "jac_sweep": j_sweep,
+                                "solves_sweep_share": round(n_sweep / max(n_eig + n_sweep, 1e-300), 4)}
+                per = lambda col, n_: float(tp[:, col].mean() / n_) if n_ > 0 else None
+                out["solve_cycles_per_call"] = {"QtBQ": per(10, nsol), "QYQt": per(14, nsol), "sym_W": per(15, nsol),
+                                                "block_scaling": per(9, n_eig), "stencil_in": per(11, n_sweep),
+                                                "sweep": per(12, n_sweep), "stencil_out": per(13, n_sweep)}
                 nj = cnt[:, 5].mean()
                 out["schur_cycles_per_call"] = {nm: float(tp[:, 16 + i].mean() / nj) for i, nm in enumerate(
-                    ["hessenberg", "qr_scans", "qr_scans_plus_chase", "rotations", "rotations_plus_packing"])}
+                    ["hessenberg", "qr_scans", "qr_scans_plus_chase", "rotations", "rotations_plus_packing", "eig_basis"])}
                 out["counters_mean"] = {"rhs": cnt[:, 0].mean(), "steps": cnt[:, 1].mean(), "lu": cnt[:, 4].mean(), "jac": nj}
             print(json.dumps(out), flush=True)
 
