@@ -21,8 +21,8 @@
 extern "C" {
 #endif
 
-/* per-problem solver status written by cpdp_solve */
-enum { CPDP_RUNNING = 0, CPDP_CONVERGED = 1, CPDP_MAXITER = 2, CPDP_LINESEARCH = 3, CPDP_NUMERIC = 4 };
+/* per-problem solver status written by cpdp_solve; CPDP_INFEASIBLE: x0 is not strictly inside a finite state bound */
+enum { CPDP_RUNNING = 0, CPDP_CONVERGED = 1, CPDP_MAXITER = 2, CPDP_LINESEARCH = 3, CPDP_NUMERIC = 4, CPDP_INFEASIBLE = 5 };
 
 /* Model dimensions compiled into this library (COCSys.n_state / n_control / n_auxvar, CPDP.py:17,22,36);
  * q = number of per-problem constants (pdata, e.g. a goal position), 0 for most models. */
@@ -30,6 +30,18 @@ int cpdp_model_dims(int* n, int* m, int* r, int* q);
 
 /* Length of one packed Riccati node [upper-tri(P) | W] = n(n+1)/2 + n*r (internal table of auxSysSolver). */
 int cpdp_riccati_state_dim(void);
+
+/* Box bounds compiled into this library (COCSys.setStateVariable / setControlVariable bounds): lb[n+m], ub[n+m] host arrays,
+ * states then controls, -1e20 / +1e20 where there is none.  Returns 1 when some bound is finite, 0 otherwise.  A bounded library's
+ * cpdp_solve runs a primal-dual interior-point (barrier) method and keeps the bound multipliers in the workspace. */
+int cpdp_bounds(double* lb, double* ub);
+
+/* Copy the bound multipliers z_L, z_U [B][N+1][n+m] (row N: the final state's entries; 0 where there is no bound) and the barrier
+ * parameter mu[B] out of the workspace a bounded cpdp_solve left them in (get), or into it (set).  cpdp_aux mode 2 reads them
+ * there, so a solution passed in from elsewhere is differentiated after a set.  Device arrays; -11 for an unbounded library. */
+int cpdp_get_bound_multipliers(void* ws, size_t ws_bytes, int B, int N, int S, double* Zl, double* Zu, double* mu, void* stream);
+int cpdp_set_bound_multipliers(void* ws, size_t ws_bytes, int B, int N, int S, const double* Zl, const double* Zu,
+                               const double* mu, void* stream);
 
 /* 1 if mode 1 (as-shipped BDF backward sweep) of cpdp_aux is compiled in; ints per row of `counters`. */
 int cpdp_has_bdf(void);
@@ -39,7 +51,8 @@ int cpdp_num_counters(void);
 size_t cpdp_workspace_bytes(int B, int N, int S);
 
 /* Replaces COCSys.cocSolver (CPDP.py:92-198) for B problems: RK4 multiple-shooting NLP, all-zeros seed,
- * Newton-KKT with IPOPT's inertia correction and filter line search.
+ * Newton-KKT with IPOPT's inertia correction and filter line search; with box bounds (cpdp_bounds) IPOPT's primal-dual
+ * barrier method on the same recursion (z_L, z_U, mu: cpdp_get_bound_multipliers).
  *   x0[B][n]; theta[B][r] (theta_stride = r) or shared theta[r] (theta_stride = 0); T horizon;
  *   tol: KKT tolerance; max_iter: Newton iteration cap, 0..255 (the per-problem filter holds 256 corners; -10 otherwise);
  *   rounds > 0: launch exactly that many Newton rounds with no host synchronisation (CUDA-graph capturable);

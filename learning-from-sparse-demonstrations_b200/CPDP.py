@@ -99,29 +99,38 @@ class COCSys:
         self._lib = None
 
     def setStateVariable(self, state, state_lb=[], state_ub=[]):
-        """CPDP.py:20-31.  Bounds are accepted for signature parity; the reference examples never set them and
-        the B200 path supports the unbounded case only."""
+        """CPDP.py:20-31.  Bounds of the wrong length mean "none" (+-1e20), as in the reference; finite bounds are compiled
+        into the model and enforced by the solver's barrier method (DESIGN.md §3.8)."""
         self.state = state
         self.n_state = self.state.numel()
-        self.state_lb = state_lb if len(state_lb) == self.n_state else self.n_state * [-1e20]
-        self.state_ub = state_ub if len(state_ub) == self.n_state else self.n_state * [1e20]
-        self._check_unbounded(self.state_lb, self.state_ub)
+        self.state_lb, self.state_ub = self._check_bounds(state_lb, state_ub, self.n_state)
         self._lib = None
 
     def setControlVariable(self, control, control_lb=[], control_ub=[]):
         """CPDP.py:34-46"""
         self.control = control
         self.n_control = self.control.numel()
-        self.control_lb = control_lb if len(control_lb) == self.n_control else self.n_control * [-1e20]
-        self.control_ub = control_ub if len(control_ub) == self.n_control else self.n_control * [1e20]
-        self._check_unbounded(self.control_lb, self.control_ub)
+        self.control_lb, self.control_ub = self._check_bounds(control_lb, control_ub, self.n_control)
         self._lib = None
 
     @staticmethod
-    def _check_unbounded(lb, ub):
-        if any(v > -1e19 for v in lb) or any(v < 1e19 for v in ub):
-            raise NotImplementedError("finite state/control bounds are not supported by the batched Newton-KKT "
-                                      "solver (no reference example uses them)")
+    def _check_bounds(lb, ub, n):
+        lb = list(numpy.asarray(lb, dtype=float).ravel())
+        ub = list(numpy.asarray(ub, dtype=float).ravel())
+        lb, ub = codegen.normalize_bounds(lb, ub, n)
+        for i, (lo, hi) in enumerate(zip(lb, ub)):
+            if not lo < hi:
+                raise ValueError("bound %d: lower bound %r is not below upper bound %r (fixed variables are not supported)"
+                                 % (i, lo, hi))
+        return lb, ub
+
+    def _bounds(self):
+        return (self.state_lb, self.state_ub, self.control_lb, self.control_ub)
+
+    @property
+    def bounded(self):
+        """True when some state or control bound is finite."""
+        return any(abs(v) < 1e19 for v in self.state_lb + self.state_ub + self.control_lb + self.control_ub)
 
     def setProblemVariable(self, pvar):
         """Extension: symbols that are per-problem constants (e.g. a goal position) — not learnable, not states.
@@ -206,13 +215,15 @@ class COCSys:
             return self._lib
         text, info = codegen.generate_model_header(name or self.sys_name, self.state, self.control, self.auxvar,
                                                     self.dyn, self.path_cost, self.final_cost, self.pvar,
-                                                    time=getattr(self, 'time', None))
+                                                    time=getattr(self, 'time', None), bounds=self._bounds())
         self.codegen_info = info
         libname = name if name is not None else "m" + info["hash"]
         so = _capi.build_model_library(libname, text, force=force, verbose=verbose)
         self._lib = _capi.CpdpLib(so)
         assert (self._lib.n, self._lib.m, self._lib.r, self._lib.q) == \
             (self.n_state, self.n_control, self.n_auxvar, self.n_pvar)
+        assert (self._lib.has_bounds, self._lib.lb, self._lib.ub) == \
+            (self.bounded, self.state_lb + self.control_lb, self.state_ub + self.control_ub)
         return self._lib
 
     def _device(self):
@@ -254,7 +265,8 @@ class COCSys:
     def cocSolverBatch(self, ini_states, horizon, auxvar_value, pdata=None, rounds=0, _slot=0):
         """Batched cocSolver: ini_states [B,n]; auxvar_value [r] (shared) or [B,r]; pdata [B,q].
         Returns a dict of device arrays X [B,N+1,n], U [B,N+1,m], Lam [B,N+1,n], status, iters, kkt, cost
-        and the host time_grid."""
+        and the host time_grid; a bounded model adds the bound multipliers Zl, Zu [B,N+1,n+m] (row N: the final state's) and
+        the final barrier parameter mu [B]."""
         self._assert_defined()
         if not hasattr(self, 'n_grid'):
             self.setIntegrator()
@@ -278,6 +290,11 @@ class COCSys:
                   float(self.tol), int(self.max_iter), int(rounds),
                   mem.ptr(out["X"]), mem.ptr(out["U"]), mem.ptr(out["Lam"]), mem.ptr(out["status"]), mem.ptr(out["iters"]),
                   mem.ptr(out["kkt"]), mem.ptr(out["cost"]), mem.stream())
+        if lib.has_bounds:
+            nz = self.n_state + self.n_control
+            out.update(Zl=mem.empty((B, N + 1, nz)), Zu=mem.empty((B, N + 1, nz)), mu=mem.empty((B,)))
+            lib.get_bound_multipliers(mem.ptr(ws), int(ws.shape[0]), B, N, S, mem.ptr(out["Zl"]), mem.ptr(out["Zu"]),
+                                      mem.ptr(out["mu"]), mem.stream())
         out.update(time_grid=self._time_grid(horizon, N), horizon=float(horizon),
                    theta=th, theta_stride=th_stride, pdata=pd, B=B, x0=x0, _slot=_slot)
         return out
@@ -314,6 +331,12 @@ class COCSys:
             wp_h = waypoints if hasattr(waypoints, 'data_ptr') else numpy.asarray(waypoints, dtype=float).reshape(B, W, D)
             wp_d = mem.from_host(wp_h)
         ws = self._workspace(B, sol.get("_slot", 0))
+        if lib.has_bounds and int(mode) == COCSys.MODE_DISCRETE and phases & 1:
+            # mode 2 differentiates the barrier-perturbed KKT system: it reads the bound multipliers from the workspace
+            if sol.get("Zl") is None:
+                raise ValueError("mode 2 on a bounded model needs the bound multipliers Zl, Zu, mu of the solution")
+            lib.set_bound_multipliers(mem.ptr(ws), int(ws.shape[0]), B, N, S, mem.ptr(sol["Zl"]), mem.ptr(sol["Zu"]),
+                                      mem.ptr(sol["mu"]), mem.stream())
         if out is None:
             out = dict(Xa=mem.empty((B, N + 1, n * r)), Ua=mem.empty((B, N + 1, m * r)), loss=mem.empty((B,)),
                        dtheta=mem.empty((B, r)), aux_status=mem.zeros((B,), "i4"),
@@ -423,7 +446,8 @@ class COCSys:
             auxs.append(aux)
         for st in streams[:chunks]:
             main.wait_stream(st)
-        sol = {k: torch.cat([s_[k] for s_ in sols]) for k in ("X", "U", "Lam", "status", "iters", "kkt", "cost")}
+        sol = {k: torch.cat([s_[k] for s_ in sols]) for k in ("X", "U", "Lam", "status", "iters", "kkt", "cost")
+               + (("Zl", "Zu", "mu") if "Zl" in sols[0] else ())}
         sol.update(time_grid=sols[0]["time_grid"], horizon=float(horizon), B=B, chunks=sols)
         aux = {k: torch.cat([a_[k] for a_ in auxs]) for k in ("Xa", "Ua", "loss", "dtheta", "aux_status", "counters")}
         full = self.reduceRows(self.packRows(sol, aux))
@@ -476,6 +500,9 @@ class COCSys:
                    X=mem.from_host(nodes[:, :n].reshape(1, N + 1, n)),
                    U=mem.from_host(nodes[:, n:n + m].reshape(1, N + 1, m)),
                    Lam=mem.from_host(nodes[:, n + m:].reshape(1, N + 1, n)), status=None)
+        batch = getattr(opt_sol, '_batch', None)       # bound multipliers of the cocSolver call behind opt_sol (bounded models)
+        if batch is not None and batch.get("Zl") is not None:
+            sol.update(Zl=batch["Zl"], Zu=batch["Zu"], mu=batch["mu"])
         aux = self.auxSysSolverBatch(sol)
         self.last_aux_status = int(mem.to_host(aux["aux_status"])[0])
         self.last_aux_counters = mem.to_host(aux["counters"])[0]

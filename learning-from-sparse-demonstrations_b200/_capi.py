@@ -20,7 +20,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 # build digest, so that a variant built in this container is used as it is on a GPU box that does not set the variable
 EXTRA_NVCC_FLAGS = os.environ.get("CPDP_EXTRA_NVCC_FLAGS", "").split()
 
-STATUS_NAMES = {0: "running", 1: "converged", 2: "max_iter", 3: "linesearch_fail", 4: "numeric"}
+STATUS_NAMES = {0: "running", 1: "converged", 2: "max_iter", 3: "linesearch_fail", 4: "numeric", 5: "infeasible"}
 
 _vp = ctypes.c_void_p
 _i = ctypes.c_int
@@ -136,6 +136,11 @@ class CpdpLib:
         L.cpdp_reduce_rows.restype = _i
         L.cpdp_optim_step.argtypes = [_i, _i, _d, _d, _d, _d, _d, _d, _d, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp]
         L.cpdp_optim_step.restype = _i
+        L.cpdp_bounds.argtypes = [ctypes.POINTER(_d), ctypes.POINTER(_d)]
+        L.cpdp_bounds.restype = _i
+        for fn in (L.cpdp_get_bound_multipliers, L.cpdp_set_bound_multipliers):
+            fn.argtypes = [_vp, _sz, _i, _i, _i, _vp, _vp, _vp, _vp]
+            fn.restype = _i
         if hasattr(L, "cpdp_error_string"):
             L.cpdp_error_string.argtypes = [_i]
             L.cpdp_error_string.restype = ctypes.c_char_p
@@ -147,6 +152,9 @@ class CpdpLib:
         L.cpdp_has_bdf.restype = _i
         self.ncounters = int(L.cpdp_num_counters())
         self.has_bdf = bool(L.cpdp_has_bdf())
+        lb, ub = (_d * (self.n + self.m))(), (_d * (self.n + self.m))()
+        self.has_bounds = bool(L.cpdp_bounds(lb, ub))
+        self.lb, self.ub = list(lb), list(ub)          # states then controls, +-1e20 for none
 
     def check(self, rc, what):
         if rc != 0:
@@ -175,6 +183,12 @@ class CpdpLib:
             self.check(self.L.cpdp_aux(*args), "cpdp_aux")
         else:
             self.check(self.L.cpdp_aux_phases(*(args + (phases,))), "cpdp_aux_phases")
+
+    def get_bound_multipliers(self, ws, ws_bytes, B, N, S, Zl, Zu, mu, stream):
+        self.check(self.L.cpdp_get_bound_multipliers(ws, ws_bytes, B, N, S, Zl, Zu, mu, stream), "cpdp_get_bound_multipliers")
+
+    def set_bound_multipliers(self, ws, ws_bytes, B, N, S, Zl, Zu, mu, stream):
+        self.check(self.L.cpdp_set_bound_multipliers(ws, ws_bytes, B, N, S, Zl, Zu, mu, stream), "cpdp_set_bound_multipliers")
 
     def dfma_probe(self, sink, blocks, iters, stream):
         self.check(self.L.cpdp_dfma_probe(sink, blocks, iters, stream), "cpdp_dfma_probe")

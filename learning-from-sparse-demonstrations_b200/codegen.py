@@ -97,11 +97,43 @@ def _sparse_tables(name, M):
                       "    static constexpr int %s_nnz = %d;" % (name, len(colidx))])
 
 
-def generate_model_header(name, state, control, auxvar, dyn, path_cost, final_cost, pdata=None, time=None):
+BOUND_INF = 1e20          # the reference's "no bound" (CPDP.py:24-29); |bound| >= 1e19 counts as none
+
+
+def normalize_bounds(lb, ub, n):
+    """Lists of n lower / upper bounds with every absent or infinite entry replaced by -/+BOUND_INF."""
+    lb = [-BOUND_INF if v <= -1e19 else float(v) for v in (lb if len(lb) == n else [-BOUND_INF] * n)]
+    ub = [BOUND_INF if v >= 1e19 else float(v) for v in (ub if len(ub) == n else [BOUND_INF] * n)]
+    return lb, ub
+
+
+def _bounds_block(bounds, n, m):
+    """Model members of the box bounds on the states and controls; empty text when no bound is finite, so that an unbounded
+    model's header does not change."""
+    if bounds is None:
+        return ""
+    xlb, xub, ulb, uub = bounds
+    if all(v <= -1e19 for v in list(xlb) + list(ulb)) and all(v >= 1e19 for v in list(xub) + list(uub)):
+        return ""
+    xlb, xub = normalize_bounds(xlb, xub, n)
+    ulb, uub = normalize_bounds(ulb, uub, m)
+    lines = ["    static constexpr int HAS_BOUNDS = 1;      // box bounds (+-1e20: none), read by the kernels' barrier method"]
+    for nm, v in (("XLB", xlb), ("XUB", xub), ("ULB", ulb), ("UUB", uub)):
+        # a chain of selects, not a table: a table indexed by a lane-dependent i would live in local memory
+        expr = repr(v[-1])
+        for i in range(len(v) - 2, -1, -1):
+            expr = "i == %d ? %r : %s" % (i, v[i], expr)
+        lines.append("    CPDP_HD static constexpr double %s(int i) { return %s; }" % (nm, expr))
+    return "\n".join(lines) + "\n"
+
+
+def generate_model_header(name, state, control, auxvar, dyn, path_cost, final_cost, pdata=None, time=None, bounds=None):
     """Returns (header_text, info dict).  All arguments are SX / sympy matrices / scalars.
     ``pdata``: optional per-problem constants (e.g. a goal position) that are not learnable.
     ``time``: the explicit time variable of a COCSys_TimeVarying model (CPDP.py:434); the generated functions read it as
-    one more constant, pd[nq], which the kernels fill in (the node time t_k in the RK4 map, the true t in the sweeps)."""
+    one more constant, pd[nq], which the kernels fill in (the node time t_k in the RK4 map, the true t in the sweeps).
+    ``bounds``: optional (state_lb, state_ub, control_lb, control_ub); the header gets HAS_BOUNDS and the four bound tables
+    only when some bound is finite."""
     x, u, th = _vec(state), _vec(control), _vec(auxvar)
     pdv = _vec(pdata) if pdata is not None else []
     n, m, r = len(x), len(u), len(th)
@@ -251,10 +283,11 @@ struct Model {{
     static constexpr int NQ = {nq};
     static constexpr int HAS_TIME = {has_time};
     static constexpr int NZ = {nz};
-{offs}
+{bounds}{offs}
 {tables}
 {parts}
 }};
-""".format(name=name, nz=nz, has_time=len(tv), offs="\n".join(offs), tables=tables, parts="\n\n".join(parts), **info)
+""".format(name=name, nz=nz, has_time=len(tv), bounds=_bounds_block(bounds, n, m), offs="\n".join(offs), tables=tables,
+           parts="\n\n".join(parts), **info)
     info["hash"] = hashlib.sha1(text.encode()).hexdigest()[:16]
     return text, info

@@ -1439,7 +1439,8 @@ CPDP_D int bdf_interval(double* sm, double* D, const AuxProblem& p, const double
 // k_riccati_bdf: backward sweep of COCSys.auxSysSolver as shipped (CPDP.py:327-338).
 CPDP_GLOBAL void __launch_bounds__(BDF_THREADS, CPDP_BDF_MINB) k_riccati_bdf(AuxArgs a) {
     const int b = blockIdx.x, lane = threadIdx.x;
-    if (a.solve_status && (a.solve_status[b] == ST_NUMERIC || a.solve_status[b] == ST_RUNNING)) {
+    if (a.solve_status && (a.solve_status[b] == ST_NUMERIC || a.solve_status[b] == ST_RUNNING ||
+                           (HAS_BOUNDS && a.solve_status[b] == ST_INFEASIBLE))) {
         if (lane == 0) a.aux_status[b] = 3;
         return;
     }
@@ -1646,7 +1647,8 @@ CPDP_D int rkw_interval(double* sm, const AuxProblem& p, const double t0, const 
 
 CPDP_GLOBAL void __launch_bounds__(BDF_THREADS, CPDP_BDF_MINB) k_riccati_rk45(AuxArgs a) {
     const int b = blockIdx.x, lane = threadIdx.x;
-    if (a.solve_status && (a.solve_status[b] == ST_NUMERIC || a.solve_status[b] == ST_RUNNING)) {
+    if (a.solve_status && (a.solve_status[b] == ST_NUMERIC || a.solve_status[b] == ST_RUNNING ||
+                           (HAS_BOUNDS && a.solve_status[b] == ST_INFEASIBLE))) {
         if (lane == 0) a.aux_status[b] = 3;
         return;
     }

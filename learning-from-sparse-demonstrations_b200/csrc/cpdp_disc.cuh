@@ -21,7 +21,8 @@ struct DiscWs {
 };
 
 CPDP_HD bool disc_usable(const int* solve_status, int b) {
-    return !solve_status || (solve_status[b] != ST_NUMERIC && solve_status[b] != ST_RUNNING);
+    return !solve_status || (solve_status[b] != ST_NUMERIC && solve_status[b] != ST_RUNNING &&
+                             !(HAS_BOUNDS && solve_status[b] == ST_INFEASIBLE));
 }
 
 // k_disc_select: ordered list of the problems with a usable trajectory (single CTA, as k_compact); aux_status 0 / 3, counters 0.
@@ -204,6 +205,15 @@ CPDP_GLOBAL void __launch_bounds__(DISC_THREADS) k_aux_discrete(AuxArgs x, Solve
         for (int q = lane; q < NX * NX; q += DISC_THREADS) {
             const int i = q / NX, c = q % NX;
             s_V[i * NXS + c] = 0.5 * (s_hxx[i * NX + c] + s_hxx[c * NX + i]);
+            if constexpr (HAS_BOUNDS) {
+                // bounded model: the barrier-perturbed KKT system adds Sigma = Z_L S_L^-1 + Z_U S_U^-1 of the final state
+                if (i == c) {
+                    const size_t o = ((size_t)b * (N + 1) + N) * NZ + i;
+                    double sg, bg;
+                    bnd_terms(i, a.X[((size_t)b * (N + 1) + N) * NX + i], a.zL[o], a.zU[o], 0.0, sg, bg);
+                    s_V[i * NXS + c] += sg;
+                }
+            }
         }
         for (int q = lane; q < NX * NP; q += DISC_THREADS) s_W[(q / NP) * NPS_D + q % NP] = s_hxe[q];
         NWT_SYNC();
@@ -223,6 +233,15 @@ CPDP_GLOBAL void __launch_bounds__(DISC_THREADS) k_aux_discrete(AuxArgs x, Solve
                 NWT_UNROLL for (int i = 0; i < NX; ++i) s_Y[i * DCS + c] = y[i];
                 double q[NZ];
                 NWT_UNROLL for (int r_ = 0; r_ < NZ; ++r_) q[r_] = (c < NZ) ? Hg[r_ * NZ + c] : Htg[r_ * NP + c - NZ];
+                if constexpr (HAS_BOUNDS) {
+                    if (c < NZ) {                          // + Sigma_k (diagonal) of the barrier-perturbed KKT system
+                        const size_t o = ((size_t)b * (N + 1) + k) * NZ + c;
+                        const double w = (c < NX) ? a.X[((size_t)b * (N + 1) + k) * NX + c] : a.U[((size_t)b * (N + 1) + k) * NU + c - NX];
+                        double sg, bg;
+                        bnd_terms(c, w, a.zL[o], a.zU[o], 0.0, sg, bg);
+                        NWT_UNROLL for (int r_ = 0; r_ < NZ; ++r_) if (r_ == c) q[r_] += sg;
+                    }
+                }
                 nwt_mac<NZ>(s_G, DCS, s_Y + c, DCS, NX, q);                    // (my own column of Y: no barrier needed)
                 NWT_UNROLL for (int r_ = 0; r_ < NZ; ++r_) s_Q[r_ * DCS + c] = q[r_];
             }

@@ -9,6 +9,7 @@
 //   reduction      : k_reduce_tree                                        (new: cross-problem sum, fixed order)
 // No tensor cores: per-step matrices are <= 13x13 (+ sparse), fp64.  Bound: FP64 pipe / latency, not HBM.
 #pragma once
+#include <type_traits>
 #include "cpdp_port.h"
 
 namespace CPDP_NS {
@@ -23,12 +24,73 @@ constexpr int NQT = NQ + HAS_TIME;          // the generated model code reads t 
 
 constexpr int FILTER_CAP = 256;        // filter entries per problem (one is added per h-type iteration at most)
 
-enum Status { ST_RUNNING = 0, ST_CONVERGED = 1, ST_MAXITER = 2, ST_LINESEARCH = 3, ST_NUMERIC = 4 };
+enum Status { ST_RUNNING = 0, ST_CONVERGED = 1, ST_MAXITER = 2, ST_LINESEARCH = 3, ST_NUMERIC = 4, ST_INFEASIBLE = 5 };
+
+// Box bounds on the states and controls (DESIGN.md §3.8).  A model header defines HAS_BOUNDS and XLB / XUB / ULB / UUB only when
+// some bound is finite; every other model takes the unbounded code path unchanged.
+template <class M, class = void> struct ModelBounds {
+    static constexpr int HAS = 0;
+    CPDP_HD static double lo(int) { return -1e20; }
+    CPDP_HD static double hi(int) { return 1e20; }
+};
+template <class M> struct ModelBounds<M, std::void_t<decltype(M::HAS_BOUNDS)>> {
+    static constexpr int HAS = M::HAS_BOUNDS;
+    // bound of component j of z = [x; u] (a chain of selects: no local-memory table for a lane-dependent j)
+    CPDP_HD static double lo(int j) {
+        double v = 0.0;
+        CPDP_PRAGMA_UNROLL(NX) for (int i = 0; i < NX; ++i) if (i == j) v = M::XLB(i);
+        CPDP_PRAGMA_UNROLL(NU) for (int i = 0; i < NU; ++i) if (NX + i == j) v = M::ULB(i);
+        return v;
+    }
+    CPDP_HD static double hi(int j) {
+        double v = 0.0;
+        CPDP_PRAGMA_UNROLL(NX) for (int i = 0; i < NX; ++i) if (i == j) v = M::XUB(i);
+        CPDP_PRAGMA_UNROLL(NU) for (int i = 0; i < NU; ++i) if (NX + i == j) v = M::UUB(i);
+        return v;
+    }
+};
+constexpr int HAS_BOUNDS = ModelBounds<Model>::HAS;
+CPDP_HD bool bnd_finite(double v) { return fabs(v) < 1e19; }
+
+// Barrier terms of component j (value w, multipliers zl, zu of its lower / upper bound, barrier parameter mu):
+// sig = zl/sl + zu/su (the diagonal Sigma), bg = -mu/sl + mu/su (the barrier's gradient), sl = w - lb, su = ub - w.
+CPDP_HD void bnd_terms(int j, double w, double zl, double zu, double mu, double& sig, double& bg) {
+    const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+    sig = 0.0; bg = 0.0;
+    if (bnd_finite(lb)) { const double s = w - lb; sig += zl / s; bg -= mu / s; }
+    if (bnd_finite(ub)) { const double s = ub - w; sig += zu / s; bg += mu / s; }
+}
+
+// Newton step of a bound multiplier z with slack s whose step is ds:  dz = mu/s - z - (z/s) ds.
+CPDP_HD double bnd_dz(double s, double z, double mu, double ds) { return mu / s - z - (z / s) * ds; }
+// ln of the slacks of component j at value w (the barrier's log terms; 0 for no finite bound)
+CPDP_HD double bnd_log(int j, double w) {
+    const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+    double v = 0.0;
+    if (bnd_finite(lb)) v += log(w - lb);
+    if (bnd_finite(ub)) v += log(ub - w);
+    return v;
+}
+
+// Workspace of the barrier method.  An unbounded model's SolveArgs gets an empty base (static null pointers), so that its layout --
+// and with it the kernel parameters of every kernel -- is the same as without bound support.
+template <int H> struct BoundPtrs {
+    double* zL;                  // [B][N+1][NZ]  multipliers of the lower bounds (row N: states only; 0 where no bound)
+    double* zU;                  // [B][N+1][NZ]  multipliers of the upper bounds
+    double* bmu;                 // [B]  barrier parameter
+};
+template <> struct BoundPtrs<0> {
+    static constexpr double* zL = nullptr;
+    static constexpr double* zU = nullptr;
+    static constexpr double* bmu = nullptr;
+};
+CPDP_HD void bind_bounds(BoundPtrs<1>& p, double* zl, double* zu, double* mu) { p.zL = zl; p.zU = zu; p.bmu = mu; }
+CPDP_HD void bind_bounds(BoundPtrs<0>&, double*, double*, double*) {}
 
 // ------------------------------------------------------------------------------------------------
 // Arguments of the forward-solve kernels (passed by value).
 // ------------------------------------------------------------------------------------------------
-struct SolveArgs {
+struct SolveArgs : BoundPtrs<HAS_BOUNDS> {
     int B, N, S;                 // problems, grid intervals, RK4 substeps per interval
     double T;                    // horizon
     double tol;                  // KKT tolerance
@@ -537,18 +599,70 @@ CPDP_D void newton_step_problem(const SolveArgs& a, const int b) {
 
     // ---- KKT error and objective
     double e = 0.0, Jp = 0.0, g1 = 0.0;
-    for (int k = lane; k < N; k += nt) {
-        const double* g = a.gL + (ib + k) * NZ;
-        for (int i = 0; i < NX; ++i) e = fmax(e, fabs(g[i] - Lam[(size_t)k * NX + i]));
-        for (int i = 0; i < NU; ++i) e = fmax(e, fabs(g[NX + i]));
-        Jp += a.cost[ib + k];
+    double* zL = nullptr;
+    double* zU = nullptr;
+    if constexpr (!HAS_BOUNDS) {
+        for (int k = lane; k < N; k += nt) {
+            const double* g = a.gL + (ib + k) * NZ;
+            for (int i = 0; i < NX; ++i) e = fmax(e, fabs(g[i] - Lam[(size_t)k * NX + i]));
+            for (int i = 0; i < NU; ++i) e = fmax(e, fabs(g[NX + i]));
+            Jp += a.cost[ib + k];
+        }
+    } else {
+        // gradient of the Lagrangian with the bound multipliers: grad L - z_L + z_U
+        zL = a.zL + (size_t)b * (N + 1) * NZ;
+        zU = a.zU + (size_t)b * (N + 1) * NZ;
+        for (int k = lane; k < N; k += nt) {
+            const double* g = a.gL + (ib + k) * NZ;
+            for (int i = 0; i < NX; ++i) e = fmax(e, fabs(g[i] - Lam[(size_t)k * NX + i] - zL[(size_t)k * NZ + i] + zU[(size_t)k * NZ + i]));
+            for (int i = 0; i < NU; ++i) e = fmax(e, fabs(g[NX + i] - zL[(size_t)k * NZ + NX + i] + zU[(size_t)k * NZ + NX + i]));
+            Jp += a.cost[ib + k];
+        }
     }
     for (int i = lane; i < (N + 1) * NX; i += nt) { e = fmax(e, fabs(dfc[i])); g1 += fabs(dfc[i]); }
-    for (int i = lane; i < NX; i += nt) e = fmax(e, fabs(s_hx[i] - Lam[(size_t)N * NX + i]));
-    const double kkt = nwt_reduce(e, red, true);
+    if constexpr (!HAS_BOUNDS) {
+        for (int i = lane; i < NX; i += nt) e = fmax(e, fabs(s_hx[i] - Lam[(size_t)N * NX + i]));
+    } else {
+        for (int i = lane; i < NX; i += nt) e = fmax(e, fabs(s_hx[i] - Lam[(size_t)N * NX + i] - zL[(size_t)N * NZ + i] + zU[(size_t)N * NZ + i]));
+    }
+    double kkt = nwt_reduce(e, red, true);
     const double J0 = nwt_reduce(Jp, red, false) + s_h;
     g1 = nwt_reduce(g1, red, false);
+    // Barrier method (IPOPT's monotone mode, Waechter & Biegler 2006, §2-3; unscaled): the stop test is E_0 < tol, and while
+    // E_mu <= 10 mu the barrier parameter drops to max(tol/10, min(0.2 mu, mu^1.5)) and the filter is emptied.
+    // E_mu = max(|grad L - z_L + z_U|, |c|, |S z - mu|): the complementarity enters through max(S z) and min(S z).
+    double mu = 0.0, P0 = J0;                     // barrier parameter, barrier objective phi_mu at the current iterate
+    bool freset = false;
+    if constexpr (HAS_BOUNDS) {
+        mu = a.bmu[b];                              // (read before the reductions: lane 0 writes it back below)
+        double szmax = 0.0, nszmin = -1e300, lg = 0.0;
+        for (int idx = lane; idx < (N + 1) * NZ; idx += nt) {
+            const int k = idx / NZ, j = idx % NZ;
+            if (k == N && j >= NX) continue;
+            const double w = (j < NX) ? X[(size_t)k * NX + j] : U[(size_t)k * NU + j - NX];
+            const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+            if (bnd_finite(lb)) { const double sl = w - lb, p = sl * zL[idx]; szmax = fmax(szmax, p); nszmin = fmax(nszmin, -p); lg += log(sl); }
+            if (bnd_finite(ub)) { const double su = ub - w, p = su * zU[idx]; szmax = fmax(szmax, p); nszmin = fmax(nszmin, -p); lg += log(su); }
+        }
+        szmax = nwt_reduce(szmax, red, true);
+        nszmin = nwt_reduce(nszmin, red, true);
+        lg = nwt_reduce(lg, red, false);
+        const double est = kkt;
+        kkt = fmax(est, szmax);
+        if (kkt >= a.tol) {
+            while (fmax(est, fmax(szmax - mu, mu + nszmin)) <= 10.0 * mu) {
+                const double mn = fmax(a.tol / 10.0, fmin(0.2 * mu, pow(mu, 1.5)));
+                if (!(mn < mu)) break;
+                mu = mn;
+                freset = true;
+            }
+        }
+        P0 = J0 - mu * lg;
+    }
     if (lane == 0) { a.kkt[b] = kkt; a.J[b] = J0; }
+    if constexpr (HAS_BOUNDS) {
+        if (lane == 0) { a.bmu[b] = mu; if (freset) a.nfilt[b] = 0; }
+    }
     const int it = a.iters[b];
     if (!(kkt == kkt)) { if (lane == 0) a.status[b] = ST_NUMERIC; }
     if (kkt < a.tol || it >= a.max_iter || !(kkt == kkt)) {
@@ -557,19 +671,27 @@ CPDP_D void newton_step_problem(const SolveArgs& a, const int b) {
         return;
     }
 
+    // barrier terms of the final state (lane i: component i)
+    double sgN = 0.0, bgN = 0.0;
+    if constexpr (HAS_BOUNDS) {
+        if (isX) bnd_terms(jx, X[(size_t)N * NX + jx], zL[(size_t)N * NZ + jx], zU[(size_t)N * NZ + jx], mu, sgN, bgN);
+    }
+
     // ---- Riccati factorisation with inertia correction (IPOPT Alg. IC)
     const double dlast = a.dlast[b];
     double delta = 0.0;
     int attempt = 0;
     while (true) {
         if (isX) {
+            const double dN = HAS_BOUNDS ? delta + sgN : delta;          // (+ Sigma of the final state)
             NWT_UNROLL for (int i = 0; i < NX; ++i) {
-                const double v = s_hxx[i * NX + jx] + ((i == jx) ? delta : 0.0);
+                const double v = s_hxx[i * NX + jx] + ((i == jx) ? dN : 0.0);
                 s_V[i * NXS + jx] = v;
                 Vs[(size_t)N * NX * NX + i * NX + jx] = v;
             }
-            s_v[jx] = s_hx[jx];
-            vs[(size_t)N * NX + jx] = s_hx[jx];
+            const double hN = HAS_BOUNDS ? s_hx[jx] + bgN : s_hx[jx];      // (+ barrier gradient)
+            s_v[jx] = hN;
+            vs[(size_t)N * NX + jx] = hN;
         }
         if (lane == 0) s_flag = 0;
         NWT_SYNC();
@@ -586,6 +708,11 @@ CPDP_D void newton_step_problem(const SolveArgs& a, const int b) {
             NWT_UNROLL for (int e2 = 0; e2 < NX; ++e2) ab[e2] = isZ ? ABg[e2 * NZ + jz] : 0.0;
             NWT_UNROLL for (int r_ = 0; r_ < NZ; ++r_) hq[r_] = isZ ? Hg[r_ * NZ + jz] : 0.0;     // (k_stage_hessian writes H exactly symmetric: 0.5 (H + H') = H)
             const double gl = isZ ? gLg[jz] : 0.0;
+            double sgk = 0.0, bgk = 0.0;                 // barrier terms of my component of z_k
+            if constexpr (HAS_BOUNDS) {
+                if (isZ) bnd_terms(jz, jz < NX ? X[(size_t)k * NX + jz] : U[(size_t)k * NU + jz - NX], zL[(size_t)k * NZ + jz],
+                                   zU[(size_t)k * NZ + jz], mu, sgk, bgk);
+            }
             if (isX) { s_dk[jx] = dk1[jx]; s_lk[jx] = lk1[jx]; }
             NWT_UNROLL for (int e2 = 0; e2 < NX; ++e2) if (isZ) s_AB[e2 * NZS + jz] = ab[e2];
             NWT_SYNC();
@@ -602,12 +729,14 @@ CPDP_D void newton_step_problem(const SolveArgs& a, const int b) {
             // gq[j] = gL[j] - [A B][:, j]' lam_{k+1};  qv[j] = gq[j] + [A B][:, j]' vt
             double gqj = gl;
             NWT_UNROLL for (int e2 = 0; e2 < NX; ++e2) gqj -= ab[e2] * s_lk[e2];
+            if constexpr (HAS_BOUNDS) gqj += bgk;       // gradient of the barrier objective
             double qvj = gqj;
             NWT_UNROLL for (int e2 = 0; e2 < NX; ++e2) qvj += ab[e2] * s_vt[e2];
             if (isZ) { NWT_UNROLL for (int e2 = 0; e2 < NX; ++e2) s_T[e2 * NZS + jz] = t[e2]; a.gq[(ib + k) * NZ + jz] = gqj; }
-            // Q[:, j] = sym(H)[:, j] + delta e_j + [A B]' T[:, j]
+            // Q[:, j] = sym(H)[:, j] + (delta + Sigma_j) e_j + [A B]' T[:, j]
             double q[NZ];
-            NWT_UNROLL for (int r_ = 0; r_ < NZ; ++r_) q[r_] = hq[r_] + ((isZ && r_ == jz) ? delta : 0.0);
+            const double dk = HAS_BOUNDS ? delta + sgk : delta;
+            NWT_UNROLL for (int r_ = 0; r_ < NZ; ++r_) q[r_] = hq[r_] + ((isZ && r_ == jz) ? dk : 0.0);
             if (isZ) nwt_mac<NZ>(s_AB, NZS, s_T + jz, NZS, NX, q);          // (reads my own column of T: no barrier needed)
             if (isZ) { NWT_UNROLL for (int r_ = 0; r_ < NZ; ++r_) s_Q[r_ * NZS + jz] = q[r_]; }
             NWT_SYNC();
@@ -732,13 +861,44 @@ CPDP_D void newton_step_problem(const SolveArgs& a, const int b) {
         for (int i = 0; i < NX; ++i) gd += g[i] * dX[(size_t)k * NX + i];
         for (int i = 0; i < NU; ++i) gd += g[NX + i] * dU[(size_t)k * NU + i];
     }
-    for (int i = lane; i < NX; i += nt) gd += s_hx[i] * dX[(size_t)N * NX + i];
+    if constexpr (!HAS_BOUNDS) {
+        for (int i = lane; i < NX; i += nt) gd += s_hx[i] * dX[(size_t)N * NX + i];
+    } else {
+        if (isX) gd += (s_hx[jx] + bgN) * dX[(size_t)N * NX + jx];
+    }
     bad = nwt_reduce(bad, red, true);
     gd = nwt_reduce(gd, red, false);
     if (bad != 0.0 || !(gd == gd)) {
         if (lane == 0) a.status[b] = ST_NUMERIC;
         for (int i = lane; i < NU; i += nt) U[(size_t)N * NU + i] = U[(size_t)(N - 1) * NU + i];
         return;
+    }
+
+    // ---- fraction to the boundary, tau = max(0.99, 1 - mu): the largest primal step alpha_max and dual step alpha_z in (0, 1]
+    //      that keep every slack / bound multiplier above (1 - tau) times its value
+    double amax = 1.0, az = 1.0;
+    if constexpr (HAS_BOUNDS) {
+        const double tau = fmax(0.99, 1.0 - mu);
+        double na = -1.0, nz = -1.0;               // -alpha_max, -alpha_z
+        for (int idx = lane; idx < (N + 1) * NZ; idx += nt) {
+            const int k = idx / NZ, j = idx % NZ;
+            if (k == N && j >= NX) continue;
+            const double w = (j < NX) ? X[(size_t)k * NX + j] : U[(size_t)k * NU + j - NX];
+            const double dw = (j < NX) ? dX[(size_t)k * NX + j] : dU[(size_t)k * NU + j - NX];
+            const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+            if (bnd_finite(lb)) {
+                const double sl = w - lb, dz = bnd_dz(sl, zL[idx], mu, dw);
+                if (dw < 0.0) na = fmax(na, tau * sl / dw);
+                if (dz < 0.0) nz = fmax(nz, tau * zL[idx] / dz);
+            }
+            if (bnd_finite(ub)) {
+                const double su = ub - w, dz = bnd_dz(su, zU[idx], mu, -dw);
+                if (dw > 0.0) na = fmax(na, -(tau * su / dw));
+                if (dz < 0.0) nz = fmax(nz, tau * zU[idx] / dz);
+            }
+        }
+        amax = -nwt_reduce(na, red, true);
+        az = -nwt_reduce(nz, red, true);
     }
 
     // ---- IPOPT filter line search (Waechter & Biegler 2006, Sec. 2.3; phi = J, theta = |g|_1, default constants
@@ -751,22 +911,25 @@ CPDP_D void newton_step_problem(const SolveArgs& a, const int b) {
 #endif
     NWT_SYNC();
     const double theta_min = 1e-4 * a.th_init[b], theta_max = 1e4 * a.th_init[b];
-    const int nf = a.nfilt[b];
+    int nf = a.nfilt[b];
+    if constexpr (HAS_BOUNDS) { if (freset) nf = 0; }
     const double* filt = a.filt + (size_t)b * FILTER_CAP * 2;
     const double sw_rhs = pow(th0, 1.1);
     const double sw_lhs = (gd < 0) ? pow(-gd, 2.3) : 0.0;
-    double alpha = 1.0;
+    double alpha = amax;
     bool ok = false, ftype = false;
     for (int ls = 0; ls <= 30; ++ls) {
-        double Jt = 0.0, gt = 0.0;
+        double Jt = 0.0, gt = 0.0, lt = 0.0;
         for (int k = lane; k <= N; k += nt) {
             double xk[NX];
             PdBuf pdb;
             const double* pd = pd_at(pd0, grid_time(a.T, N, k), pdb);
             for (int i = 0; i < NX; ++i) xk[i] = X[(size_t)k * NX + i] + alpha * dX[(size_t)k * NX + i];
+            if constexpr (HAS_BOUNDS) { NWT_UNROLL for (int i = 0; i < NX; ++i) lt += bnd_log(i, xk[i]); }
             if (k < N) {
                 double uk[NU], xe[NX], q;
                 for (int i = 0; i < NU; ++i) uk[i] = U[(size_t)k * NU + i] + alpha * dU[(size_t)k * NU + i];
+                if constexpr (HAS_BOUNDS) { NWT_UNROLL for (int i = 0; i < NU; ++i) lt += bnd_log(NX + i, uk[i]); }
                 rk4_interval(xk, uk, th, pd, DT, a.S, xe, q);
                 Jt += q;
                 for (int i = 0; i < NX; ++i)
@@ -780,15 +943,16 @@ CPDP_D void newton_step_problem(const SolveArgs& a, const int b) {
         }
         Jt = nwt_reduce(Jt, red, false);
         gt = nwt_reduce(gt, red, false);
+        if constexpr (HAS_BOUNDS) Jt -= mu * nwt_reduce(lt, red, false);        // barrier objective at the trial point
         bool acc = (Jt == Jt) && (gt == gt) && fabs(Jt) < 1e300 && gt <= theta_max;
         for (int e2 = 0; acc && e2 < nf; ++e2) if (gt >= filt[2 * e2] && Jt >= filt[2 * e2 + 1]) acc = false;
         if (acc) {
             const bool switching = (gd < 0) && (alpha * sw_lhs > sw_rhs);
             if (switching && th0 <= theta_min) {
-                acc = (Jt <= J0 + 1e-8 * alpha * gd);
+                acc = (Jt <= P0 + 1e-8 * alpha * gd);
                 ftype = acc;
             } else {
-                acc = (gt <= (1 - 1e-5) * th0) || (Jt <= J0 - 1e-8 * th0);
+                acc = (gt <= (1 - 1e-5) * th0) || (Jt <= P0 - 1e-8 * th0);
             }
         }
         if (acc) { ok = true; break; }
@@ -801,11 +965,32 @@ CPDP_D void newton_step_problem(const SolveArgs& a, const int b) {
     }
     if (!ftype && lane == 0 && nf < FILTER_CAP) {
         a.filt[((size_t)b * FILTER_CAP + nf) * 2] = (1 - 1e-5) * th0;
-        a.filt[((size_t)b * FILTER_CAP + nf) * 2 + 1] = J0 - 1e-8 * th0;
+        a.filt[((size_t)b * FILTER_CAP + nf) * 2 + 1] = P0 - 1e-8 * th0;
         a.nfilt[b] = nf + 1;
     }
 
     // ---- update
+    if constexpr (HAS_BOUNDS) {
+        // z += alpha_z dz, then IPOPT's safeguard: z_L within [mu / (kappa_Sigma s_L), kappa_Sigma mu / s_L] at the new slack s_L,
+        // kappa_Sigma = 1e10 (before the primal update below: the new slacks are formed here from the old values)
+        for (int idx = lane; idx < (N + 1) * NZ; idx += nt) {
+            const int k = idx / NZ, j = idx % NZ;
+            if (k == N && j >= NX) continue;
+            const double w = (j < NX) ? X[(size_t)k * NX + j] : U[(size_t)k * NU + j - NX];
+            const double dw = (j < NX) ? dX[(size_t)k * NX + j] : dU[(size_t)k * NU + j - NX];
+            const double wn = w + alpha * dw;
+            const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+            if (bnd_finite(lb)) {
+                const double z = zL[idx] + az * bnd_dz(w - lb, zL[idx], mu, dw), sn = wn - lb;
+                zL[idx] = fmax(fmin(z, 1e10 * mu / sn), mu / (1e10 * sn));
+            }
+            if (bnd_finite(ub)) {
+                const double z = zU[idx] + az * bnd_dz(ub - w, zU[idx], mu, -dw), sn = ub - wn;
+                zU[idx] = fmax(fmin(z, 1e10 * mu / sn), mu / (1e10 * sn));
+            }
+        }
+        NWT_SYNC();
+    }
     for (int i = lane; i < (N + 1) * NX; i += nt) {
         X[i] += alpha * dX[i];
         Lam[i] += alpha * (lamn[i] - Lam[i]);
@@ -831,10 +1016,40 @@ CPDP_GLOBAL void __launch_bounds__(NEWTON_THREADS, CPDP_NEWTON_MINB) k_newton_st
 CPDP_GLOBAL void k_solve_init(SolveArgs a) {
     const size_t tot = (size_t)a.B * (a.N + 1);
     const size_t gs = (size_t)gridDim.x * blockDim.x;
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < tot * NX; i += gs) { a.X[i] = 0.0; a.Lam[i] = 0.0; }
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < tot * NU; i += gs) a.U[i] = 0.0;
+    if constexpr (!HAS_BOUNDS) {
+        for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < tot * NX; i += gs) { a.X[i] = 0.0; a.Lam[i] = 0.0; }
+        for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < tot * NU; i += gs) a.U[i] = 0.0;
+    } else {
+        for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < tot * NX; i += gs) a.Lam[i] = 0.0;
+    }
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < (size_t)a.B; i += gs) {
         a.status[i] = ST_RUNNING; a.iters[i] = 0; a.th_init[i] = 1.0; a.nfilt[i] = 0; a.dlast[i] = 0.0; a.J[i] = 0.0; a.kkt[i] = 0.0;
+    }
+    if constexpr (HAS_BOUNDS) {
+        // IPOPT's start (Waechter & Biegler 2006, §3.6): the zero seed pushed into the interior by bound_push = bound_frac = 1e-2,
+        // z = 1 for every finite bound, mu = 0.1; x0 outside a finite state bound cannot be reached: status CPDP_INFEASIBLE
+        for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < tot * NZ; i += gs) {
+            const int j = (int)(i % NZ);
+            const size_t k = i / NZ;
+            const bool var = (k % (a.N + 1)) < (size_t)a.N || j < NX;           // (row N holds the final state only)
+            const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+            const bool fl = var && bnd_finite(lb), fu = var && bnd_finite(ub);
+            double w = 0.0;
+            const double pl = fl ? (fu ? fmin(1e-2 * fmax(1.0, fabs(lb)), 1e-2 * (ub - lb)) : 1e-2 * fmax(1.0, fabs(lb))) : 0.0;
+            const double pu = fu ? (fl ? fmin(1e-2 * fmax(1.0, fabs(ub)), 1e-2 * (ub - lb)) : 1e-2 * fmax(1.0, fabs(ub))) : 0.0;
+            if (fl && w < lb + pl) w = lb + pl;
+            else if (fu && w > ub - pu) w = ub - pu;
+            if (j < NX) a.X[k * NX + j] = w; else a.U[k * NU + j - NX] = w;
+            a.zL[i] = fl ? 1.0 : 0.0;
+            a.zU[i] = fu ? 1.0 : 0.0;
+        }
+        for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < (size_t)a.B; i += gs) {
+            a.bmu[i] = 0.1;
+            for (int j = 0; j < NX; ++j) {
+                const double v = a.x0[i * NX + j], lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+                if ((bnd_finite(lb) && !(v > lb)) || (bnd_finite(ub) && !(v < ub))) a.status[i] = ST_INFEASIBLE;
+            }
+        }
     }
 }
 

@@ -77,6 +77,7 @@ extern "C" CPDP_API const char* cpdp_error_string(int code) {
             case -8: return "model has per-problem constants but pdata is null";
             case -9: return "phases must be 1, 2 or 3";
             case -10: return "max_iter must be in [0, 255]";
+            case -11: return "the model has no finite bound";
             default: return "invalid argument";
         }
     }

@@ -172,13 +172,42 @@ def rocket_cost1_oc(n_grid=15):
 VARIANTS = {"robotarm_wd": robotarm_wd_oc, "quadrotor_cost1": quadrotor_cost1_oc, "quadrotor_cost2": quadrotor_cost2_oc,
             "rocket_cost1": rocket_cost1_oc}
 
+# ---- box-bounded versions (actuator limits, one joint-speed limit) whose bounds are active at the fixtures' optima ----------
+def pendulum_bounded_oc(n_grid=10):
+    """pendulum_oc with the torque bounded, |u| <= 5 (the unbounded optimum of the fixture reaches 9.95)."""
+    oc = pendulum_oc(n_grid)
+    oc.setControlVariable(oc.env.U, [-5.0], [5.0])
+    oc.lib_name = "pendulum_bounded"
+    return oc
+
+
+def robotarm_bounded_oc(n_grid=30):
+    """robotarm_oc with |u_i| <= 3 and the state bound |dq2| <= 4 (unbounded optimum: torque -5.8, dq2 +-6.2)."""
+    oc = robotarm_oc(n_grid)
+    oc.setStateVariable(oc.env.X, [-1e20, -1e20, -1e20, -4.0], [1e20, 1e20, 1e20, 4.0])
+    oc.setControlVariable(oc.env.U, [-3.0, -3.0], [3.0, 3.0])
+    oc.lib_name = "robotarm_bounded"
+    return oc
+
+
+def quadrotor_bounded_oc(n_grid=25):
+    """quadrotor_oc (goal position per problem) with the rotor thrusts bounded, 1 <= f_i <= 4 (unbounded: 0.54 - 5.88)."""
+    oc = quadrotor_oc(n_grid)
+    oc.setControlVariable(oc.env.U, [1.0] * 4, [4.0] * 4)
+    oc.lib_name = "quadrotor_bounded"
+    return oc
+
+
+BOUNDED = {"pendulum_bounded": pendulum_bounded_oc, "robotarm_bounded": robotarm_bounded_oc,
+           "quadrotor_bounded": quadrotor_bounded_oc}
+
 STANDARD = {"pendulum": pendulum_oc, "pendulum_tw2": pendulum_timewarp_oc, "robotarm": robotarm_oc, "rocket": rocket_oc, "quadrotor": quadrotor_oc,
             "cartpole": cartpole_oc}
 
 
 def build_all(verbose=False):
     libs = {}
-    for name, fn in list(STANDARD.items()) + list(VARIANTS.items()):
+    for name, fn in list(STANDARD.items()) + list(VARIANTS.items()) + list(BOUNDED.items()):
         oc = fn()
         libs[name] = oc.build(name=oc.lib_name, verbose=verbose).path
     return libs
