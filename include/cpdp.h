@@ -102,6 +102,19 @@ int cpdp_aux_phases(void* ws, size_t ws_bytes, int B, int N, int S, double T,
              int W, int D, const int* sel /* host */, const double* taus, int taus_stride, const double* wp,
              double* Xa, double* Ua, double* loss, double* dtheta, int* aux_status, int* counters, void* stream, int phases);
 
+/* Adjoint of mode 2: for cotangents Xbar[B][N+1][n] and Ubar[B][N+1][m] of the trajectory (either may be NULL, meaning zero; not
+ * both), theta_bar[B][r] = sum_k (dX_k/dtheta)' Xbar_k + (dU_k/dtheta)' Ubar_k and x0_bar[B][n] (may be NULL) the same with
+ * respect to x0, the exact derivatives of the discretised problem cpdp_solve solves (mode 2's), by one reverse sweep per problem
+ * instead of r forward columns.  U_N = U_{N-1} (CPDP.py:191), so a cotangent on U_N acts on U_{N-1}.  Self-contained: it runs
+ * mode 2's stage derivatives and backward recursion first (S > 0; bounded models read z_L, z_U, mu from the workspace as mode 2
+ * does: cpdp_set_bound_multipliers).  aux_status[B] as in mode 2 (0 ok, 3 no usable trajectory, 4 Quu not positive definite).
+ * Rows are zero where aux_status != 0 or solve_status (may be NULL) is not CPDP_CONVERGED.  Bit-identical per problem for any
+ * batching.  Same workspace and argument-error codes as cpdp_aux. */
+int cpdp_aux_adjoint(void* ws, size_t ws_bytes, int B, int N, int S, double T,
+                     const double* theta, int theta_stride, const double* pdata,
+                     const double* X, const double* U, const double* Lam, const int* solve_status,
+                     const double* Xbar, const double* Ubar, double* theta_bar, double* x0_bar, int* aux_status, void* stream);
+
 /* FP64 FMA throughput probe used by bench.py for the roofline denominator: one kernel of `blocks` x 256 threads,
  * 8 independent chains of `iters` DFMAs per thread (flops = blocks*256*8*iters*2).  sink: >= 1 device double. */
 int cpdp_dfma_probe(double* sink, int blocks, int iters, void* stream);

@@ -332,11 +332,7 @@ class COCSys:
             wp_d = mem.from_host(wp_h)
         ws = self._workspace(B, sol.get("_slot", 0))
         if lib.has_bounds and int(mode) == COCSys.MODE_DISCRETE and phases & 1:
-            # mode 2 differentiates the barrier-perturbed KKT system: it reads the bound multipliers from the workspace
-            if sol.get("Zl") is None:
-                raise ValueError("mode 2 on a bounded model needs the bound multipliers Zl, Zu, mu of the solution")
-            lib.set_bound_multipliers(mem.ptr(ws), int(ws.shape[0]), B, N, S, mem.ptr(sol["Zl"]), mem.ptr(sol["Zu"]),
-                                      mem.ptr(sol["mu"]), mem.stream())
+            self._set_bound_multipliers(sol, ws)
         if out is None:
             out = dict(Xa=mem.empty((B, N + 1, n * r)), Ua=mem.empty((B, N + 1, m * r)), loss=mem.empty((B,)),
                        dtheta=mem.empty((B, r)), aux_status=mem.zeros((B,), "i4"),
@@ -347,6 +343,44 @@ class COCSys:
                 W, D, sel, mem.ptr(tau_d), tau_stride, mem.ptr(wp_d),
                 mem.ptr(out["Xa"]), mem.ptr(out["Ua"]), mem.ptr(out["loss"]), mem.ptr(out["dtheta"]),
                 mem.ptr(out["aux_status"]), mem.ptr(out["counters"]), mem.stream(), phases=phases)
+        return out
+
+    def _set_bound_multipliers(self, sol, ws):
+        """Mode 2 differentiates the barrier-perturbed KKT system: it reads the bound multipliers from the workspace."""
+        if sol.get("Zl") is None:
+            raise ValueError("mode 2 on a bounded model needs the bound multipliers Zl, Zu, mu of the solution")
+        mem = self._device()
+        self._lib.set_bound_multipliers(mem.ptr(ws), int(ws.shape[0]), sol["B"], self.n_grid, self.steps_per_grid,
+                                        mem.ptr(sol["Zl"]), mem.ptr(sol["Zu"]), mem.ptr(sol["mu"]), mem.stream())
+
+    def auxSysAdjointBatch(self, sol, Xbar=None, Ubar=None):
+        """Adjoint of mode 2: the gradient of a loss l(X, U) of the trajectory with respect to theta and x0, from its cotangents
+        Xbar = dl/dX [B,N+1,n] and Ubar = dl/dU [B,N+1,m] (either may be None, meaning zero), by one reverse sweep per problem
+        (DESIGN.md §3.9).  ``sol`` is the dict returned by cocSolverBatch (or one shaped like it; a bounded model needs its
+        Zl, Zu, mu).  Returns device arrays theta_bar [B,r] (per-problem rows, also for a theta shared by the batch), x0_bar
+        [B,n] and aux_status [B] (as mode 2: 0 ok, 3 no usable trajectory, 4 Quu not positive definite).  Rows are zero for a
+        problem with aux_status != 0 or whose solve did not end `converged`."""
+        if Xbar is None and Ubar is None:
+            raise ValueError("auxSysAdjointBatch needs a cotangent Xbar or Ubar")
+        lib = self.build()
+        mem = self._device()
+        B, N, S = sol["B"], self.n_grid, self.steps_per_grid
+        n, m, r = self.n_state, self.n_control, self.n_auxvar
+        cot = []
+        for v, w in ((Xbar, n), (Ubar, m)):
+            if v is not None:
+                v = mem.from_host(v if hasattr(v, 'data_ptr') else numpy.asarray(v, dtype=float))
+                if tuple(v.shape) != (B, N + 1, w):
+                    raise ValueError("cotangent of shape %s, expected %s" % (tuple(v.shape), (B, N + 1, w)))
+            cot.append(v)
+        ws = self._workspace(B, sol.get("_slot", 0))
+        if lib.has_bounds:
+            self._set_bound_multipliers(sol, ws)
+        out = dict(theta_bar=mem.empty((B, r)), x0_bar=mem.empty((B, n)), aux_status=mem.zeros((B,), "i4"))
+        lib.aux_adjoint(mem.ptr(ws), int(ws.shape[0]), B, N, S, sol["horizon"], mem.ptr(sol["theta"]), sol["theta_stride"],
+                        mem.ptr(sol["pdata"]), mem.ptr(sol["X"]), mem.ptr(sol["U"]), mem.ptr(sol["Lam"]),
+                        mem.ptr(sol.get("status")), mem.ptr(cot[0]), mem.ptr(cot[1]), mem.ptr(out["theta_bar"]),
+                        mem.ptr(out["x0_bar"]), mem.ptr(out["aux_status"]), mem.stream())
         return out
 
     def fp64PeakProbe(self, blocks, iters):

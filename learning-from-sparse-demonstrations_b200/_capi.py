@@ -126,6 +126,8 @@ class CpdpLib:
         L.cpdp_aux.restype = _i
         L.cpdp_aux_phases.argtypes = L.cpdp_aux.argtypes + [_i]
         L.cpdp_aux_phases.restype = _i
+        L.cpdp_aux_adjoint.argtypes = [_vp, _sz, _i, _i, _i, _d, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]
+        L.cpdp_aux_adjoint.restype = _i
         L.cpdp_dfma_probe.argtypes = [_vp, _i, _i, _vp]
         L.cpdp_dfma_probe.restype = _i
         L.cpdp_reduce.argtypes = [_vp, _vp, _i, _vp, _vp, _vp]
@@ -183,6 +185,11 @@ class CpdpLib:
             self.check(self.L.cpdp_aux(*args), "cpdp_aux")
         else:
             self.check(self.L.cpdp_aux_phases(*(args + (phases,))), "cpdp_aux_phases")
+
+    def aux_adjoint(self, ws, ws_bytes, B, N, S, T, theta, theta_stride, pdata, X, U, Lam, solve_status, Xbar, Ubar,
+                    theta_bar, x0_bar, aux_status, stream):
+        self.check(self.L.cpdp_aux_adjoint(ws, ws_bytes, B, N, S, T, theta, theta_stride, pdata, X, U, Lam, solve_status, Xbar,
+                                           Ubar, theta_bar, x0_bar, aux_status, stream), "cpdp_aux_adjoint")
 
     def get_bound_multipliers(self, ws, ws_bytes, B, N, S, Zl, Zu, mu, stream):
         self.check(self.L.cpdp_get_bound_multipliers(ws, ws_bytes, B, N, S, Zl, Zu, mu, stream), "cpdp_get_bound_multipliers")

@@ -1,0 +1,66 @@
+"""torch.autograd layer over the batched solve: ``X, U, info = cpdp_layer(oc, x0, theta, horizon)`` returns the optimal trajectories
+as tensors that any loss written in torch can consume, and ``loss.backward()`` carries its gradient to ``x0`` and ``theta``.
+
+Forward is ``COCSys.cocSolverBatch``; backward is ``COCSys.auxSysAdjointBatch`` (the adjoint of mode 2, DESIGN.md §3.9) on the
+saved solution, so the gradient is the exact derivative of the discretised problem the solver solves.  Problems whose solve did
+not converge, or whose auxiliary system failed (``info["aux_status"]`` != 0 after backward), contribute zero gradient: check
+``info["status"]`` before stepping on it.  Only first derivatives exist (``once_differentiable``)."""
+import torch
+from torch.autograd.function import once_differentiable
+
+__all__ = ["cpdp_layer"]
+
+_SAVED = ("X", "U", "Lam", "status", "theta", "pdata", "Zl", "Zu", "mu")
+
+
+class CpdpSolve(torch.autograd.Function):
+    """(x0 [B,n], theta [r] or [B,r]) -> (X [B,N+1,n], U [B,N+1,m]); the non-differentiable outputs go to ``info``."""
+
+    @staticmethod
+    def forward(ctx, x0, theta, oc, horizon, pdata, rounds, info):
+        sol = oc.cocSolverBatch(x0.detach(), horizon, theta.detach(), pdata=pdata, rounds=rounds)
+        mem = oc._device()
+        info.update({k: sol[k] for k in ("Lam", "status", "iters", "kkt", "cost", "Zl", "Zu", "mu") if k in sol})
+        info["aux_status"] = mem.zeros((sol["B"],), "i4")
+        ctx.oc, ctx.info = oc, info
+        ctx.keep = {k: sol[k] for k in ("B", "horizon", "theta_stride", "_slot")}
+        ctx.saved_keys = [k for k in _SAVED if k in sol]
+        ctx.save_for_backward(*(sol[k] for k in ctx.saved_keys))
+        ctx.shared = theta.dim() == 1
+        ctx.like = ((x0.device, x0.dtype), (theta.device, theta.dtype))
+        ctx.set_materialize_grads(False)
+        X, U = sol["X"], sol["U"]
+        return X, U
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, Xbar, Ubar):
+        oc, info = ctx.oc, ctx.info
+        (x0_dev, x0_dt), (th_dev, th_dt) = ctx.like
+        if Xbar is None and Ubar is None:
+            return None, None, None, None, None, None, None
+        sol = dict(ctx.keep, **dict(zip(ctx.saved_keys, ctx.saved_tensors)))
+        adj = oc.auxSysAdjointBatch(sol, Xbar, Ubar)
+        info["aux_status"].copy_(adj["aux_status"])
+        gx0 = gth = None
+        if ctx.needs_input_grad[0]:
+            gx0 = adj["x0_bar"].to(device=x0_dev, dtype=x0_dt)
+        if ctx.needs_input_grad[1]:
+            tb = adj["theta_bar"]
+            if ctx.shared:
+                # a theta shared by the batch: fixed-tree sum of the per-problem rows (depends on B only, not on timing)
+                tb = oc.reduceRows(tb)
+            gth = tb.to(device=th_dev, dtype=th_dt)
+        return gx0, gth, None, None, None, None, None
+
+
+def cpdp_layer(oc, x0, theta, horizon, pdata=None, rounds=0):
+    """Differentiable batched solve.  x0 [B,n]; theta [r] (shared by the batch) or [B,r]; pdata [B,q] (constants, not
+    differentiable); rounds as in ``cocSolverBatch``.  Returns (X [B,N+1,n], U [B,N+1,m], info) where info holds Lam, status,
+    iters, kkt, cost (and Zl, Zu, mu for a bounded model), and an aux_status tensor that backward fills in place."""
+    if pdata is not None and getattr(pdata, "requires_grad", False):
+        raise NotImplementedError("cpdp_layer differentiates with respect to x0 and theta only: the generated model code has "
+                                  "no derivatives with respect to the per-problem constants pdata")
+    info = {}
+    X, U = CpdpSolve.apply(x0, theta, oc, float(horizon), pdata, int(rounds), info)
+    return X, U, info
