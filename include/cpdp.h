@@ -65,7 +65,25 @@ int cpdp_solve(void* ws, size_t ws_bytes, int B, int N, int S, double T,
                double* X, double* U, double* Lam, int* status, int* iters,
                double* kkt_out, double* cost_out, void* stream);
 
-/* Newton rounds launched by the most recent cpdp_solve of the calling thread (4 kernel launches per round + 2). */
+/* cpdp_solve started from a given trajectory instead of the all-zeros seed (warm start; the Newton iteration itself is the same).
+ *   Xg[B][N+1][n], Ug[B][N+1][m], Lg[B][N+1][n]: the guess, e.g. the outputs of a previous call; they may alias X, U, Lam.
+ *   Zlg, Zug[B][N+1][n+m]: bound multipliers of the guess (bounded models; both or NULL, meaning z = mu_init / slack).
+ *   init_status[B] (may be NULL; may alias status): a problem whose entry is not CPDP_CONVERGED gets cpdp_solve's cold seed.
+ *   shift 0: row k starts from guess row k; shift 1 (receding horizon): from guess row min(k+1, last row), i.e. X, Lam and the
+ *   states' z repeat row N, U and the controls' z row N-1.  Either way X_0 = x0 and U_N = U_{N-1}.
+ *   mu_init > 0: barrier parameter of a warm-started problem (bounded models; ignored otherwise).  A bounded model follows IPOPT's
+ *   warm_start_init_point: the guess is pushed into the interior by 1e-3 (warm_start_bound_push / _frac), z = max(z, 1e-3).
+ * Outputs and per-problem status as cpdp_solve; a converged guess of the same problem ends with iters = 0.  -12: shift not 0 or 1;
+ * -13: mu_init <= 0 on a bounded library. */
+int cpdp_solve_warm(void* ws, size_t ws_bytes, int B, int N, int S, double T,
+                    const double* x0, const double* theta, int theta_stride, const double* pdata,
+                    double tol, int max_iter, int rounds,
+                    double* X, double* U, double* Lam, int* status, int* iters,
+                    double* kkt_out, double* cost_out, void* stream,
+                    const double* Xg, const double* Ug, const double* Lg, const double* Zlg, const double* Zug,
+                    const int* init_status, int shift, double mu_init);
+
+/* Newton rounds launched by the most recent cpdp_solve or cpdp_solve_warm of the calling thread (4 kernel launches per round + 2). */
 int cpdp_last_rounds(void);
 
 /* Replaces COCSys.auxSysSolver (CPDP.py:301-381) and the getloss_*corrections closures

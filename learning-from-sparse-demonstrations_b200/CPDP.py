@@ -75,6 +75,8 @@ class COCSys:
     MODE_RK45 = 0     # explicit Dormand-Prince with tolerance knobs (what COCSys_TimeVarying uses, CPDP.py:740)
     MODE_BDF = 1      # scheme of the as-shipped COCSys (CPDP.py:335): scipy-style BDF at default tolerances
     MODE_DISCRETE = 2  # exact derivative of the discretised problem the solver solves (DESIGN.md §3.7); tolerances unused
+    # barrier parameter a warm start of a bounded model begins with (mu_init of cocSolverBatch; DESIGN.md §3.10)
+    WARM_MU_INIT = 1e-8
 
     def __init__(self, project_name="myOc"):
         self.sys_name = project_name
@@ -90,6 +92,7 @@ class COCSys:
         self.aux_mode = COCSys.MODE_BDF
         self.rtol_back, self.atol_back = 1e-3, 1e-6      # scipy defaults (bdf.py:198, rk.py:85)
         self.rtol_fwd, self.atol_fwd = 1e-3, 1e-6
+        self.warm_mu_init = COCSys.WARM_MU_INIT
 
     # ------------------------------------------------------------------ problem definition
     def setAuxvarVariable(self, auxvar=None):
@@ -262,11 +265,17 @@ class COCSys:
         assert tuple(th.shape) == (B, self.n_auxvar)
         return mem.from_host(th), self.n_auxvar
 
-    def cocSolverBatch(self, ini_states, horizon, auxvar_value, pdata=None, rounds=0, _slot=0):
+    def cocSolverBatch(self, ini_states, horizon, auxvar_value, pdata=None, rounds=0, init=None, shift=0, mu_init=None, _slot=0):
         """Batched cocSolver: ini_states [B,n]; auxvar_value [r] (shared) or [B,r]; pdata [B,q].
         Returns a dict of device arrays X [B,N+1,n], U [B,N+1,m], Lam [B,N+1,n], status, iters, kkt, cost
         and the host time_grid; a bounded model adds the bound multipliers Zl, Zu [B,N+1,n+m] (row N: the final state's) and
-        the final barrier parameter mu [B]."""
+        the final barrier parameter mu [B].
+
+        Warm start (DESIGN.md §3.10): ``init`` is a mapping with X, U, Lam and optionally Zl, Zu, status -- the dict this method
+        returns qualifies -- and Newton starts from it instead of the zero seed (tensors are used detached).  Problems whose
+        ``init["status"]`` is not `converged` start cold.  shift=1 starts row k from row k+1 of the guess (receding horizon).  A
+        bounded model starts a warm problem's barrier parameter at ``mu_init`` (default ``warm_mu_init``; an ``init["mu"]`` is
+        not used).  init=None is the cold solve."""
         self._assert_defined()
         if not hasattr(self, 'n_grid'):
             self.setIntegrator()
@@ -286,10 +295,16 @@ class COCSys:
         out = dict(X=mem.empty((B, N + 1, self.n_state)), U=mem.empty((B, N + 1, self.n_control)),
                    Lam=mem.empty((B, N + 1, self.n_state)), status=mem.empty((B,), "i4"), iters=mem.empty((B,), "i4"),
                    kkt=mem.empty((B,)), cost=mem.empty((B,)))
-        lib.solve(mem.ptr(ws), int(ws.shape[0]), B, N, S, float(horizon), mem.ptr(x0), mem.ptr(th), th_stride, mem.ptr(pd),
-                  float(self.tol), int(self.max_iter), int(rounds),
-                  mem.ptr(out["X"]), mem.ptr(out["U"]), mem.ptr(out["Lam"]), mem.ptr(out["status"]), mem.ptr(out["iters"]),
-                  mem.ptr(out["kkt"]), mem.ptr(out["cost"]), mem.stream())
+        args = (mem.ptr(ws), int(ws.shape[0]), B, N, S, float(horizon), mem.ptr(x0), mem.ptr(th), th_stride, mem.ptr(pd),
+                float(self.tol), int(self.max_iter), int(rounds),
+                mem.ptr(out["X"]), mem.ptr(out["U"]), mem.ptr(out["Lam"]), mem.ptr(out["status"]), mem.ptr(out["iters"]),
+                mem.ptr(out["kkt"]), mem.ptr(out["cost"]), mem.stream())
+        if init is None:
+            lib.solve(*args)
+        else:
+            g = self._warm_guess(init, B, N)
+            lib.solve_warm(*args, *(mem.ptr(g[k]) for k in ("X", "U", "Lam", "Zl", "Zu", "status")), int(shift),
+                           float(self.warm_mu_init if mu_init is None else mu_init))
         if lib.has_bounds:
             nz = self.n_state + self.n_control
             out.update(Zl=mem.empty((B, N + 1, nz)), Zu=mem.empty((B, N + 1, nz)), mu=mem.empty((B,)))
@@ -298,6 +313,27 @@ class COCSys:
         out.update(time_grid=self._time_grid(horizon, N), horizon=float(horizon),
                    theta=th, theta_stride=th_stride, pdata=pd, B=B, x0=x0, _slot=_slot)
         return out
+
+    def _warm_guess(self, init, B, N):
+        """Device arrays of a warm-start mapping (shapes checked; tensors detached)."""
+        mem = self._device()
+        nz = self.n_state + self.n_control
+        shapes = dict(X=(B, N + 1, self.n_state), U=(B, N + 1, self.n_control), Lam=(B, N + 1, self.n_state),
+                      Zl=(B, N + 1, nz), Zu=(B, N + 1, nz), status=(B,))
+        g = {}
+        for k, shp in shapes.items():
+            v = init.get(k) if k in ("Zl", "Zu", "status") else init[k]
+            if v is None or (k in ("Zl", "Zu") and not self._lib.has_bounds):
+                g[k] = None
+                continue
+            v = v.detach() if hasattr(v, "detach") else numpy.asarray(v)
+            v = mem.from_host(v, "i4" if k == "status" else "f8")
+            if tuple(v.shape) != shp:
+                raise ValueError("init[%r] has shape %s, expected %s" % (k, tuple(v.shape), shp))
+            g[k] = v
+        if (g["Zl"] is None) != (g["Zu"] is None):
+            raise ValueError("init needs both Zl and Zu, or neither")
+        return g
 
     @staticmethod
     def _time_grid(horizon, N):
@@ -430,7 +466,7 @@ class COCSys:
         return out
 
     def gradIterBatch(self, ini_states, horizon, auxvar_value, taus, waypoints, sel, pdata=None, mode=None, rounds=0,
-                      chunks=1):
+                      chunks=1, init=None, shift=0):
         """One CPDP gradient iteration for a batch: forward solve, auxiliary system, loss and dL/dtheta, and their
         fixed-order sums.  Returns (sum_loss_and_grad [1+r] device array, sol dict, aux dict).  ``aux["n_failed"]`` is a
         one-element device array (no host synchronisation): the number of OCPs whose forward solve did not end `converged`
@@ -441,10 +477,12 @@ class COCSys:
         contiguous chunks, each running solve -> backward sweep -> forward sweep on its own CUDA stream with its own
         workspace, so that the under-filled tails of one chunk's kernels (last Newton rounds, last wave of the sweeps)
         overlap the other chunk's work.  Per-problem results do not depend on the chunking and the reduction tree is
-        over the whole batch, so the result is bit-identical to chunks=1 (measured: 288 -> 274 ms for 4096 OCPs)."""
+        over the whole batch, so the result is bit-identical to chunks=1 (measured: 288 -> 274 ms for 4096 OCPs).
+
+        init, shift: warm start of the forward solve (cocSolverBatch); with chunks > 1 ``init`` is cut along the same bounds."""
         mem = self._device()
         if chunks <= 1 or not hasattr(mem, "torch"):
-            sol = self.cocSolverBatch(ini_states, horizon, auxvar_value, pdata=pdata, rounds=rounds)
+            sol = self.cocSolverBatch(ini_states, horizon, auxvar_value, pdata=pdata, rounds=rounds, init=init, shift=shift)
             aux = self.auxSysSolverBatch(sol, taus, waypoints, sel, mode=mode)
             full = self.reduceRows(self.packRows(sol, aux))
             aux["n_failed"] = full[1 + self.n_auxvar:]
@@ -473,8 +511,11 @@ class COCSys:
             st = streams[c]
             st.wait_stream(main)
             with torch.cuda.stream(st):
+                ini = None if init is None else {k: v[lo:hi] for k, v in init.items()
+                                                 if k in ("X", "U", "Lam", "Zl", "Zu", "status") and v is not None}
                 sol = self.cocSolverBatch(x0[lo:hi], horizon, th[lo:hi] if th.ndim == 2 else th,
-                                          pdata=None if pd is None else pd[lo:hi], rounds=rounds, _slot=c + 1)
+                                          pdata=None if pd is None else pd[lo:hi], rounds=rounds, init=ini, shift=shift,
+                                          _slot=c + 1)
                 aux = self.auxSysSolverBatch(sol, t_h[lo:hi] if t_h.ndim == 2 else t_h, wp[lo:hi], sel, mode=mode)
             sols.append(sol)
             auxs.append(aux)

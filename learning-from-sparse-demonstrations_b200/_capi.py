@@ -120,6 +120,8 @@ class CpdpLib:
         L.cpdp_solve.argtypes = [_vp, _sz, _i, _i, _i, _d, _vp, _vp, _i, _vp, _d, _i, _i,
                                  _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]
         L.cpdp_solve.restype = _i
+        L.cpdp_solve_warm.argtypes = L.cpdp_solve.argtypes + [_vp, _vp, _vp, _vp, _vp, _vp, _i, _d]
+        L.cpdp_solve_warm.restype = _i
         L.cpdp_aux.argtypes = [_vp, _sz, _i, _i, _i, _d, _vp, _i, _vp, _vp, _vp, _vp, _vp,
                                _i, _d, _d, _d, _d, _i, _i, ctypes.POINTER(_i), _vp, _i, _vp,
                                _vp, _vp, _vp, _vp, _vp, _vp, _vp]
@@ -173,6 +175,12 @@ class CpdpLib:
               X, U, Lam, status, iters, kkt, cost, stream):
         self.check(self.L.cpdp_solve(ws, ws_bytes, B, N, S, T, x0, theta, theta_stride, pdata, tol, max_iter, rounds,
                                      X, U, Lam, status, iters, kkt, cost, stream), "cpdp_solve")
+
+    def solve_warm(self, ws, ws_bytes, B, N, S, T, x0, theta, theta_stride, pdata, tol, max_iter, rounds,
+                   X, U, Lam, status, iters, kkt, cost, stream, Xg, Ug, Lg, Zlg, Zug, init_status, shift, mu_init):
+        self.check(self.L.cpdp_solve_warm(ws, ws_bytes, B, N, S, T, x0, theta, theta_stride, pdata, tol, max_iter, rounds,
+                                          X, U, Lam, status, iters, kkt, cost, stream, Xg, Ug, Lg, Zlg, Zug, init_status, shift,
+                                          mu_init), "cpdp_solve_warm")
 
     def aux(self, ws, ws_bytes, B, N, S, T, theta, theta_stride, pdata, X, U, Lam, solve_status,
             mode, rtol_b, atol_b, rtol_f, atol_f, W, D, sel, taus, taus_stride, wp,

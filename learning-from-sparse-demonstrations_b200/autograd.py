@@ -17,8 +17,8 @@ class CpdpSolve(torch.autograd.Function):
     """(x0 [B,n], theta [r] or [B,r]) -> (X [B,N+1,n], U [B,N+1,m]); the non-differentiable outputs go to ``info``."""
 
     @staticmethod
-    def forward(ctx, x0, theta, oc, horizon, pdata, rounds, info):
-        sol = oc.cocSolverBatch(x0.detach(), horizon, theta.detach(), pdata=pdata, rounds=rounds)
+    def forward(ctx, x0, theta, oc, horizon, pdata, rounds, info, init, shift):
+        sol = oc.cocSolverBatch(x0.detach(), horizon, theta.detach(), pdata=pdata, rounds=rounds, init=init, shift=shift)
         mem = oc._device()
         info.update({k: sol[k] for k in ("Lam", "status", "iters", "kkt", "cost", "Zl", "Zu", "mu") if k in sol})
         info["aux_status"] = mem.zeros((sol["B"],), "i4")
@@ -38,7 +38,7 @@ class CpdpSolve(torch.autograd.Function):
         oc, info = ctx.oc, ctx.info
         (x0_dev, x0_dt), (th_dev, th_dt) = ctx.like
         if Xbar is None and Ubar is None:
-            return None, None, None, None, None, None, None
+            return None, None, None, None, None, None, None, None, None
         sol = dict(ctx.keep, **dict(zip(ctx.saved_keys, ctx.saved_tensors)))
         adj = oc.auxSysAdjointBatch(sol, Xbar, Ubar)
         info["aux_status"].copy_(adj["aux_status"])
@@ -51,16 +51,19 @@ class CpdpSolve(torch.autograd.Function):
                 # a theta shared by the batch: fixed-tree sum of the per-problem rows (depends on B only, not on timing)
                 tb = oc.reduceRows(tb)
             gth = tb.to(device=th_dev, dtype=th_dt)
-        return gx0, gth, None, None, None, None, None
+        return gx0, gth, None, None, None, None, None, None, None
 
 
-def cpdp_layer(oc, x0, theta, horizon, pdata=None, rounds=0):
+def cpdp_layer(oc, x0, theta, horizon, pdata=None, rounds=0, init=None, shift=0):
     """Differentiable batched solve.  x0 [B,n]; theta [r] (shared by the batch) or [B,r]; pdata [B,q] (constants, not
     differentiable); rounds as in ``cocSolverBatch``.  Returns (X [B,N+1,n], U [B,N+1,m], info) where info holds Lam, status,
-    iters, kkt, cost (and Zl, Zu, mu for a bounded model), and an aux_status tensor that backward fills in place."""
+    iters, kkt, cost (and Zl, Zu, mu for a bounded model), and an aux_status tensor that backward fills in place.
+
+    init, shift: warm start of the solve as in ``cocSolverBatch``, e.g. ``init=dict(info, X=X, U=U)`` of the previous call.  It is
+    not differentiated: the converged point does not depend on where the solve started, beyond the solver tolerance."""
     if pdata is not None and getattr(pdata, "requires_grad", False):
         raise NotImplementedError("cpdp_layer differentiates with respect to x0 and theta only: the generated model code has "
                                   "no derivatives with respect to the per-problem constants pdata")
     info = {}
-    X, U = CpdpSolve.apply(x0, theta, oc, float(horizon), pdata, int(rounds), info)
+    X, U = CpdpSolve.apply(x0, theta, oc, float(horizon), pdata, int(rounds), info, init, int(shift))
     return X, U, info

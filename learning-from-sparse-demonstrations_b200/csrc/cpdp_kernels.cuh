@@ -1012,6 +1012,44 @@ CPDP_GLOBAL void __launch_bounds__(NEWTON_THREADS, CPDP_NEWTON_MINB) k_newton_st
     }
 }
 
+// ---- starting point of the solve: the cold seed of k_solve_init and the pieces k_solve_init_warm (cpdp_warm.cuh) shares with it
+constexpr double MU_COLD = 0.1;        // IPOPT's mu_init: barrier parameter of the cold start
+constexpr double COLD_PUSH = 1e-2;     // IPOPT's bound_push = bound_frac of the cold start
+
+// Per-problem solver state of a fresh solve (both starts).
+CPDP_HD void start_state(const SolveArgs& a, size_t i) {
+    a.status[i] = ST_RUNNING; a.iters[i] = 0; a.th_init[i] = 1.0; a.nfilt[i] = 0; a.dlast[i] = 0.0; a.J[i] = 0.0; a.kkt[i] = 0.0;
+}
+
+// IPOPT's projection of value w into the interior of its bounds lb, ub (fl, fu: the bound is finite and applies), with
+// bound_push = bound_frac = kappa (Waechter & Biegler 2006, §3.6).
+CPDP_HD double bnd_push(double lb, double ub, bool fl, bool fu, double w, double kappa) {
+    const double pl = fl ? (fu ? fmin(kappa * fmax(1.0, fabs(lb)), kappa * (ub - lb)) : kappa * fmax(1.0, fabs(lb))) : 0.0;
+    const double pu = fu ? (fl ? fmin(kappa * fmax(1.0, fabs(ub)), kappa * (ub - lb)) : kappa * fmax(1.0, fabs(ub))) : 0.0;
+    if (fl && w < lb + pl) w = lb + pl;
+    else if (fu && w > ub - pu) w = ub - pu;
+    return w;
+}
+
+// Cold seed of component j of z = [x; u] in a row where it is a variable (var; row N holds the final state only): the zero seed
+// (CPDP.py:139,155,167) pushed into the interior by bound_push = bound_frac = 1e-2, and z = 1 for every finite bound (0 else).
+// k_solve_init spells out the same three statements: routing its stores through this helper changes its generated code.
+CPDP_HD void cold_seed(int j, bool var, double& w, double& zl, double& zu) {
+    const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+    const bool fl = var && bnd_finite(lb), fu = var && bnd_finite(ub);
+    w = bnd_push(lb, ub, fl, fu, 0.0, COLD_PUSH);
+    zl = fl ? 1.0 : 0.0;
+    zu = fu ? 1.0 : 0.0;
+}
+
+// x0 outside a finite state bound cannot be reached: status CPDP_INFEASIBLE (both starts).
+CPDP_HD void check_x0(const SolveArgs& a, size_t i) {
+    for (int j = 0; j < NX; ++j) {
+        const double v = a.x0[i * NX + j], lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+        if ((bnd_finite(lb) && !(v > lb)) || (bnd_finite(ub) && !(v < ub))) a.status[i] = ST_INFEASIBLE;
+    }
+}
+
 // k_solve_init: zero seed (CPDP.py:139,155,167), multipliers 0, per-problem solver state.
 CPDP_GLOBAL void k_solve_init(SolveArgs a) {
     const size_t tot = (size_t)a.B * (a.N + 1);
@@ -1022,33 +1060,23 @@ CPDP_GLOBAL void k_solve_init(SolveArgs a) {
     } else {
         for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < tot * NX; i += gs) a.Lam[i] = 0.0;
     }
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < (size_t)a.B; i += gs) {
-        a.status[i] = ST_RUNNING; a.iters[i] = 0; a.th_init[i] = 1.0; a.nfilt[i] = 0; a.dlast[i] = 0.0; a.J[i] = 0.0; a.kkt[i] = 0.0;
-    }
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < (size_t)a.B; i += gs) start_state(a, i);
     if constexpr (HAS_BOUNDS) {
-        // IPOPT's start (Waechter & Biegler 2006, §3.6): the zero seed pushed into the interior by bound_push = bound_frac = 1e-2,
-        // z = 1 for every finite bound, mu = 0.1; x0 outside a finite state bound cannot be reached: status CPDP_INFEASIBLE
+        // IPOPT's start (Waechter & Biegler 2006, §3.6): cold_seed, mu = 0.1, check_x0
         for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < tot * NZ; i += gs) {
             const int j = (int)(i % NZ);
             const size_t k = i / NZ;
             const bool var = (k % (a.N + 1)) < (size_t)a.N || j < NX;           // (row N holds the final state only)
             const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
             const bool fl = var && bnd_finite(lb), fu = var && bnd_finite(ub);
-            double w = 0.0;
-            const double pl = fl ? (fu ? fmin(1e-2 * fmax(1.0, fabs(lb)), 1e-2 * (ub - lb)) : 1e-2 * fmax(1.0, fabs(lb))) : 0.0;
-            const double pu = fu ? (fl ? fmin(1e-2 * fmax(1.0, fabs(ub)), 1e-2 * (ub - lb)) : 1e-2 * fmax(1.0, fabs(ub))) : 0.0;
-            if (fl && w < lb + pl) w = lb + pl;
-            else if (fu && w > ub - pu) w = ub - pu;
+            const double w = bnd_push(lb, ub, fl, fu, 0.0, COLD_PUSH);
             if (j < NX) a.X[k * NX + j] = w; else a.U[k * NU + j - NX] = w;
             a.zL[i] = fl ? 1.0 : 0.0;
             a.zU[i] = fu ? 1.0 : 0.0;
         }
         for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < (size_t)a.B; i += gs) {
-            a.bmu[i] = 0.1;
-            for (int j = 0; j < NX; ++j) {
-                const double v = a.x0[i * NX + j], lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
-                if ((bnd_finite(lb) && !(v > lb)) || (bnd_finite(ub) && !(v < ub))) a.status[i] = ST_INFEASIBLE;
-            }
+            a.bmu[i] = MU_COLD;
+            check_x0(a, i);
         }
     }
 }

@@ -78,6 +78,8 @@ extern "C" CPDP_API const char* cpdp_error_string(int code) {
             case -9: return "phases must be 1, 2 or 3";
             case -10: return "max_iter must be in [0, 255]";
             case -11: return "the model has no finite bound";
+            case -12: return "shift must be 0 or 1";
+            case -13: return "mu_init must be > 0 on a bounded model";
             default: return "invalid argument";
         }
     }

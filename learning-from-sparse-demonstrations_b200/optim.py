@@ -155,12 +155,17 @@ class DeviceLearner:
 
     Difference from the reference, stated: once the stop rule fires the remaining launches of the run are no-ops on the
     parameter (the stream cannot `break`); ``check_every`` > 0 makes the host poll the stop flag every that many iterations
-    and leave early."""
+    and leave early.
 
-    def __init__(self, oc, ini_states, horizon, taus, waypoints, sel, pdata=None, mode=None, rounds=0, chunks=1):
+    warm_start=True: every evaluation after the first starts its forward solve from the previous evaluation's solution (kept on
+    the device; with Nesterov's second evaluation, the last solve of either kind), and a problem whose previous solve did not
+    converge starts cold (``COCSys.cocSolverBatch(init=...)``, DESIGN.md §3.10)."""
+
+    def __init__(self, oc, ini_states, horizon, taus, waypoints, sel, pdata=None, mode=None, rounds=0, chunks=1, warm_start=False):
         self.oc = oc
         self.args = (ini_states, horizon, taus, waypoints, sel)
         self.kw = dict(pdata=pdata, mode=mode, rounds=rounds, chunks=chunks)
+        self.warm_start = bool(warm_start)
         self.n_auxvar = oc.n_auxvar
         self.loss_trace = []
         self.parameter_trace = []
@@ -206,9 +211,13 @@ class DeviceLearner:
             lib.optim_step(phase, *hyper, mem.ptr(theta), mem.ptr(theta_eval), mem.ptr(state), mem.ptr(red), mem.ptr(it),
                            mem.ptr(loss_trace), mem.ptr(ptrace), cap, defer, mem.stream())
 
+        prev = {}
+
         def evaluate():
-            full, sol, aux = oc.gradIterBatch(x0, horizon, theta_eval.reshape(r), taus, wp, sel, **self.kw)
+            full, sol, aux = oc.gradIterBatch(x0, horizon, theta_eval.reshape(r), taus, wp, sel, init=prev.get("sol"), **self.kw)
             failed.__iadd__(aux["n_failed"])
+            if self.warm_start:
+                prev["sol"] = sol
             return full
 
         for j in range(cap):
