@@ -61,6 +61,11 @@ constexpr int BDF_WS_DOUBLES = BDF_NROWS * NX * NC;      // differences array of
 #define CPDP_BDF_EIG_KAPPA 1e4
 #endif
 constexpr double BDF_EIG_KAPPA = CPDP_BDF_EIG_KAPPA;
+// Warm start of the eigen path (bdf_eig_refine): a Jacobian that follows one on the eigen path first refines the previous
+// eigenbasis and runs bdf_schur only when that is rejected; 0 compiles the refinement out (every Jacobian runs bdf_schur).
+#ifndef CPDP_BDF_EIG_WARM
+#define CPDP_BDF_EIG_WARM 1
+#endif
 #ifdef __CUDACC__
 #define BDF_SYNC() __syncwarp()
 #define BDF_UNROLL _Pragma("unroll")
@@ -116,7 +121,7 @@ constexpr int FLAG = RU + 128;                   // 4 ints: prepare ok | Schur o
 constexpr int NODE = FLAG + 2;                   // the two node rows (x, u, lambda) bracketing the current grid interval
 constexpr int NODE_W = 2 * NX + NU;
 #ifdef CPDP_BDF_TIMING
-constexpr int TS = NODE + ((2 * NODE_W + 1) & ~1);   // developer timing build: Schur sub-phase clocks (8)
+constexpr int TS = NODE + ((2 * NODE_W + 1) & ~1);   // developer timing build: Schur sub-phase clocks (8; 6: warm refinement)
 constexpr int END = TS + 8;
 #else
 constexpr int END = NODE + ((2 * NODE_W + 1) & ~1);
@@ -186,14 +191,17 @@ CPDP_D double bdf_rcp(double x) {
 #define BDF_TS(i)
 #endif
 // Developer path counts (-DCPDP_BDF_PATH_COUNTS, implied by the timing build): Newton solves on the eigen path | on the
-// sweep, Jacobians on the eigen path | on the sweep, written over Ua[24..27] of the problem at kernel end.
+// sweep, Jacobians on the eigen path | on the sweep, Jacobians whose warm refinement was accepted | rejected, written over
+// Ua[24..29] of the problem at kernel end.
 #ifdef CPDP_BDF_TIMING
 #define CPDP_BDF_PATH_COUNTS
 #endif
 #ifdef CPDP_BDF_PATH_COUNTS
 #define BDF_PATH(sm, k) do { cnt[4 + (k) + ((BDF_EIG_KAPPA > 0.0 && ((const int*)((sm) + bo::FLAG))[3]) ? 0 : 1)] += 1; } while (0)
+#define BDF_WARM(dk) do { cnt[8] += (dk) == 2; cnt[9] += (dk) == 3; } while (0)
 #else
 #define BDF_PATH(sm, k) do { } while (0)
+#define BDF_WARM(dk) do { } while (0)
 #endif
 
 // THE product of the hot loop, one out-of-line instance:  dst[(i0 + i) * ds] = sum_k AT[k][i0 + i] x[k * xs],  i < NH.
@@ -912,15 +920,48 @@ CPDP_D bool bdf_factor_eig(double* sm, const double c) {
     return !bdf_ballot(sm, bad != 0.0);
 }
 
-// scipy's "LU" event for a new c: the Lyapunov pivots of the sweep and (I + c L)^{-1} by Gauss-Jordan elimination with partial
-// pivoting on [I + cL | I]: lane c < n owns column c of the left half, lane 16 + c column c of the right half.
-CPDP_D_NOINLINE bool bdf_factor(const double c) {
+// A^{-1} by Gauss-Jordan elimination with partial pivoting on [A | I]: lane c < n owns column c of the left half (A in XA,
+// written by the caller), lane 16 + c column c of the right half (XB).  Out: dstT[k][i] = A^{-1}[i][k] (row stride QS), XA
+// and XB overwritten.  False (uniformly, dstT untouched) when a pivot column is zero.
+CPDP_D_NOINLINE bool bdf_gauss_jordan(double* dstT) {
     BDF_SM();
     constexpr int n = NX;
     const int lane = threadIdx.x;
     const bool isP = lane < n, isB = (lane >= 16) && (lane < 16 + n);
-    const double* TD = sm + bo::TD;
     double* XA = sm + bo::XA; double* XB = sm + bo::XB;
+    if (isB) { BDF_UNROLL for (int i = 0; i < n; ++i) XB[i * NCS + lane - 16] = (i == lane - 16) ? 1.0 : 0.0; }
+    double* mine = isP ? XA + lane : XB + (isB ? lane - 16 : 0);
+    const bool own = isP || isB;
+    BDF_SYNC();
+    CPDP_LOOP for (int k = 0; k < n; ++k) {
+        const int p = bdf_argmax(sm, (isP && lane >= k) ? XA[lane * NCS + k] : 0.0, isP && lane >= k);     // lane = candidate row
+        if (p < 0) return false;                                 // (uniform)
+        if (own && p != k) { const double a = mine[k * NCS], b = mine[p * NCS]; mine[k * NCS] = b; mine[p * NCS] = a; }
+        BDF_SYNC();
+        double ak[n];
+        BDF_UNROLL for (int i = 0; i < n; ++i) ak[i] = XA[i * NCS + k];
+        const double ip = bdf_rcp(XA[k * NCS + k]);              // (either sign; the argmax above made it the largest of its column)
+        BDF_SYNC();
+        if (own) {
+            const double t = mine[k * NCS] * ip;
+            BDF_UNROLL for (int i = 0; i < n; ++i) mine[i * NCS] -= ak[i] * t;
+            mine[k * NCS] = t;                                   // (row k itself: the scaled pivot row)
+        }
+        BDF_SYNC();
+    }
+    if (isB) { BDF_UNROLL for (int i = 0; i < n; ++i) dstT[(lane - 16) * QS + i] = XB[i * NCS + lane - 16]; }
+    BDF_SYNC();
+    return true;
+}
+
+// scipy's "LU" event for a new c: the Lyapunov pivots of the sweep and (I + c L)^{-1} by Gauss-Jordan elimination on [I + cL | I]
+CPDP_D_NOINLINE bool bdf_factor(const double c) {
+    BDF_SM();
+    constexpr int n = NX;
+    const int lane = threadIdx.x;
+    const bool isP = lane < n;
+    const double* TD = sm + bo::TD;
+    double* XA = sm + bo::XA;
     if (BDF_EIG_KAPPA > 0.0 && ((const int*)(sm + bo::FLAG))[3]) return bdf_factor_eig(sm, c);
     BDF_SYNC();
     double bad = 0.0;
@@ -936,33 +977,136 @@ CPDP_D_NOINLINE bool bdf_factor(const double c) {
             BDF_ST2(sm + bo::PV + 2 * (i * n + j), er * ie, -ei * ie);
         }
         BDF_UNROLL for (int i = 0; i < n; ++i) XA[i * NCS + j] = ((i == j) ? 1.0 : 0.0) + c * sm[bo::LM + i * n + j];
-    } else if (isB) {
-        BDF_UNROLL for (int i = 0; i < n; ++i) XB[i * NCS + lane - 16] = (i == lane - 16) ? 1.0 : 0.0;
     }
-    double* mine = isP ? XA + lane : XB + (isB ? lane - 16 : 0);
-    const bool own = isP || isB;
-    BDF_SYNC();
-    CPDP_LOOP for (int k = 0; k < n; ++k) {
-        const int p = bdf_argmax(sm, (isP && lane >= k) ? XA[lane * NCS + k] : 0.0, isP && lane >= k);     // lane = candidate row
-        if (p < 0) { bad = 1.0; break; }                         // (uniform)
-        if (own && p != k) { const double a = mine[k * NCS], b = mine[p * NCS]; mine[k * NCS] = b; mine[p * NCS] = a; }
-        BDF_SYNC();
-        double ak[n];
-        BDF_UNROLL for (int i = 0; i < n; ++i) ak[i] = XA[i * NCS + k];
-        const double ip = bdf_rcp(XA[k * NCS + k]);              // (either sign; the argmax above made it the largest of its column)
-        BDF_SYNC();
-        if (own) {
-            const double t = mine[k * NCS] * ip;
-            BDF_UNROLL for (int i = 0; i < n; ++i) mine[i * NCS] -= ak[i] * t;
-            mine[k * NCS] = t;                                   // (row k itself: the scaled pivot row)
-        }
-        BDF_SYNC();
-    }
-    if (bdf_ballot(sm, bad != 0.0)) return false;
-    if (isB) { BDF_UNROLL for (int i = 0; i < n; ++i) sm[bo::WT + (lane - 16) * QS + i] = XB[i * NCS + lane - 16]; }     // WT[k][i] = Winv[i][k]
-    BDF_SYNC();
-    return true;
+    if (!bdf_gauss_jordan(sm + bo::WT)) return false;           // WT[k][i] = Winv[i][k]
+    return !bdf_ballot(sm, bad != 0.0);
 }
+
+// Warm start of the eigen path: L = G D H (H = G^{-1}, D real block diagonal as bdf_eig_basis leaves it) from the previous
+// Jacobian's G, by Newton refinement of the similarity instead of a new Schur form.  One step:
+//   H = G^{-1} (bdf_gauss_jordan),  M = H L G,  D = the part of M's diagonal blocks that commutes with the rotation
+//   generator J = [[0, 1], [-1, 0]] (a = mean of the diagonal, b = (m01 - m10) / 2), and F from  D_I F_IJ - F_IJ D_J = -M_IJ
+//   on every block pair: the parts of M_IJ that commute / anticommute with J are scaled by 1 / (l_I - l_J) and
+//   1 / (l_I - conj l_J) (l = a + ib), which gives every entry as  F_ij = -(k1 M_ij + k2 M_pi,j + k3 M_i,pj + k4 M_pi,pj)
+//   (p: partner index, s = +1 / -1 for the first / second index of a pair, 0 for a real eigenvalue):
+//     k1 = Re(w+ + w-) / 2,  k2 = s_i Im(w+ + w-) / 2,  k3 = s_j Im(w- - w+) / 2,  k4 = s_i s_j Re(w+ - w-) / 2
+//   with w+ = 1 / (l_I - l_J) (0 inside a block: its commuting part is D's) and w- = 1 / (l_I - conj l_J) (0 for a real
+//   diagonal entry);  then G <- G + G F.
+// The columns of G are first scaled by powers of two (exact; both columns of a pair by one factor) to unit norm within a factor
+// of two.  Accepted when ||M - D||_F <= BDF_REFINE_TOL ||L||_F and ||G||_F ||H||_F <= CPDP_BDF_EIG_KAPPA (the cold path's
+// conditions), with every pair still complex (b > 0); rejected, uniformly, when a step has max |F| > BDF_REFINE_FMAX or a
+// non-finite F, or after BDF_REFINE_STEPS steps.  On accept H' (Q), G' (QT) and TD hold what bdf_eig_basis leaves there; the
+// pair structure (ROT's partner row) is the previous Jacobian's.  On reject Q, QT, TD are garbage: bdf_schur rebuilds them from LM.
+// Scratch: L' in PV, the products in XA / XB.
+constexpr int BDF_REFINE_STEPS = 5;
+constexpr double BDF_REFINE_FMAX = 0.5;
+#ifndef CPDP_BDF_REFINE_TOL
+#define CPDP_BDF_REFINE_TOL 1e-13     // the cold path's own ||H L G - D||_F / ||L||_F reaches 6.5e-14 on the quadrotor fixtures
+#endif
+constexpr double BDF_REFINE_TOL = CPDP_BDF_REFINE_TOL;
+CPDP_D_NOINLINE bool bdf_eig_refine() {
+    BDF_SM();
+    constexpr int n = NX;
+    const int lane = threadIdx.x;
+    const bool own = lane < n;
+    const int j = own ? lane : 0;
+    double* G = sm + bo::QT;                                           // G[i][k] = G[k * QS + i]: k-major operand of G x
+    double* LT = sm + bo::PV;                                          // L[i][k] = LT[k * QS + i]
+    double* XA = sm + bo::XA; double* XB = sm + bo::XB;
+    const double* part = sm + bo::ROT + 3 * n;
+    BDF_SYNC();
+    const int pj = (int)part[j];
+    const double sj = (pj > j) ? 1.0 : ((pj < j) ? -1.0 : 0.0);
+    double nl = 0.0, s2 = 0.0;
+    if (own) {
+        CPDP_LOOP for (int i = 0; i < n; ++i) {
+            const double v = sm[bo::LM + i * n + j], g = G[j * QS + i], gp = G[pj * QS + i];
+            LT[j * QS + i] = v;
+            nl += v * v;
+            s2 += (pj != j) ? g * g + gp * gp : g * g;
+        }
+    }
+    nl = bdf_reduce(nl, false);
+    BDF_SYNC();
+    if (own) {
+        int e;
+        (void)frexp(s2, &e);
+        CPDP_LOOP for (int i = 0; i < n; ++i) G[j * QS + i] = ldexp(G[j * QS + i], -(e >> 1));
+    }
+    int hc, hi0;
+    const bool hact = bdf_half(lane, hc, hi0);
+    for (int it = 0;; ++it) {
+        if (own) { BDF_UNROLL for (int i = 0; i < n; ++i) XA[i * NCS + j] = G[j * QS + i]; }
+        if (!bdf_gauss_jordan(sm + bo::Q)) return false;            // Q[k][i] = H[i][k]
+        if (hact) bdf_lmul_to(LT, QS, G + hc * QS, 1, XA + hc, NCS, hi0);              // (L G)[:, c]
+        BDF_SYNC();
+        if (hact) bdf_lmul_to(sm + bo::Q, QS, XA + hc, NCS, XB + hc, NCS, hi0);        // M[:, c] = H (L G)[:, c]
+        BDF_SYNC();
+        double a = 0.0, b = 0.0, res = 0.0, ng = 0.0, nh = 0.0;
+        if (own) {
+            if (pj == j) a = XB[j * NCS + j];
+            else {
+                const int f = (pj > j) ? j : pj, s = (pj > j) ? pj : j;
+                a = 0.5 * (XB[f * NCS + f] + XB[s * NCS + s]);
+                b = 0.5 * (XB[f * NCS + s] - XB[s * NCS + f]);
+            }
+            BDF_UNROLL for (int i = 0; i < n; ++i) {
+                const double d = (i == j) ? a : ((i == pj) ? -sj * b : 0.0);
+                const double r = XB[i * NCS + j] - d, g = G[j * QS + i], h = sm[bo::Q + j * QS + i];
+                res += r * r; ng += g * g; nh += h * h;
+            }
+            BDF_ST2(sm + bo::TD + 2 * j, a, b);
+        }
+        res = bdf_reduce(res, false); ng = bdf_reduce(ng, false); nh = bdf_reduce(nh, false);
+        if (bdf_ballot(sm, own && pj != j && !(b > 0.0))) return false;
+        if (res <= (BDF_REFINE_TOL * BDF_REFINE_TOL) * nl) return ng * nh <= BDF_EIG_KAPPA * BDF_EIG_KAPPA;
+        if (it == BDF_REFINE_STEPS) return false;
+        BDF_SYNC();
+        bool bad = false;
+        if (own) {                                                     // column j of F -> XA
+            const auto lj = BDF_LD2(sm + bo::TD + 2 * j);
+            CPDP_LOOP for (int i = 0; i < n; ++i) {
+                const auto li = BDF_LD2(sm + bo::TD + 2 * i);
+                const int pi = (int)part[i];
+                const double si = (pi > i) ? 1.0 : ((pi < i) ? -1.0 : 0.0);
+                const bool blk = (i == j) || (i == pj);
+                const double dr = li.x - lj.x, dp = li.y - lj.y, dm = li.y + lj.y;
+                const double ip = blk ? 0.0 : 1.0 / (dr * dr + dp * dp);
+                const double im = (i == j && pj == j) ? 0.0 : 1.0 / (dr * dr + dm * dm);
+                const double ur = dr * ip, ui = -dp * ip, wr = dr * im, wi = -dm * im;     // w+ = ur + i ui, w- = wr + i wi
+                const double k1 = 0.5 * (ur + wr), k2 = si * (0.5 * (ui + wi)), k3 = sj * (0.5 * (wi - ui)), k4 = (si * sj) * (0.5 * (ur - wr));
+                const double f = -(((k1 * XB[i * NCS + j] + k2 * XB[pi * NCS + j]) + k3 * XB[i * NCS + pj]) + k4 * XB[pi * NCS + pj]);
+                if (!(fabs(f) <= BDF_REFINE_FMAX)) bad = true;
+                XA[i * NCS + j] = f;
+            }
+        }
+        if (bdf_ballot(sm, bad)) return false;
+        BDF_SYNC();
+        if (hact) bdf_lmul_to(G, QS, XA + hc, NCS, XB + hc, NCS, hi0);                 // (G F)[:, c]
+        BDF_SYNC();
+        if (own) { BDF_UNROLL for (int i = 0; i < n; ++i) G[j * QS + i] += XB[i * NCS + j]; }
+        BDF_SYNC();
+    }
+}
+
+// A new Jacobian's decomposition: the warm refinement when the previous Jacobian took the eigen path, else (and when the
+// refinement is rejected) the Schur form.  0: the QR iteration did not converge; 1: Schur form; 2: refinement accepted;
+// 3: refinement rejected, then the Schur form.
+#if CPDP_BDF_EIG_WARM
+CPDP_D_NOINLINE int bdf_decompose() {
+    BDF_SM();
+    if (BDF_EIG_KAPPA > 0.0 && ((const int*)(sm + bo::FLAG))[3]) {
+        BDF_TS0();
+        const bool warm = bdf_eig_refine();
+        BDF_TS(6);
+        if (warm) return 2;
+        return bdf_schur() ? 3 : 0;
+    }
+    return bdf_schur() ? 1 : 0;
+}
+#else
+CPDP_D int bdf_decompose() { return bdf_schur() ? 1 : 0; }      // (the call sites of the Schur form as without the refinement)
+#endif
 
 // Lyapunov sweep  (1/2 + cT) Y + Y (1/2 + cT)^H = C  along anti-diagonals i + j = d, four lanes per entry.  C in Y2 (upper
 // triangle), Y overwrites it, both triangles are kept (Y is Hermitian), so both sums of an entry have one form:
@@ -1235,7 +1379,7 @@ CPDP_D int bdf_interval(double* sm, double* D, const AuxProblem& p, const double
     BDF_T(1, bdf_rhs_smem(true)); ++cnt[0];
     bdf_get_col(sm + bo::XB, lc, f0);
     BDF_SYNC();
-    { bool oks__; BDF_TB(3, oks__, bdf_schur()); if (!oks__) return 4; }
+    { int dk__; BDF_TB(3, dk__, bdf_decompose()); if (!dk__) return 4; BDF_WARM(dk__); }
     BDF_PATH(sm, 2);
     double h_abs;
     {
@@ -1368,7 +1512,7 @@ CPDP_D int bdf_interval(double* sm, double* D, const AuxProblem& p, const double
                     }
                     BDF_SYNC();
                     BDF_T(2, bdf_jacobian()); ++cnt[3];
-                    { bool oks__; BDF_TB(3, oks__, bdf_schur()); if (!oks__) return 4; }
+                    { int dk__; BDF_TB(3, dk__, bdf_decompose()); if (!dk__) return 4; BDF_WARM(dk__); }
                     BDF_PATH(sm, 2);
                     lu_valid = false;
                     current_jac = true;
@@ -1478,7 +1622,8 @@ CPDP_GLOBAL void __launch_bounds__(BDF_THREADS, CPDP_BDF_MINB) k_riccati_bdf(Aux
         }                                                                                               \
     }
     BDF_STORE_NODE(N)
-    int cnt[8] = {0, 0, 0, 0, 0, 0, 0, 0};                          // (4..7: CPDP_BDF_PATH_COUNTS)
+    int cnt[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};                   // (4..9: CPDP_BDF_PATH_COUNTS)
+    if (lane == 0) ((int*)(sm + bo::FLAG))[3] = 0;                  // no eigenbasis to warm-start the first Jacobian from
     int st = 0;
 #ifdef CPDP_BDF_TIMING
     long long tp[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
@@ -1500,7 +1645,7 @@ CPDP_GLOBAL void __launch_bounds__(BDF_THREADS, CPDP_BDF_MINB) k_riccati_bdf(Aux
     }
 #endif
 #ifdef CPDP_BDF_PATH_COUNTS
-    if (lane == 0) { for (int i = 0; i < 4; ++i) a.Ua[(size_t)b * (N + 1) * NU * NP + 24 + i] = (double)cnt[4 + i]; }
+    if (lane == 0) { for (int i = 0; i < 6; ++i) a.Ua[(size_t)b * (N + 1) * NU * NP + 24 + i] = (double)cnt[4 + i]; }
 #endif
     if (lane == 0) {
         a.aux_status[b] = st;

@@ -20,6 +20,8 @@ VARIANTS = {
     "time": ["-DCPDP_BDF_TIMING"],
     "eig_off": ["-DCPDP_BDF_EIG_KAPPA=0"],                    # every Newton solve on the Bartels-Stewart sweep
     "time_eig_off": ["-DCPDP_BDF_TIMING", "-DCPDP_BDF_EIG_KAPPA=0"],
+    "warm_off": ["-DCPDP_BDF_EIG_WARM=0"],                   # every Jacobian through bdf_schur (no warm refinement)
+    "time_warm_off": ["-DCPDP_BDF_TIMING", "-DCPDP_BDF_EIG_WARM=0"],
     "l2s1": ["-DCPDP_BDF_LMUL_UNROLL=2", "-DCPDP_BDF_STENCIL_UNROLL=1"],
     "l1s1": ["-DCPDP_BDF_LMUL_UNROLL=1", "-DCPDP_BDF_STENCIL_UNROLL=1"],
     "l4s2": ["-DCPDP_BDF_LMUL_UNROLL=4", "-DCPDP_BDF_STENCIL_UNROLL=2"],
@@ -80,7 +82,7 @@ def main():
             out = {"variant": v, "batch": B, "ms": [round(t, 3) for t in times],
                    "failed": int((aux["aux_status"] != 0).sum().item())}
             if "time" in v:
-                tp = aux["Ua"].reshape(B, -1)[:, :28].cpu().numpy()
+                tp = aux["Ua"].reshape(B, -1)[:, :30].cpu().numpy()
                 tot = tp[:, 8].mean()
                 out["cycles_total_mean"] = float(tot)
                 out["phase_share"] = {PHASES[i]: round(float(tp[:, i].mean() / tot), 4) for i in range(8)}
@@ -104,7 +106,11 @@ def main():
                                                 "block_scaling": per(9, n_eig), "stencil_in": per(11, n_sweep),
                                                 "sweep": per(12, n_sweep), "stencil_out": per(13, n_sweep)}
                 nj = cnt[:, 5].mean()
-                out["schur_cycles_per_call"] = {nm: float(tp[:, 16 + i].mean() / nj) for i, nm in enumerate(
+                # Jacobians whose warm refinement was accepted | rejected; the Schur form runs for all but the accepted ones
+                w_acc, w_rej = float(tp[:, 28].mean()), float(tp[:, 29].mean())
+                out["warm"] = {"accepted": w_acc, "rejected": w_rej, "accepted_share_of_jac": round(w_acc / nj, 4),
+                               "refine_cycles_per_attempt": per(22, w_acc + w_rej)}
+                out["schur_cycles_per_call"] = {nm: float(tp[:, 16 + i].mean() / (nj - w_acc)) for i, nm in enumerate(
                     ["hessenberg", "qr_scans", "qr_scans_plus_chase", "rotations", "rotations_plus_packing", "eig_basis"])}
                 out["counters_mean"] = {"rhs": cnt[:, 0].mean(), "steps": cnt[:, 1].mean(), "lu": cnt[:, 4].mean(), "jac": nj}
             print(json.dumps(out), flush=True)
