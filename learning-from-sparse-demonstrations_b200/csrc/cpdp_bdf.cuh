@@ -93,7 +93,8 @@ CPDP_D double bdf_mul(double a, double b) { volatile double r = a * b; return r;
 // Shared-memory layout of one problem: compile-time offsets (in doubles) into the dynamic block.
 constexpr int QS = (NX + 1) & ~1;                // row stride of the k-major product operands
 constexpr int NCS = NC | 1;                      // odd row stride of the column exchange buffers (conflict-free transposes)
-constexpr int SWQ = (NX - 1 + 3) / 4;            // Lyapunov sweep: terms per lane and sum (4 lanes per entry)
+constexpr int SWQ = NX > 1 ? (NX - 1 + 3) / 4 : 1;   // Lyapunov sweep: terms per lane and sum (4 lanes per entry; >= 1: the eigen
+                                                 // path's scratch in T2S needs a nonzero TW, and at NX = 1 every term is a stored zero)
 constexpr int TW = 4 * SWQ;                      // row width of the skewed T: T2S[r][t] = T[r][r + 1 + t], zero beyond the matrix
 constexpr int NH = (NX + 1) / 2;                 // rows per half in the two-halves products (lanes c and 16 + c)
 namespace bo {
