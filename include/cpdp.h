@@ -133,6 +133,21 @@ int cpdp_aux_adjoint(void* ws, size_t ws_bytes, int B, int N, int S, double T,
                      const double* X, const double* U, const double* Lam, const int* solve_status,
                      const double* Xbar, const double* Ubar, double* theta_bar, double* x0_bar, int* aux_status, void* stream);
 
+/* Bytes of the pdata workspace of cpdp_aux_adjoint_pd for B problems of N intervals (0 when the model has no per-problem
+ * constants).  Separate from cpdp_workspace_bytes, which does not change. */
+size_t cpdp_pdata_workspace_bytes(int B, int N);
+
+/* cpdp_aux_adjoint plus pdata_bar[B][q] = sum_k (dX_k/dpdata)' Xbar_k + (dU_k/dpdata)' Ubar_k, the gradient with respect to the
+ * per-problem constants (DESIGN.md §3.11).  The q constants ride along as q extra parameter columns of the same sweep; pd_ws
+ * (cpdp_pdata_workspace_bytes(B, N) bytes, -3 if smaller) holds their stage derivatives and gains.  theta_bar and x0_bar are those
+ * of cpdp_aux_adjoint; same zero-row rule and argument-error codes, plus -14 (the model has no per-problem constants) and -15 (the
+ * library was built without the pdata derivatives, or n + m + r + q > 32). */
+int cpdp_aux_adjoint_pd(void* ws, size_t ws_bytes, void* pd_ws, size_t pd_ws_bytes, int B, int N, int S, double T,
+                        const double* theta, int theta_stride, const double* pdata,
+                        const double* X, const double* U, const double* Lam, const int* solve_status,
+                        const double* Xbar, const double* Ubar, double* theta_bar, double* x0_bar, double* pdata_bar,
+                        int* aux_status, void* stream);
+
 /* FP64 FMA throughput probe used by bench.py for the roofline denominator: one kernel of `blocks` x 256 threads,
  * 8 independent chains of `iters` DFMAs per thread (flops = blocks*256*8*iters*2).  sink: >= 1 device double. */
 int cpdp_dfma_probe(double* sink, int blocks, int iters, void* stream);

@@ -220,8 +220,10 @@ class COCSys:
                                                     self.dyn, self.path_cost, self.final_cost, self.pvar,
                                                     time=getattr(self, 'time', None), bounds=self._bounds())
         self.codegen_info = info
+        pd_text, _ = codegen.generate_pdata_header(name or self.sys_name, self.state, self.control, self.auxvar, self.dyn,
+                                                   self.path_cost, self.final_cost, self.pvar, time=getattr(self, 'time', None))
         libname = name if name is not None else "m" + info["hash"]
-        so = _capi.build_model_library(libname, text, force=force, verbose=verbose)
+        so = _capi.build_model_library(libname, text, force=force, verbose=verbose, pd_header_text=pd_text)
         self._lib = _capi.CpdpLib(so)
         assert (self._lib.n, self._lib.m, self._lib.r, self._lib.q) == \
             (self.n_state, self.n_control, self.n_auxvar, self.n_pvar)
@@ -389,15 +391,30 @@ class COCSys:
         self._lib.set_bound_multipliers(mem.ptr(ws), int(ws.shape[0]), sol["B"], self.n_grid, self.steps_per_grid,
                                         mem.ptr(sol["Zl"]), mem.ptr(sol["Zu"]), mem.ptr(sol["mu"]), mem.stream())
 
-    def auxSysAdjointBatch(self, sol, Xbar=None, Ubar=None):
+    def _pdata_workspace(self, B, slot=0):
+        """Scratch of the pdata adjoint (cpdp_pdata_workspace_bytes), allocated on first use per slot as _workspace's."""
+        lib = self.build()
+        key = (B, self.n_grid)
+        pool = self.__dict__.setdefault("_pd_ws_pool", {})
+        if pool.get(slot, (None, None))[0] != key:
+            pool[slot] = (key, self._device().empty((lib.pdata_workspace_bytes(*key),), "u1"))
+        return pool[slot][1]
+
+    def auxSysAdjointBatch(self, sol, Xbar=None, Ubar=None, pdata_bar=False):
         """Adjoint of mode 2: the gradient of a loss l(X, U) of the trajectory with respect to theta and x0, from its cotangents
         Xbar = dl/dX [B,N+1,n] and Ubar = dl/dU [B,N+1,m] (either may be None, meaning zero), by one reverse sweep per problem
         (DESIGN.md §3.9).  ``sol`` is the dict returned by cocSolverBatch (or one shaped like it; a bounded model needs its
         Zl, Zu, mu).  Returns device arrays theta_bar [B,r] (per-problem rows, also for a theta shared by the batch), x0_bar
         [B,n] and aux_status [B] (as mode 2: 0 ok, 3 no usable trajectory, 4 Quu not positive definite).  Rows are zero for a
-        problem with aux_status != 0 or whose solve did not end `converged`."""
+        problem with aux_status != 0 or whose solve did not end `converged`.
+
+        pdata_bar=True also returns pdata_bar [B,q], the gradient with respect to the per-problem constants, from the same sweep
+        with q more parameter columns (DESIGN.md §3.11); theta_bar and x0_bar are unchanged.  A model without per-problem
+        constants raises ValueError."""
         if Xbar is None and Ubar is None:
             raise ValueError("auxSysAdjointBatch needs a cotangent Xbar or Ubar")
+        if pdata_bar and self.n_pvar == 0:
+            raise ValueError("pdata_bar=True needs a model with per-problem constants (setProblemVariable)")
         lib = self.build()
         mem = self._device()
         B, N, S = sol["B"], self.n_grid, self.steps_per_grid
@@ -413,6 +430,15 @@ class COCSys:
         if lib.has_bounds:
             self._set_bound_multipliers(sol, ws)
         out = dict(theta_bar=mem.empty((B, r)), x0_bar=mem.empty((B, n)), aux_status=mem.zeros((B,), "i4"))
+        if pdata_bar:
+            pws = self._pdata_workspace(B, sol.get("_slot", 0))
+            out["pdata_bar"] = mem.empty((B, self.n_pvar))
+            lib.aux_adjoint_pd(mem.ptr(ws), int(ws.shape[0]), mem.ptr(pws), int(pws.shape[0]), B, N, S, sol["horizon"],
+                               mem.ptr(sol["theta"]), sol["theta_stride"], mem.ptr(sol["pdata"]), mem.ptr(sol["X"]),
+                               mem.ptr(sol["U"]), mem.ptr(sol["Lam"]), mem.ptr(sol.get("status")), mem.ptr(cot[0]),
+                               mem.ptr(cot[1]), mem.ptr(out["theta_bar"]), mem.ptr(out["x0_bar"]), mem.ptr(out["pdata_bar"]),
+                               mem.ptr(out["aux_status"]), mem.stream())
+            return out
         lib.aux_adjoint(mem.ptr(ws), int(ws.shape[0]), B, N, S, sol["horizon"], mem.ptr(sol["theta"]), sol["theta_stride"],
                         mem.ptr(sol["pdata"]), mem.ptr(sol["X"]), mem.ptr(sol["U"]), mem.ptr(sol["Lam"]),
                         mem.ptr(sol.get("status")), mem.ptr(cot[0]), mem.ptr(cot[1]), mem.ptr(out["theta_bar"]),

@@ -46,14 +46,17 @@ def _sources_digest():
     return h.hexdigest()[:16]
 
 
-def build_model_library(name, header_text, force=False, verbose=False):
-    """Writes csrc/generated/model_<name>.cuh and compiles lib/libcpdp_<name>.so (skipped when up to date)."""
+def build_model_library(name, header_text, force=False, verbose=False, pd_header_text=None):
+    """Writes csrc/generated/model_<name>.cuh (and, given ``pd_header_text``, the companion model_<name>_pd.cuh with the pdata
+    derivatives, codegen.generate_pdata_header) and compiles lib/libcpdp_<name>.so (skipped when up to date)."""
     os.makedirs(GEN_DIR, exist_ok=True)
     os.makedirs(LIB_DIR, exist_ok=True)
     hdr = os.path.join(GEN_DIR, "model_%s.cuh" % name)
+    pd_hdr = os.path.join(GEN_DIR, "model_%s_pd.cuh" % name)
     so = os.path.join(LIB_DIR, "libcpdp_%s.so" % name)
     stamp = so + ".stamp"
-    digest = hashlib.sha1((header_text + _sources_digest() + " ".join(NVCC_FLAGS + EXTRA_NVCC_FLAGS)).encode()).hexdigest()
+    digest = hashlib.sha1((header_text + (pd_header_text or "") + _sources_digest() +
+                           " ".join(NVCC_FLAGS + EXTRA_NVCC_FLAGS)).encode()).hexdigest()
 
     def up_to_date():
         # The digest of (model header, kernel sources, all flags) is compiled INTO the library (cpdp_build_digest), so a prebuilt
@@ -80,10 +83,15 @@ def build_model_library(name, header_text, force=False, verbose=False):
                 return so
             with open(hdr, "w") as f:
                 f.write(header_text)
+            pd_flags = []
+            if pd_header_text is not None:
+                with open(pd_hdr, "w") as f:
+                    f.write(pd_header_text)
+                pd_flags = ["-DCPDP_PD_HEADER=\"%s\"" % pd_hdr]
             ns = "cpdp_" + "".join(ch if ch.isalnum() else "_" for ch in name)
             tmp = "%s.tmp%d" % (so, os.getpid())
             cmd = [nvcc] + NVCC_FLAGS + EXTRA_NVCC_FLAGS + ["-I", CSRC, "-DCPDP_NS=%s" % ns, "-DCPDP_MODEL_HEADER=\"%s\"" % hdr,
-                                         "-DCPDP_BUILD_DIGEST=\"%s%s\"" % (_DIGEST_MARK, digest),
+                                         "-DCPDP_BUILD_DIGEST=\"%s%s\"" % (_DIGEST_MARK, digest)] + pd_flags + [
                                          os.path.join(CSRC, "cpdp_lib.cu"), "-o", tmp]
             if verbose:
                 cmd.insert(1, "-Xptxas=-v")
@@ -130,6 +138,11 @@ class CpdpLib:
         L.cpdp_aux_phases.restype = _i
         L.cpdp_aux_adjoint.argtypes = [_vp, _sz, _i, _i, _i, _d, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]
         L.cpdp_aux_adjoint.restype = _i
+        L.cpdp_pdata_workspace_bytes.argtypes = [_i, _i]
+        L.cpdp_pdata_workspace_bytes.restype = _sz
+        L.cpdp_aux_adjoint_pd.argtypes = [_vp, _sz, _vp, _sz, _i, _i, _i, _d, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                          _vp, _vp, _vp]
+        L.cpdp_aux_adjoint_pd.restype = _i
         L.cpdp_dfma_probe.argtypes = [_vp, _i, _i, _vp]
         L.cpdp_dfma_probe.restype = _i
         L.cpdp_reduce.argtypes = [_vp, _vp, _i, _vp, _vp, _vp]
@@ -198,6 +211,15 @@ class CpdpLib:
                     theta_bar, x0_bar, aux_status, stream):
         self.check(self.L.cpdp_aux_adjoint(ws, ws_bytes, B, N, S, T, theta, theta_stride, pdata, X, U, Lam, solve_status, Xbar,
                                            Ubar, theta_bar, x0_bar, aux_status, stream), "cpdp_aux_adjoint")
+
+    def pdata_workspace_bytes(self, B, N):
+        return int(self.L.cpdp_pdata_workspace_bytes(B, N))
+
+    def aux_adjoint_pd(self, ws, ws_bytes, pd_ws, pd_ws_bytes, B, N, S, T, theta, theta_stride, pdata, X, U, Lam, solve_status,
+                       Xbar, Ubar, theta_bar, x0_bar, pdata_bar, aux_status, stream):
+        self.check(self.L.cpdp_aux_adjoint_pd(ws, ws_bytes, pd_ws, pd_ws_bytes, B, N, S, T, theta, theta_stride, pdata, X, U, Lam,
+                                              solve_status, Xbar, Ubar, theta_bar, x0_bar, pdata_bar, aux_status, stream),
+                   "cpdp_aux_adjoint_pd")
 
     def get_bound_multipliers(self, ws, ws_bytes, B, N, S, Zl, Zu, mu, stream):
         self.check(self.L.cpdp_get_bound_multipliers(ws, ws_bytes, B, N, S, Zl, Zu, mu, stream), "cpdp_get_bound_multipliers")

@@ -127,13 +127,9 @@ def _bounds_block(bounds, n, m):
     return "\n".join(lines) + "\n"
 
 
-def generate_model_header(name, state, control, auxvar, dyn, path_cost, final_cost, pdata=None, time=None, bounds=None):
-    """Returns (header_text, info dict).  All arguments are SX / sympy matrices / scalars.
-    ``pdata``: optional per-problem constants (e.g. a goal position) that are not learnable.
-    ``time``: the explicit time variable of a COCSys_TimeVarying model (CPDP.py:434); the generated functions read it as
-    one more constant, pd[nq], which the kernels fill in (the node time t_k in the RK4 map, the true t in the sweeps).
-    ``bounds``: optional (state_lb, state_ub, control_lb, control_ub); the header gets HAS_BOUNDS and the four bound tables
-    only when some bound is finite."""
+def _model_exprs(state, control, auxvar, dyn, path_cost, final_cost, pdata, time):
+    """The model's expressions in the array names of the generated C (x[i], u[i], th[i], pd[i], mu[i], w, dx[i], du[i]) and the
+    derivatives that every generated function shares."""
     x, u, th = _vec(state), _vec(control), _vec(auxvar)
     pdv = _vec(pdata) if pdata is not None else []
     n, m, r = len(x), len(u), len(th)
@@ -172,6 +168,22 @@ def generate_model_header(name, state, control, auxvar, dyn, path_cost, final_co
     Hz = sp.Matrix([Ham]).jacobian(z)
     Hzz = Hz.jacobian(z)
     dz = sp.Matrix(dxs + dus)
+
+    return dict(n=n, m=m, r=r, nq=nq, nz=nz, tv=tv, f=f, c=c, h=h, xs=xs, us=us, ts=ts, ps=ps, z=z, mus=mus, w=w,
+                fz=fz, Hz=Hz, Hzz=Hzz, dz=dz)
+
+
+def generate_model_header(name, state, control, auxvar, dyn, path_cost, final_cost, pdata=None, time=None, bounds=None):
+    """Returns (header_text, info dict).  All arguments are SX / sympy matrices / scalars.
+    ``pdata``: optional per-problem constants (e.g. a goal position) that are not learnable.
+    ``time``: the explicit time variable of a COCSys_TimeVarying model (CPDP.py:434); the generated functions read it as
+    one more constant, pd[nq], which the kernels fill in (the node time t_k in the RK4 map, the true t in the sweeps).
+    ``bounds``: optional (state_lb, state_ub, control_lb, control_ub); the header gets HAS_BOUNDS and the four bound tables
+    only when some bound is finite."""
+    e = _model_exprs(state, control, auxvar, dyn, path_cost, final_cost, pdata, time)
+    n, m, r, nq, nz, tv = e["n"], e["m"], e["r"], e["nq"], e["nz"], e["tv"]
+    f, c, h, xs, us, ts, z, mus, w = (e[k] for k in ("f", "c", "h", "xs", "us", "ts", "z", "mus", "w"))
+    fz, Hz, Hzz, dz = e["fz"], e["Hz"], e["Hzz"], e["dz"]
 
     info = {}
     parts = []
@@ -289,5 +301,44 @@ struct Model {{
 }};
 """.format(name=name, nz=nz, has_time=len(tv), bounds=_bounds_block(bounds, n, m), offs="\n".join(offs), tables=tables,
            parts="\n\n".join(parts), **info)
+    info["hash"] = hashlib.sha1(text.encode()).hexdigest()[:16]
+    return text, info
+
+
+def generate_pdata_header(name, state, control, auxvar, dyn, path_cost, final_cost, pdata=None, time=None):
+    """Companion header ``model_<name>_pd.cuh``: ``struct ModelPd`` with the derivatives with respect to the NQ per-problem
+    constants that the pdata adjoint (csrc/cpdp_pd.cuh, DESIGN.md §3.11) needs.  A separate file, so that the model header and
+    its hash do not change.  Only the user constants pd[0..NQ-1] are differentiated; the time of a time-varying model, pd[NQ], is
+    not a pdata column.  Returns (header_text, info dict).
+      dir_pd(x,u,th,pd,mu,w,dx,du,dpd, df[n], hz[nz])   df = fz dz + f_pd dpd ; hz = Hess_z(Ham) dz + Hess_zpd(Ham) dpd
+      term2_pd(x,th,pd, hxp[n*nq])                     d(grad_x h)/dpd, row-major
+    For NQ = 0 the struct holds NQ only."""
+    e = _model_exprs(state, control, auxvar, dyn, path_cost, final_cost, pdata, time)
+    n, nq, nz = e["n"], e["nq"], e["nz"]
+    info = dict(nq=nq)
+    parts = []
+    if nq > 0:
+        pq = e["ps"][:nq]
+        dpd = sp.Matrix([sp.Symbol("dpd[%d]" % i, real=True) for i in range(nq)])
+        df = e["fz"] * e["dz"] + e["f"].jacobian(pq) * dpd
+        hz = e["Hzz"] * e["dz"] + e["Hz"].T.jacobian(pq) * dpd
+        body, info["ops_dir_pd"] = _emit_body([("df[%d]" % i, df[i]) for i in range(n)] +
+                                              [("hz[%d]" % i, hz[i]) for i in range(nz)])
+        parts.append("    CPDP_HD static void dir_pd(const double* __restrict__ x, const double* __restrict__ u, "
+                     "const double* __restrict__ th, const double* __restrict__ pd, const double* __restrict__ mu, const double w, "
+                     "const double* __restrict__ dx, const double* __restrict__ du, const double* __restrict__ dpd, "
+                     "double* __restrict__ df, double* __restrict__ hz) {\n%s\n    }" % body)
+        hxp = sp.Matrix([e["h"]]).jacobian(e["xs"]).jacobian(pq)
+        body, info["ops_term2_pd"] = _emit_body([("hxp[%d]" % (i * nq + j), hxp[i, j]) for i in range(n) for j in range(nq)])
+        parts.append("    CPDP_HD static void term2_pd(const double* __restrict__ x, const double* __restrict__ th, "
+                     "const double* __restrict__ pd, double* __restrict__ hxp) {\n%s\n    }" % body)
+    text = """// GENERATED by lfsd_b200/codegen.py -- do not edit.  model: {name}, derivatives with respect to the per-problem constants
+#pragma once
+#include "cpdp_port.h"
+struct ModelPd {{
+    static constexpr int NQ = {nq};
+{parts}
+}};
+""".format(name=name, nq=nq, parts="\n\n".join(parts))
     info["hash"] = hashlib.sha1(text.encode()).hexdigest()[:16]
     return text, info

@@ -11,6 +11,16 @@
 
 namespace CPDP_NS {
 
+// The NQ per-problem constants as extra parameter columns (cpdp_pd.cuh, DESIGN.md §3.11): mode 2's three arrays for them, in a
+// separate caller-provided workspace.  The body of k_aux_adjoint is a template on the model's pdata derivatives PM (PM::NQ extra
+// columns); NoPd (0 columns) is k_aux_adjoint as it is.
+struct PdWs {
+    double* Hpd;           // [B*N][NZ][NQ]  d(grad_z (q_k + lam_{k+1}'F_k))/dpd
+    double* Epd;           // [B*N][NX][NQ]  dF_k/dpd
+    double* Kpd;           // [B*N][NU][NQ]  feed-forward gains
+};
+struct NoPd { static constexpr int NQ = 0; };
+
 struct AdjArgs {
     const double* Xbar;    // [B][N+1][NX] or null (zero)
     const double* Ubar;    // [B][N+1][NU] or null (zero)
@@ -36,7 +46,10 @@ struct AdjStage {
     double e[ADJ_RP][NX], kt[ADJ_RP][NU];               // column q of E and of Kth
 };
 
-CPDP_D void adj_fetch(const SolveArgs& a, const DiscWs& d, const AdjArgs& j, int b, int k, int lane,
+// PM::NQ > 0 (cpdp_pd.cuh): lane l owns column l of [theta | pdata], i.e. column l of [E | E^pd] and [Kth | K^pd] (NP + NQ <= 32,
+// so that the stage operands do not grow).
+template <class PM>
+CPDP_D void adj_fetch(const SolveArgs& a, const DiscWs& d, const PdWs& pw, const AdjArgs& j, int b, int k, int lane,
                       AdjStage& s) {
     const int N = a.N;
     const size_t g = (size_t)b * N + k;
@@ -60,18 +73,34 @@ CPDP_D void adj_fetch(const SolveArgs& a, const DiscWs& d, const AdjArgs& j, int
         }
         s.ub[t] = v;
     }
-    NWT_UNROLL for (int t = 0; t < ADJ_RP; ++t) {
-        const int q0 = lane + t * ADJ_THREADS, q = q0 < NP ? q0 : 0;
-        NWT_UNROLL for (int e = 0; e < NX; ++e) s.e[t][e] = Eg[e * NP + q];
-        NWT_UNROLL for (int c = 0; c < NU; ++c) s.kt[t][c] = Ktk[c * NP + q];
+    if constexpr (PM::NQ > 0) {
+        constexpr int XQ = PM::NQ;
+        static_assert(ADJ_RP == 1 && NP + XQ <= ADJ_THREADS, "one column of [theta | pdata] per lane");
+        const int l = lane < NP + XQ ? lane : 0;
+        const bool th = l < NP;
+        const double* Ec = th ? Eg + l : pw.Epd + g * NX * XQ + (l - NP);
+        const double* Kc = th ? Ktk + l : pw.Kpd + g * NU * XQ + (l - NP);
+        const int ld = th ? NP : XQ;
+        NWT_UNROLL for (int e = 0; e < NX; ++e) s.e[0][e] = Ec[e * ld];
+        NWT_UNROLL for (int c = 0; c < NU; ++c) s.kt[0][c] = Kc[c * ld];
+    } else {
+        NWT_UNROLL for (int t = 0; t < ADJ_RP; ++t) {
+            const int q0 = lane + t * ADJ_THREADS, q = q0 < NP ? q0 : 0;
+            NWT_UNROLL for (int e = 0; e < NX; ++e) s.e[t][e] = Eg[e * NP + q];
+            NWT_UNROLL for (int c = 0; c < NU; ++c) s.kt[t][c] = Ktk[c * NP + q];
+        }
     }
 }
 
-CPDP_GLOBAL void __launch_bounds__(ADJ_THREADS) k_aux_adjoint(AuxArgs x, SolveArgs a, DiscWs d, AdjArgs j) {
+// PM::NQ > 0: the same sweep with pdata_bar[B][NQ] += K^pd' g + E^pd' p accumulated by lanes NP .. NP + NQ - 1.
+template <class PM>
+CPDP_D void adjoint_body(AuxArgs x, SolveArgs a, DiscWs d, AdjArgs j, PdWs pw, double* pdata_bar) {
+    constexpr int XQ = PM::NQ;
     const int b = blockIdx.x, lane = threadIdx.x;
     const int N = a.N;
     if (x.aux_status[b] != 0 || (x.solve_status && x.solve_status[b] != ST_CONVERGED)) {
         for (int q = lane; q < NP; q += ADJ_THREADS) j.theta_bar[(size_t)b * NP + q] = 0.0;
+        for (int q = lane; q < XQ; q += ADJ_THREADS) pdata_bar[(size_t)b * XQ + q] = 0.0;
         if (j.x0_bar) for (int i = lane; i < NX; i += ADJ_THREADS) j.x0_bar[(size_t)b * NX + i] = 0.0;
         return;
     }
@@ -80,11 +109,11 @@ CPDP_GLOBAL void __launch_bounds__(ADJ_THREADS) k_aux_adjoint(AuxArgs x, SolveAr
     double tb[ADJ_RP];
     NWT_UNROLL for (int t = 0; t < ADJ_RP; ++t) tb[t] = 0.0;
     AdjStage cur, nxt;
-    adj_fetch(a, d, j, b, N - 1, lane, nxt);
+    adj_fetch<PM>(a, d, pw, j, b, N - 1, lane, nxt);
     NWT_SYNC();
     CPDP_LOOP for (int k = N - 1; k >= 0; --k) {
         cur = nxt;
-        if (k > 0) adj_fetch(a, d, j, b, k - 1, lane, nxt);
+        if (k > 0) adj_fetch<PM>(a, d, pw, j, b, k - 1, lane, nxt);
         // g = Ubar'_k + B_k' p
         NWT_UNROLL for (int t = 0; t < ADJ_RU; ++t) {
             const int u = lane + t * ADJ_THREADS;
@@ -119,8 +148,13 @@ CPDP_GLOBAL void __launch_bounds__(ADJ_THREADS) k_aux_adjoint(AuxArgs x, SolveAr
     NWT_UNROLL for (int t = 0; t < ADJ_RP; ++t) {
         const int q = lane + t * ADJ_THREADS;
         if (q < NP) j.theta_bar[(size_t)b * NP + q] = tb[t];
+        else if (XQ > 0 && q < NP + XQ) pdata_bar[(size_t)b * XQ + q - NP] = tb[t];
     }
     if (j.x0_bar) for (int i = lane; i < NX; i += ADJ_THREADS) j.x0_bar[(size_t)b * NX + i] = s_p[i];
+}
+
+CPDP_GLOBAL void __launch_bounds__(ADJ_THREADS) k_aux_adjoint(AuxArgs x, SolveArgs a, DiscWs d, AdjArgs j) {
+    adjoint_body<NoPd>(x, a, d, j, PdWs{}, nullptr);
 }
 
 }  // namespace CPDP_NS

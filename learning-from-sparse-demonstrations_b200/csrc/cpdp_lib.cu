@@ -80,6 +80,8 @@ extern "C" CPDP_API const char* cpdp_error_string(int code) {
             case -11: return "the model has no finite bound";
             case -12: return "shift must be 0 or 1";
             case -13: return "mu_init must be > 0 on a bounded model";
+            case -14: return "the model has no per-problem constants (pdata)";
+            case -15: return "the library was built without the pdata derivatives (or n + m + r + q > 32)";
             default: return "invalid argument";
         }
     }
