@@ -307,7 +307,7 @@ struct Model {{
 
 def generate_pdata_header(name, state, control, auxvar, dyn, path_cost, final_cost, pdata=None, time=None):
     """Companion header ``model_<name>_pd.cuh``: ``struct ModelPd`` with the derivatives with respect to the NQ per-problem
-    constants that the pdata adjoint (csrc/cpdp_pd.cuh, DESIGN.md §3.11) needs.  A separate file, so that the model header and
+    constants that the pdata adjoint (cpdp_aux_adjoint_pd, DESIGN.md §3.11) needs.  A separate file, so that the model header and
     its hash do not change.  Only the user constants pd[0..NQ-1] are differentiated; the time of a time-varying model, pd[NQ], is
     not a pdata column.  Returns (header_text, info dict).
       dir_pd(x,u,th,pd,mu,w,dx,du,dpd, df[n], hz[nz])   df = fz dz + f_pd dpd ; hz = Hess_z(Ham) dz + Hess_zpd(Ham) dpd

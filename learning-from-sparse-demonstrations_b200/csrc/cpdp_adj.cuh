@@ -6,20 +6,14 @@
 //     Ubar'_{N-1} = Ubar_{N-1} + Ubar_N,   p = Xbar_N,   theta_bar = 0
 //     k = N-1 .. 0:   g = Ubar'_k + B_k' p,   theta_bar += Kth_k' g + E_k' p,   p = Xbar_k + A_k' p + K_k' g
 //     x0_bar = p
+// The NQ per-problem constants pdata enter the KKT system exactly as theta does (cpdp_aux_adjoint_pd, DESIGN.md §3.11), so they
+// ride along as NQ extra parameter columns of mode 2's phase 1 and of this sweep, PM = ModelPd of the companion header
+// model_<name>_pd.cuh (codegen.py generate_pdata_header):  pdata_bar += K^pd' g + E^pd' p.  A library instantiates the kernels on
+// ModelPd only when the model has constants and NZ + NP + NQ <= 32 (the columns fit the idle lanes and threads).
 #pragma once
 #include "cpdp_disc.cuh"
 
 namespace CPDP_NS {
-
-// The NQ per-problem constants as extra parameter columns (cpdp_pd.cuh, DESIGN.md §3.11): mode 2's three arrays for them, in a
-// separate caller-provided workspace.  The body of k_aux_adjoint is a template on the model's pdata derivatives PM (PM::NQ extra
-// columns); NoPd (0 columns) is k_aux_adjoint as it is.
-struct PdWs {
-    double* Hpd;           // [B*N][NZ][NQ]  d(grad_z (q_k + lam_{k+1}'F_k))/dpd
-    double* Epd;           // [B*N][NX][NQ]  dF_k/dpd
-    double* Kpd;           // [B*N][NU][NQ]  feed-forward gains
-};
-struct NoPd { static constexpr int NQ = 0; };
 
 struct AdjArgs {
     const double* Xbar;    // [B][N+1][NX] or null (zero)
@@ -29,8 +23,8 @@ struct AdjArgs {
 };
 
 // ------------------------------------------------------------------------------------------------
-// k_aux_adjoint: one warp per problem (grid = B).  p and g live in shared memory; lane i forms row i of A'p + K'g (rows i, i + 32,
-// ...), lane j forms g_j, lane q accumulates theta_bar_q in registers.  Every global operand of stage k - 1 (the columns of
+// k_aux_adjoint<PM>: one warp per problem (grid = B).  p and g live in shared memory; lane i forms row i of A'p + K'g (rows i,
+// i + 32, ...), lane j forms g_j, lane q accumulates theta_bar_q in registers.  Every global operand of stage k - 1 (the columns of
 // [A B], K, Kth, E this lane contracts and its entries of Xbar, Ubar) is fetched in one batch of independent loads while stage k
 // is computed.  The summation order depends on N only (no atomics): a problem's row does not depend on the batch around it.
 // Rows are zero for a problem with aux_status != 0 or a solve that did not end CPDP_CONVERGED (the rule of k_pack_rows).
@@ -46,8 +40,8 @@ struct AdjStage {
     double e[ADJ_RP][NX], kt[ADJ_RP][NU];               // column q of E and of Kth
 };
 
-// PM::NQ > 0 (cpdp_pd.cuh): lane l owns column l of [theta | pdata], i.e. column l of [E | E^pd] and [Kth | K^pd] (NP + NQ <= 32,
-// so that the stage operands do not grow).
+// PM::NQ > 0 (cpdp_aux_adjoint_pd): lane l owns column l of [theta | pdata], i.e. column l of [E | E^pd] and [Kth | K^pd]
+// (NP + NQ <= 32, so that the stage operands do not grow).
 template <class PM>
 CPDP_D void adj_fetch(const SolveArgs& a, const DiscWs& d, const PdWs& pw, const AdjArgs& j, int b, int k, int lane,
                       AdjStage& s) {
@@ -94,7 +88,8 @@ CPDP_D void adj_fetch(const SolveArgs& a, const DiscWs& d, const PdWs& pw, const
 
 // PM::NQ > 0: the same sweep with pdata_bar[B][NQ] += K^pd' g + E^pd' p accumulated by lanes NP .. NP + NQ - 1.
 template <class PM>
-CPDP_D void adjoint_body(AuxArgs x, SolveArgs a, DiscWs d, AdjArgs j, PdWs pw, double* pdata_bar) {
+CPDP_GLOBAL void __launch_bounds__(ADJ_THREADS) k_aux_adjoint(AuxArgs x, SolveArgs a, DiscWs d, AdjArgs j, PdWs pw,
+                                                              double* pdata_bar) {
     constexpr int XQ = PM::NQ;
     const int b = blockIdx.x, lane = threadIdx.x;
     const int N = a.N;
@@ -151,10 +146,6 @@ CPDP_D void adjoint_body(AuxArgs x, SolveArgs a, DiscWs d, AdjArgs j, PdWs pw, d
         else if (XQ > 0 && q < NP + XQ) pdata_bar[(size_t)b * XQ + q - NP] = tb[t];
     }
     if (j.x0_bar) for (int i = lane; i < NX; i += ADJ_THREADS) j.x0_bar[(size_t)b * NX + i] = s_p[i];
-}
-
-CPDP_GLOBAL void __launch_bounds__(ADJ_THREADS) k_aux_adjoint(AuxArgs x, SolveArgs a, DiscWs d, AdjArgs j) {
-    adjoint_body<NoPd>(x, a, d, j, PdWs{}, nullptr);
 }
 
 }  // namespace CPDP_NS

@@ -6,9 +6,12 @@
 // with [A B], H of the interval Lagrangian q_k + lam_{k+1}'F_k (k_stage_adjoint + k_stage_hessian, unchanged), E_k = dF_k/dtheta and
 // Hth_k = d(grad_z of the interval Lagrangian)/dtheta (k_stage_theta), solved by a Riccati recursion with no regularisation
 // (k_aux_discrete).  Kernels:
-//   k_disc_select   active list of the problems with a usable trajectory (the others get aux_status 3), counters zeroed
-//   k_stage_theta   NZ + NP threads per interval: the NZ (x,u) sensitivity columns and the NP theta columns through the 4S stages
-//   k_aux_discrete  one warp per problem: phase 1 backward recursion (gains to the workspace), phase 2 rollout + loss
+//   k_disc_select       active list of the problems with a usable trajectory (the others get aux_status 3), counters zeroed
+//   k_stage_theta<PM>   NZ + NP + PM::NQ threads per interval: the NZ (x,u) sensitivity columns, the NP theta columns and the
+//                       PM::NQ pdata columns through the 4S stages
+//   k_aux_discrete<PM>  one warp per problem: phase 1 backward recursion (gains to the workspace), phase 2 rollout + loss (NoPd
+//                       only: with pdata columns the kernel runs phase 1 whatever `phase` says)
+// PM is NoPd (no pdata columns) for mode 2 and cpdp_aux_adjoint, ModelPd for cpdp_aux_adjoint_pd.
 #pragma once
 #include "cpdp_aux.cuh"
 
@@ -19,6 +22,16 @@ struct DiscWs {
     double* E;             // [B*N][NX][NP]  dF_k/dtheta
     double* Kth;           // [B*N][NU][NP]  feed-forward gains of the recursion (the feedback gains go to SolveArgs::Kf)
 };
+
+// The NQ per-problem constants as extra parameter columns (cpdp_aux_adjoint_pd, DESIGN.md §3.11): mode 2's three arrays for them,
+// in a separate caller-provided workspace.  The kernels of mode 2 are templates on the model's pdata derivatives PM (struct ModelPd
+// of the companion header, PM::NQ extra columns); NoPd (0 columns) is mode 2 and its adjoint with respect to theta and x0 alone.
+struct PdWs {
+    double* Hpd;           // [B*N][NZ][NQ]  d(grad_z (q_k + lam_{k+1}'F_k))/dpd
+    double* Epd;           // [B*N][NX][NQ]  dF_k/dpd
+    double* Kpd;           // [B*N][NU][NQ]  feed-forward gains
+};
+struct NoPd { static constexpr int NQ = 0; };
 
 CPDP_HD bool disc_usable(const int* solve_status, int b) {
     return !solve_status || (solve_status[b] != ST_NUMERIC && solve_status[b] != ST_RUNNING &&
@@ -52,22 +65,25 @@ CPDP_GLOBAL void __launch_bounds__(COMPACT_THREADS) k_disc_select(AuxArgs x, Sol
 }
 
 // ------------------------------------------------------------------------------------------------
-// k_stage_theta: NZ + NP threads per (problem, interval), TPC intervals per CTA.
+// k_stage_theta<PM>: NZ + NP + PM::NQ threads per (problem, interval), TPC intervals per CTA.
 // Thread j < NZ propagates column j of d(stage state)/d(x_k, u_k) through the 4S stages as k_stage_hessian does and parks its stage
 // rows in shared memory; thread NZ + p propagates column p of d(stage state)/dtheta (zero at the interval start) with Model::dir_th
 // and accumulates column p of  Hth = sum_s Sz_s' [Hess_zz(Ham_s) [Sth_s; 0] + Hess_ztheta(Ham_s)],  Ham_s = w_s c + mu_s'f, reading
-// the Sz rows of the stage.  Writes E = Sth at the interval end and Hth.
+// the Sz rows of the stage.  Writes E = Sth at the interval end and Hth.  PM::NQ > 0 (the pdata columns of cpdp_aux_adjoint_pd):
+// thread NZ + NP + q propagates column q of d(stage state)/dpd with PM::dir_pd the same way and writes E^pd, H^pd.
 // ------------------------------------------------------------------------------------------------
 #ifndef CPDP_THETA_THREADS
 #define CPDP_THETA_THREADS 64
 #endif
 constexpr int THETA_THREADS = CPDP_THETA_THREADS;
-constexpr int NZP = NZ + NP;                       // threads per interval
-constexpr int TPC = THETA_THREADS / NZP;           // intervals per CTA
-static_assert(TPC >= 1, "k_stage_theta: a CTA must hold the NZ + NP columns of one interval");
 static_assert(THETA_THREADS % 32 == 0, "k_stage_theta: whole warps");
 
-CPDP_GLOBAL void __launch_bounds__(THETA_THREADS) k_stage_theta(SolveArgs a, DiscWs d) {
+template <class PM>
+CPDP_GLOBAL void __launch_bounds__(THETA_THREADS) k_stage_theta(SolveArgs a, DiscWs d, PdWs pw) {
+    constexpr int XQ = PM::NQ;
+    constexpr int NZP = NZ + NP + XQ;              // threads per interval
+    constexpr int TPC = THETA_THREADS / NZP;       // intervals per CTA
+    static_assert(TPC >= 1, "k_stage_theta: a CTA must hold the NZ + NP + NQ columns of one interval");
     CPDP_SHARED double s_x[TPC][NX];
     CPDP_SHARED double s_mu[TPC][NX];
     CPDP_SHARED double s_u[TPC][NU];
@@ -79,6 +95,7 @@ CPDP_GLOBAL void __launch_bounds__(THETA_THREADS) k_stage_theta(SolveArgs a, Dis
     const int kk = tid / NZP, j = tid % NZP;
     const int kc = kk < TPC ? kk : 0;
     const bool zcol = j < NZ;                      // (x,u) column j, else theta column j - NZ
+    const bool qcol = XQ > 0 && j >= NZ + NP;      // pdata column j - NZ - NP
     const int total = *a.nact * a.N;
     const int ngroups = (total + TPC - 1) / TPC;
     const double DT = a.T / a.N / a.S;
@@ -113,6 +130,8 @@ CPDP_GLOBAL void __launch_bounds__(THETA_THREADS) k_stage_theta(SolveArgs a, Dis
         for (int i = 0; i < NX; ++i) { Sx[i] = (zcol && i == j) ? 1.0 : 0.0; df[i] = 0.0; }
         for (int i = 0; i < NU; ++i) du[i] = (zcol && NX + i == j) ? 1.0 : 0.0;
         for (int i = 0; i < NP; ++i) dth[i] = (!zcol && NZ + i == j) ? 1.0 : 0.0;
+        double dpd[XQ > 0 ? XQ : 1];
+        for (int i = 0; i < XQ; ++i) dpd[i] = (NZ + NP + i == j) ? 1.0 : 0.0;
         for (int i = 0; i < NZ; ++i) Hc[i] = 0.0;
 
         for (int s = 0; s < a.S; ++s) {
@@ -135,6 +154,9 @@ CPDP_GLOBAL void __launch_bounds__(THETA_THREADS) k_stage_theta(SolveArgs a, Dis
                     if (zcol) {
                         Model::dir(s_x[kc], s_u[kc], s_th[kc], s_pd[kc], s_mu[kc], bco[st] * DT, dX, du, df, hz);
                         for (int i = 0; i < NX; ++i) s_S[kc][j][i] = dX[i];
+                    } else if (qcol) {
+                        if constexpr (XQ > 0)
+                            PM::dir_pd(s_x[kc], s_u[kc], s_th[kc], s_pd[kc], s_mu[kc], bco[st] * DT, dX, du, dpd, df, hz);
                     } else {
                         Model::dir_th(s_x[kc], s_u[kc], s_th[kc], s_pd[kc], s_mu[kc], bco[st] * DT, dX, du, dth, df, hz);
                     }
@@ -155,7 +177,15 @@ CPDP_GLOBAL void __launch_bounds__(THETA_THREADS) k_stage_theta(SolveArgs a, Dis
             }
             for (int i = 0; i < NX; ++i) Sx[i] = Sn[i];
         }
-        if (mine && !zcol) {
+        if (mine && qcol) {
+            if constexpr (XQ > 0) {
+                const int q = j - NZ - NP;
+                double* E = pw.Epd + (size_t)gi * NX * XQ;
+                for (int i = 0; i < NX; ++i) E[i * XQ + q] = Sx[i];
+                double* Ht = pw.Hpd + (size_t)gi * NZ * XQ;
+                for (int i = 0; i < NZ; ++i) Ht[i * XQ + q] = Hc[i];
+            }
+        } else if (mine && !zcol) {
             const int p = j - NZ;
             double* E = d.E + (size_t)gi * NX * NP;
             for (int i = 0; i < NX; ++i) E[i * NP + p] = Sx[i];
@@ -166,39 +196,44 @@ CPDP_GLOBAL void __launch_bounds__(THETA_THREADS) k_stage_theta(SolveArgs a, Dis
 }
 
 // ------------------------------------------------------------------------------------------------
-// k_aux_discrete: one warp per problem (grid = B; problems with aux_status != 0 only write their zero loss row in phase 2).
+// k_aux_discrete<PM>: one warp per problem (grid = B; problems with aux_status != 0 only write their zero loss row in phase 2).
 // Phase 1, backward (k = N-1 .. 0), in the column style of k_newton_step: lane c owns column c of  G = [A B | E]  (NX x (NZ+NP)):
 //     Y[:, c] = V G[:, c] (+ W[:, c-NZ] for the theta columns),   Q[:, c] = [H | Hth][:, c] + [A B]' Y[:, c]
 //     Quu = L L' (lane 0; not positive definite -> aux_status 4),  gains  K = -Quu^{-1} Qux,  Kth = -Quu^{-1} Qu,theta
 //     V <- Qxx + Qxu K (symmetrised as in k_newton_step),  W <- Qx,theta + Qxu Kth
+// PM::NQ > 0: NQ more columns of G = [A B | E | E^pd] and Q ride along; W^pd starts at hxp = d(grad_x h)/dpd and the gains K^pd go
+// to pw.Kpd.  Every other column's arithmetic is that of NoPd.
 // Phase 2, forward: lane p < NP owns column p of dX/dtheta:  Ua_k = K Xa_k + Kth,  Xa_{k+1} = A Xa_k + B Ua_k + E_k,  Ua_N = Ua_{N-1};
 // then the loss and dL/dtheta of k_aux_forward's tail (same formula, same summation order).
 // ------------------------------------------------------------------------------------------------
 constexpr int DISC_THREADS = 32;
-constexpr int DCOL = NZ + NP;                      // columns of [A B | E] and [Q | Qtheta]
-constexpr int DCS = DCOL | 1;                      // odd row strides (conflict-free row reads by lane)
-constexpr int NPS_D = NP | 1;
 static_assert(NP <= DISC_THREADS, "k_aux_discrete maps one lane per column of dX/dtheta in the rollout");
 
-CPDP_GLOBAL void __launch_bounds__(DISC_THREADS) k_aux_discrete(AuxArgs x, SolveArgs a, DiscWs d, int phase) {
+template <class PM>
+CPDP_GLOBAL void __launch_bounds__(DISC_THREADS) k_aux_discrete(AuxArgs x, SolveArgs a, DiscWs d, int phase, PdWs pw) {
+    constexpr int XQ = PM::NQ;
+    constexpr int DCOL = NZ + NP + XQ;             // columns of [A B | E | E^pd] and [Q | Qtheta | Qpd]
+    constexpr int DCS = DCOL | 1;                  // odd row strides (conflict-free row reads by lane)
+    constexpr int NPS = (NP + XQ) | 1;
     const int b = blockIdx.x, lane = threadIdx.x;
     const int N = a.N;
     if (x.aux_status[b] != 0) {
-        if (phase == 2) {
+        if (XQ == 0 && phase == 2) {
             if (lane == 0) x.loss[b] = 0.0;
             for (int i = lane; i < NP; i += DISC_THREADS) x.dtheta[(size_t)b * NP + i] = 0.0;
         }
         return;
     }
     const size_t ib = (size_t)b * N;
-    if (phase == 1) {
-        CPDP_SHARED double s_V[NX * NXS], s_W[NX * NPS_D], s_G[NX * DCS], s_Y[NX * DCS], s_Q[NZ * DCS], s_K[NU * DCS];
+    if (XQ > 0 || phase == 1) {
+        CPDP_SHARED double s_V[NX * NXS], s_W[NX * NPS], s_G[NX * DCS], s_Y[NX * DCS], s_Q[NZ * DCS], s_K[NU * DCS];
         CPDP_SHARED double s_hxx[NX * NX], s_hxe[NX * NP], s_L[NU * NU];
         CPDP_SHARED int s_flag;
         if (lane == 0) {
             PdBuf pdb;
             const double* pd = pd_at(pdata_of(a, b), grid_time(a.T, N, N), pdb);
             Model::term2(a.X + ((size_t)b * (N + 1) + N) * NX, theta_of(a, b), pd, s_hxx, s_hxe);
+            if constexpr (XQ > 0) PM::term2_pd(a.X + ((size_t)b * (N + 1) + N) * NX, theta_of(a, b), pd, s_G);     // hxp, parked in G
             s_flag = 0;
         }
         NWT_SYNC();
@@ -215,24 +250,31 @@ CPDP_GLOBAL void __launch_bounds__(DISC_THREADS) k_aux_discrete(AuxArgs x, Solve
                 }
             }
         }
-        for (int q = lane; q < NX * NP; q += DISC_THREADS) s_W[(q / NP) * NPS_D + q % NP] = s_hxe[q];
+        for (int q = lane; q < NX * NP; q += DISC_THREADS) s_W[(q / NP) * NPS + q % NP] = s_hxe[q];
+        if constexpr (XQ > 0) {
+            for (int q = lane; q < NX * XQ; q += DISC_THREADS) s_W[(q / XQ) * NPS + NP + q % XQ] = s_G[q];     // W^pd starts at hxp
+        }
         NWT_SYNC();
         for (int k = N - 1; k >= 0; --k) {
             const double* ABg = a.AB + (ib + k) * NX * NZ;
             const double* Hg = a.H + (ib + k) * NZ * NZ;
             const double* Eg = d.E + (ib + k) * NX * NP;
             const double* Htg = d.Hth + (ib + k) * NZ * NP;
+            const double* Epg = pw.Epd + (ib + k) * NX * XQ;
+            const double* Hpg = pw.Hpd + (ib + k) * NZ * XQ;
             for (int c = lane; c < DCOL; c += DISC_THREADS) {
-                NWT_UNROLL for (int e = 0; e < NX; ++e) s_G[e * DCS + c] = (c < NZ) ? ABg[e * NZ + c] : Eg[e * NP + c - NZ];
+                NWT_UNROLL for (int e = 0; e < NX; ++e)
+                    s_G[e * DCS + c] = (c < NZ) ? ABg[e * NZ + c] : (c < NZ + NP) ? Eg[e * NP + c - NZ] : Epg[e * XQ + c - NZ - NP];
             }
             NWT_SYNC();
             for (int c = lane; c < DCOL; c += DISC_THREADS) {
                 double y[NX];
-                NWT_UNROLL for (int i = 0; i < NX; ++i) y[i] = (c < NZ) ? 0.0 : s_W[i * NPS_D + c - NZ];
+                NWT_UNROLL for (int i = 0; i < NX; ++i) y[i] = (c < NZ) ? 0.0 : s_W[i * NPS + c - NZ];
                 nwt_mac<NX>(s_V, NXS, s_G + c, DCS, NX, y);                    // (V symmetric: row e of V is column e)
                 NWT_UNROLL for (int i = 0; i < NX; ++i) s_Y[i * DCS + c] = y[i];
                 double q[NZ];
-                NWT_UNROLL for (int r_ = 0; r_ < NZ; ++r_) q[r_] = (c < NZ) ? Hg[r_ * NZ + c] : Htg[r_ * NP + c - NZ];
+                NWT_UNROLL for (int r_ = 0; r_ < NZ; ++r_)
+                    q[r_] = (c < NZ) ? Hg[r_ * NZ + c] : (c < NZ + NP) ? Htg[r_ * NP + c - NZ] : Hpg[r_ * XQ + c - NZ - NP];
                 if constexpr (HAS_BOUNDS) {
                     if (c < NZ) {                          // + Sigma_k (diagonal) of the barrier-perturbed KKT system
                         const size_t o = ((size_t)b * (N + 1) + k) * NZ + c;
@@ -264,7 +306,8 @@ CPDP_GLOBAL void __launch_bounds__(DISC_THREADS) k_aux_discrete(AuxArgs x, Solve
                 NWT_UNROLL for (int r_ = 0; r_ < NU; ++r_) {
                     s_K[r_ * DCS + c] = -rhs[r_];
                     if (c < NX) a.Kf[(ib + k) * NU * NX + r_ * NX + c] = -rhs[r_];
-                    else d.Kth[(ib + k) * NU * NP + r_ * NP + c - NZ] = -rhs[r_];
+                    else if (c < NZ + NP) d.Kth[(ib + k) * NU * NP + r_ * NP + c - NZ] = -rhs[r_];
+                    else pw.Kpd[(ib + k) * NU * XQ + r_ * XQ + c - NZ - NP] = -rhs[r_];
                 }
             }
             NWT_SYNC();
@@ -290,7 +333,7 @@ CPDP_GLOBAL void __launch_bounds__(DISC_THREADS) k_aux_discrete(AuxArgs x, Solve
                 }
                 // (every read of the old V and W of this stage lies before the barriers above)
                 if (c < NX) { NWT_UNROLL for (int r_ = 0; r_ < NX; ++r_) s_V[r_ * NXS + c] = vnew[r_]; }
-                else { NWT_UNROLL for (int r_ = 0; r_ < NX; ++r_) s_W[r_ * NPS_D + c - NZ] = vnew[r_]; }
+                else { NWT_UNROLL for (int r_ = 0; r_ < NX; ++r_) s_W[r_ * NPS + c - NZ] = vnew[r_]; }
             }
             NWT_SYNC();
         }
