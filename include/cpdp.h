@@ -21,7 +21,9 @@
 extern "C" {
 #endif
 
-/* per-problem solver status written by cpdp_solve; CPDP_INFEASIBLE: x0 is not strictly inside a finite state bound */
+/* per-problem solver status written by cpdp_solve; CPDP_INFEASIBLE: x0 is not strictly inside a finite state bound of its problem,
+ * or (bounds that depend on pdata) some component of the problem has lb(pdata) >= ub(pdata).  Set at the start, cold or warm;
+ * every auxiliary mode skips such a problem and cpdp_pack_rows counts it as failed. */
 enum { CPDP_RUNNING = 0, CPDP_CONVERGED = 1, CPDP_MAXITER = 2, CPDP_LINESEARCH = 3, CPDP_NUMERIC = 4, CPDP_INFEASIBLE = 5 };
 
 /* Model dimensions compiled into this library (COCSys.n_state / n_control / n_auxvar, CPDP.py:17,22,36);
@@ -32,9 +34,16 @@ int cpdp_model_dims(int* n, int* m, int* r, int* q);
 int cpdp_riccati_state_dim(void);
 
 /* Box bounds compiled into this library (COCSys.setStateVariable / setControlVariable bounds): lb[n+m], ub[n+m] host arrays,
- * states then controls, -1e20 / +1e20 where there is none.  Returns 1 when some bound is finite, 0 otherwise.  A bounded library's
- * cpdp_solve runs a primal-dual interior-point (barrier) method and keeps the bound multipliers in the workspace. */
+ * states then controls, -1e20 / +1e20 where there is none.  Returns 1 when some bound is finite, 0 otherwise, and 2 when some
+ * bound is an expression of the per-problem constants pdata (those entries read NaN; cpdp_eval_bounds gives their values).  A
+ * bounded library's cpdp_solve runs a primal-dual interior-point (barrier) method and keeps the bound multipliers in the
+ * workspace; with pdata bounds each problem uses its own, and a bound evaluating to +-1e20 or beyond is no bound for that problem. */
 int cpdp_bounds(double* lb, double* ub);
+
+/* Bounds of B problems: device arrays lb[B][n+m], ub[B][n+m] evaluated at pdata[B][q] (device; may be null when no bound depends
+ * on it).  Any library: constant bounds are broadcast, unbounded components read -1e20 / +1e20.  -1: lb or ub null or B <= 0;
+ * -8: pdata null although some bound depends on it. */
+int cpdp_eval_bounds(const double* pdata, int B, double* lb, double* ub, void* stream);
 
 /* Copy the bound multipliers z_L, z_U [B][N+1][n+m] (row N: the final state's entries; 0 where there is no bound) and the barrier
  * parameter mu[B] out of the workspace a bounded cpdp_solve left them in (get), or into it (set).  cpdp_aux mode 2 reads them
@@ -141,7 +150,8 @@ size_t cpdp_pdata_workspace_bytes(int B, int N);
  * per-problem constants (DESIGN.md §3.11).  The q constants ride along as q extra parameter columns of the same sweep; pd_ws
  * (cpdp_pdata_workspace_bytes(B, N) bytes, -3 if smaller) holds their stage derivatives and gains.  theta_bar and x0_bar are those
  * of cpdp_aux_adjoint; same zero-row rule and argument-error codes, plus -14 (the model has no per-problem constants) and -15 (the
- * library was built without the pdata derivatives, or n + m + r + q > 32). */
+ * library was built without the pdata derivatives, or n + m + r + q > 32).  When bounds depend on pdata, pdata_bar includes the
+ * bounds' part, -(Sigma_L dlb/dpdata + Sigma_U dub/dpdata) in the differentiated barrier KKT system (DESIGN.md §3.12). */
 int cpdp_aux_adjoint_pd(void* ws, size_t ws_bytes, void* pd_ws, size_t pd_ws_bytes, int B, int N, int S, double T,
                         const double* theta, int theta_stride, const double* pdata,
                         const double* X, const double* U, const double* Lam, const int* solve_status,

@@ -103,7 +103,9 @@ class COCSys:
 
     def setStateVariable(self, state, state_lb=[], state_ub=[]):
         """CPDP.py:20-31.  Bounds of the wrong length mean "none" (+-1e20), as in the reference; finite bounds are compiled
-        into the model and enforced by the solver's barrier method (DESIGN.md §3.8)."""
+        into the model and enforced by the solver's barrier method (DESIGN.md §3.8).  A bound entry may also be an SX / sympy
+        expression of the problem variables (setProblemVariable): each problem of a batch then has its own bound, evaluated at its
+        pdata (DESIGN.md §3.12)."""
         self.state = state
         self.n_state = self.state.numel()
         self.state_lb, self.state_ub = self._check_bounds(state_lb, state_ub, self.n_state)
@@ -118,10 +120,10 @@ class COCSys:
 
     @staticmethod
     def _check_bounds(lb, ub, n):
-        lb = list(numpy.asarray(lb, dtype=float).ravel())
-        ub = list(numpy.asarray(ub, dtype=float).ravel())
-        lb, ub = codegen.normalize_bounds(lb, ub, n)
+        lb, ub = codegen.normalize_bounds(codegen.bound_entries(lb), codegen.bound_entries(ub), n)
         for i, (lo, hi) in enumerate(zip(lb, ub)):
+            if codegen.is_symbolic(lo) or codegen.is_symbolic(hi):
+                continue                    # checked per problem at run time: lb(pdata) >= ub(pdata) gives CPDP_INFEASIBLE
             if not lo < hi:
                 raise ValueError("bound %d: lower bound %r is not below upper bound %r (fixed variables are not supported)"
                                  % (i, lo, hi))
@@ -132,8 +134,30 @@ class COCSys:
 
     @property
     def bounded(self):
-        """True when some state or control bound is finite."""
-        return any(abs(v) < 1e19 for v in self.state_lb + self.state_ub + self.control_lb + self.control_ub)
+        """True when some state or control bound is finite or an expression of the problem variables."""
+        return any(codegen.is_symbolic(v) or abs(v) < 1e19 for v in self.state_lb + self.state_ub + self.control_lb + self.control_ub)
+
+    @property
+    def bounds_depend_on_pdata(self):
+        """True when some bound is an expression of the problem variables (its value differs per problem)."""
+        return codegen.bounds_symbolic(self._bounds())
+
+    def boundsBatch(self, pdata=None):
+        """Evaluated bounds of a batch: device arrays (lb, ub) of shape [B, n+m] (states then controls; +-1e20 for none) at
+        pdata [B, q] (cpdp_eval_bounds).  For bounds that do not depend on pdata, B is pdata's row count, or 1 without pdata."""
+        lib = self.build()
+        mem = self._device()
+        pd = None
+        if pdata is not None:
+            pd = mem.from_host(numpy.asarray(pdata, dtype=float).reshape(-1, self.n_pvar) if not hasattr(pdata, 'data_ptr')
+                               else pdata)
+        elif self.bounds_depend_on_pdata:
+            raise ValueError("the bounds depend on the problem variables: pass pdata [B,%d]" % self.n_pvar)
+        B = int(pd.shape[0]) if pd is not None else 1
+        nz = self.n_state + self.n_control
+        lb, ub = mem.empty((B, nz)), mem.empty((B, nz))
+        lib.eval_bounds(mem.ptr(pd), B, mem.ptr(lb), mem.ptr(ub), mem.stream())
+        return lb, ub
 
     def setProblemVariable(self, pvar):
         """Extension: symbols that are per-problem constants (e.g. a goal position) — not learnable, not states.
@@ -221,14 +245,18 @@ class COCSys:
                                                     time=getattr(self, 'time', None), bounds=self._bounds())
         self.codegen_info = info
         pd_text, _ = codegen.generate_pdata_header(name or self.sys_name, self.state, self.control, self.auxvar, self.dyn,
-                                                   self.path_cost, self.final_cost, self.pvar, time=getattr(self, 'time', None))
+                                                   self.path_cost, self.final_cost, self.pvar, time=getattr(self, 'time', None),
+                                                   bounds=self._bounds())
         libname = name if name is not None else "m" + info["hash"]
         so = _capi.build_model_library(libname, text, force=force, verbose=verbose, pd_header_text=pd_text)
         self._lib = _capi.CpdpLib(so)
         assert (self._lib.n, self._lib.m, self._lib.r, self._lib.q) == \
             (self.n_state, self.n_control, self.n_auxvar, self.n_pvar)
-        assert (self._lib.has_bounds, self._lib.lb, self._lib.ub) == \
-            (self.bounded, self.state_lb + self.control_lb, self.state_ub + self.control_ub)
+        # (an entry that depends on pdata reads NaN in the library)
+        sym = lambda v: float("nan") if codegen.is_symbolic(v) else v
+        assert (self._lib.has_bounds, self._lib.bounds_pd) == (self.bounded, self.bounds_depend_on_pdata)
+        assert numpy.array_equal(self._lib.lb, [sym(v) for v in self.state_lb + self.control_lb], equal_nan=True) and \
+            numpy.array_equal(self._lib.ub, [sym(v) for v in self.state_ub + self.control_ub], equal_nan=True)
         return self._lib
 
     def _device(self):

@@ -155,6 +155,8 @@ class CpdpLib:
         L.cpdp_optim_step.restype = _i
         L.cpdp_bounds.argtypes = [ctypes.POINTER(_d), ctypes.POINTER(_d)]
         L.cpdp_bounds.restype = _i
+        L.cpdp_eval_bounds.argtypes = [_vp, _i, _vp, _vp, _vp]
+        L.cpdp_eval_bounds.restype = _i
         for fn in (L.cpdp_get_bound_multipliers, L.cpdp_set_bound_multipliers):
             fn.argtypes = [_vp, _sz, _i, _i, _i, _vp, _vp, _vp, _vp]
             fn.restype = _i
@@ -170,7 +172,9 @@ class CpdpLib:
         self.ncounters = int(L.cpdp_num_counters())
         self.has_bdf = bool(L.cpdp_has_bdf())
         lb, ub = (_d * (self.n + self.m))(), (_d * (self.n + self.m))()
-        self.has_bounds = bool(L.cpdp_bounds(lb, ub))
+        nb = L.cpdp_bounds(lb, ub)
+        self.has_bounds = bool(nb)
+        self.bounds_pd = nb == 2                       # some bound depends on pdata (those entries read NaN)
         self.lb, self.ub = list(lb), list(ub)          # states then controls, +-1e20 for none
 
     def check(self, rc, what):
@@ -220,6 +224,9 @@ class CpdpLib:
         self.check(self.L.cpdp_aux_adjoint_pd(ws, ws_bytes, pd_ws, pd_ws_bytes, B, N, S, T, theta, theta_stride, pdata, X, U, Lam,
                                               solve_status, Xbar, Ubar, theta_bar, x0_bar, pdata_bar, aux_status, stream),
                    "cpdp_aux_adjoint_pd")
+
+    def eval_bounds(self, pdata, B, lb, ub, stream):
+        self.check(self.L.cpdp_eval_bounds(pdata, B, lb, ub, stream), "cpdp_eval_bounds")
 
     def get_bound_multipliers(self, ws, ws_bytes, B, N, S, Zl, Zu, mu, stream):
         self.check(self.L.cpdp_get_bound_multipliers(ws, ws_bytes, B, N, S, Zl, Zu, mu, stream), "cpdp_get_bound_multipliers")

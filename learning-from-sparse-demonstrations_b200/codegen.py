@@ -24,7 +24,7 @@ import hashlib
 import sympy as sp
 from sympy.printing.c import C99CodePrinter
 
-from .sx import _to_matrix
+from .sx import SX, _to_matrix
 
 
 class _Printer(C99CodePrinter):
@@ -100,18 +100,80 @@ def _sparse_tables(name, M):
 BOUND_INF = 1e20          # the reference's "no bound" (CPDP.py:24-29); |bound| >= 1e19 counts as none
 
 
+def is_symbolic(v):
+    """True for a bound entry that is an expression (of the per-problem constants), not a number."""
+    return isinstance(v, sp.Basic)
+
+
+def bound_entry(v):
+    """One bound entry as a float, or as a sympy expression when it has free symbols (an SX / sympy scalar)."""
+    if isinstance(v, SX):
+        assert v.m.shape == (1, 1), "a bound entry is a scalar"
+        v = v.m[0, 0]
+    if isinstance(v, sp.Basic):
+        return v if v.free_symbols else float(v)
+    return float(v)
+
+
+def bound_entries(v):
+    """A bound vector (list / array of numbers or scalar expressions, or an SX / sympy column) as a flat list of bound_entry."""
+    if isinstance(v, SX):
+        v = v.m
+    if isinstance(v, sp.MatrixBase):
+        return [bound_entry(e) for e in v]
+    if isinstance(v, (list, tuple)) or hasattr(v, "__array__"):
+        out = []
+        for e in (v.ravel() if hasattr(v, "ravel") else v):
+            out.extend(bound_entries(e) if isinstance(e, (list, tuple, SX, sp.MatrixBase)) else [bound_entry(e)])
+        return out
+    return [bound_entry(v)]
+
+
 def normalize_bounds(lb, ub, n):
-    """Lists of n lower / upper bounds with every absent or infinite entry replaced by -/+BOUND_INF."""
-    lb = [-BOUND_INF if v <= -1e19 else float(v) for v in (lb if len(lb) == n else [-BOUND_INF] * n)]
-    ub = [BOUND_INF if v >= 1e19 else float(v) for v in (ub if len(ub) == n else [BOUND_INF] * n)]
+    """Lists of n lower / upper bounds with every absent or infinite entry replaced by -/+BOUND_INF (expressions as they are)."""
+    lb = [v if is_symbolic(v) else -BOUND_INF if v <= -1e19 else float(v) for v in (lb if len(lb) == n else [-BOUND_INF] * n)]
+    ub = [v if is_symbolic(v) else BOUND_INF if v >= 1e19 else float(v) for v in (ub if len(ub) == n else [BOUND_INF] * n)]
     return lb, ub
 
 
-def _bounds_block(bounds, n, m):
+def bounds_symbolic(bounds):
+    """True when some entry of (state_lb, state_ub, control_lb, control_ub) is an expression."""
+    return bounds is not None and any(is_symbolic(v) for part in bounds for v in part)
+
+
+def _bound_exprs(bounds, e):
+    """The four bound lists with every expression in the generated code's names (pd[i]); rejects an expression that uses
+    anything but the per-problem constants."""
+    names = ("state_lb", "state_ub", "control_lb", "control_ub")
+    kinds = [("state", e["sym_x"]), ("control", e["sym_u"]), ("auxvar (theta)", e["sym_th"]), ("time", e["tv"])]
+    out = []
+    for nm, part in zip(names, bounds):
+        row = []
+        for i, v in enumerate(part):
+            if is_symbolic(v):
+                for kind, syms in kinds:
+                    bad = v.free_symbols & set(syms)
+                    if bad:
+                        raise ValueError("%s[%d] = %s depends on the %s variable(s) %s: a bound may use only the problem variables "
+                                         "(setProblemVariable) and constants" % (nm, i, v, kind, sorted(map(str, bad))))
+                extra = v.free_symbols - set(e["sym_pd"])
+                if extra:
+                    raise ValueError("%s[%d] = %s has free symbols %s that are not problem variables (setProblemVariable)"
+                                     % (nm, i, v, sorted(map(str, extra))))
+                v = v.subs(dict(zip(e["sym_pd"], e["ps"])))
+            row.append(v)
+        out.append(row)
+    return out
+
+
+def _bounds_block(bounds, n, m, e=None):
     """Model members of the box bounds on the states and controls; empty text when no bound is finite, so that an unbounded
-    model's header does not change."""
+    model's header does not change.  Bounds with expressions of the per-problem constants (``e``: _model_exprs) give BOUNDS_PD
+    and bound functions of pd."""
     if bounds is None:
         return ""
+    if bounds_symbolic(bounds):
+        return _bounds_block_pd(bounds, n, m, e)
     xlb, xub, ulb, uub = bounds
     if all(v <= -1e19 for v in list(xlb) + list(ulb)) and all(v >= 1e19 for v in list(xub) + list(uub)):
         return ""
@@ -124,6 +186,23 @@ def _bounds_block(bounds, n, m):
         for i in range(len(v) - 2, -1, -1):
             expr = "i == %d ? %r : %s" % (i, v[i], expr)
         lines.append("    CPDP_HD static constexpr double %s(int i) { return %s; }" % (nm, expr))
+    return "\n".join(lines) + "\n"
+
+
+def _bounds_block_pd(bounds, n, m, e):
+    xlb, xub, ulb, uub = bounds
+    xlb, xub = normalize_bounds(xlb, xub, n)
+    ulb, uub = normalize_bounds(ulb, uub, m)
+    xlb, xub, ulb, uub = _bound_exprs((xlb, xub, ulb, uub), e)
+    lines = ["    static constexpr int HAS_BOUNDS = 1;      // box bounds (+-1e20: none), read by the kernels' barrier method",
+             "    static constexpr int BOUNDS_PD = 1;       // some bound is an expression of the per-problem constants pd"]
+    val = lambda v: "(%s)" % _pr.doprint(v) if is_symbolic(v) else repr(v)
+    for nm, v in (("XLB", xlb), ("XUB", xub), ("ULB", ulb), ("UUB", uub)):
+        # a chain of selects, as for constant bounds; pd: the problem's constants (never the time slot)
+        expr = val(v[-1])
+        for i in range(len(v) - 2, -1, -1):
+            expr = "i == %d ? %s : %s" % (i, val(v[i]), expr)
+        lines.append("    CPDP_HD static double %s(int i, const double* __restrict__ pd) { (void)pd; return %s; }" % (nm, expr))
     return "\n".join(lines) + "\n"
 
 
@@ -170,7 +249,7 @@ def _model_exprs(state, control, auxvar, dyn, path_cost, final_cost, pdata, time
     dz = sp.Matrix(dxs + dus)
 
     return dict(n=n, m=m, r=r, nq=nq, nz=nz, tv=tv, f=f, c=c, h=h, xs=xs, us=us, ts=ts, ps=ps, z=z, mus=mus, w=w,
-                fz=fz, Hz=Hz, Hzz=Hzz, dz=dz)
+                fz=fz, Hz=Hz, Hzz=Hzz, dz=dz, sym_x=x, sym_u=u, sym_th=th, sym_pd=pdv[:nq])
 
 
 def generate_model_header(name, state, control, auxvar, dyn, path_cost, final_cost, pdata=None, time=None, bounds=None):
@@ -179,7 +258,8 @@ def generate_model_header(name, state, control, auxvar, dyn, path_cost, final_co
     ``time``: the explicit time variable of a COCSys_TimeVarying model (CPDP.py:434); the generated functions read it as
     one more constant, pd[nq], which the kernels fill in (the node time t_k in the RK4 map, the true t in the sweeps).
     ``bounds``: optional (state_lb, state_ub, control_lb, control_ub); the header gets HAS_BOUNDS and the four bound tables
-    only when some bound is finite."""
+    only when some bound is finite.  An entry may be an expression of the per-problem constants (DESIGN.md §3.12): then the
+    header gets BOUNDS_PD and bound functions XLB(i, pd) ..."""
     e = _model_exprs(state, control, auxvar, dyn, path_cost, final_cost, pdata, time)
     n, m, r, nq, nz, tv = e["n"], e["m"], e["r"], e["nq"], e["nz"], e["tv"]
     f, c, h, xs, us, ts, z, mus, w = (e[k] for k in ("f", "c", "h", "xs", "us", "ts", "z", "mus", "w"))
@@ -299,19 +379,21 @@ struct Model {{
 {tables}
 {parts}
 }};
-""".format(name=name, nz=nz, has_time=len(tv), bounds=_bounds_block(bounds, n, m), offs="\n".join(offs), tables=tables,
+""".format(name=name, nz=nz, has_time=len(tv), bounds=_bounds_block(bounds, n, m, e), offs="\n".join(offs), tables=tables,
            parts="\n\n".join(parts), **info)
     info["hash"] = hashlib.sha1(text.encode()).hexdigest()[:16]
     return text, info
 
 
-def generate_pdata_header(name, state, control, auxvar, dyn, path_cost, final_cost, pdata=None, time=None):
+def generate_pdata_header(name, state, control, auxvar, dyn, path_cost, final_cost, pdata=None, time=None, bounds=None):
     """Companion header ``model_<name>_pd.cuh``: ``struct ModelPd`` with the derivatives with respect to the NQ per-problem
     constants that the pdata adjoint (cpdp_aux_adjoint_pd, DESIGN.md §3.11) needs.  A separate file, so that the model header and
     its hash do not change.  Only the user constants pd[0..NQ-1] are differentiated; the time of a time-varying model, pd[NQ], is
     not a pdata column.  Returns (header_text, info dict).
       dir_pd(x,u,th,pd,mu,w,dx,du,dpd, df[n], hz[nz])   df = fz dz + f_pd dpd ; hz = Hess_z(Ham) dz + Hess_zpd(Ham) dpd
       term2_pd(x,th,pd, hxp[n*nq])                     d(grad_x h)/dpd, row-major
+      dbounds(pd, dlb[nz*nq], dub[nz*nq])              d(bounds)/dpd, row-major, when some bound is an expression of pd
+                                                       (BOUNDS_PD = 1; ``bounds`` as for generate_model_header)
     For NQ = 0 the struct holds NQ only."""
     e = _model_exprs(state, control, auxvar, dyn, path_cost, final_cost, pdata, time)
     n, nq, nz = e["n"], e["nq"], e["nz"]
@@ -332,6 +414,20 @@ def generate_pdata_header(name, state, control, auxvar, dyn, path_cost, final_co
         body, info["ops_term2_pd"] = _emit_body([("hxp[%d]" % (i * nq + j), hxp[i, j]) for i in range(n) for j in range(nq)])
         parts.append("    CPDP_HD static void term2_pd(const double* __restrict__ x, const double* __restrict__ th, "
                      "const double* __restrict__ pd, double* __restrict__ hxp) {\n%s\n    }" % body)
+    if nq > 0 and bounds_symbolic(bounds):
+        xlb, xub = normalize_bounds(bounds[0], bounds[1], e["n"])
+        ulb, uub = normalize_bounds(bounds[2], bounds[3], e["m"])
+        xlb, xub, ulb, uub = _bound_exprs((xlb, xub, ulb, uub), e)
+        pq = e["ps"][:nq]
+        assigns = []
+        for tag, v in (("dlb", xlb + ulb), ("dub", xub + uub)):
+            for j in range(nz):
+                for q in range(nq):
+                    assigns.append(("%s[%d]" % (tag, j * nq + q), sp.diff(v[j], pq[q]) if is_symbolic(v[j]) else sp.Integer(0)))
+        body, info["ops_dbounds"] = _emit_body(assigns)
+        parts.insert(0, "    static constexpr int BOUNDS_PD = 1;       // the bounds depend on pd: dbounds gives their Jacobians")
+        parts.append("    CPDP_HD static void dbounds(const double* __restrict__ pd, double* __restrict__ dlb, double* __restrict__ dub) {"
+                     "\n    (void)pd;\n%s\n    }" % body)
     text = """// GENERATED by lfsd_b200/codegen.py -- do not edit.  model: {name}, derivatives with respect to the per-problem constants
 #pragma once
 #include "cpdp_port.h"

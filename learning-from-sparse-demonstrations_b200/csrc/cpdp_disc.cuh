@@ -226,14 +226,19 @@ CPDP_GLOBAL void __launch_bounds__(DISC_THREADS) k_aux_discrete(AuxArgs x, Solve
     }
     const size_t ib = (size_t)b * N;
     if (XQ > 0 || phase == 1) {
+        // pdata columns of a model whose bounds depend on pdata: the bound term -(Sigma_L dlb/dpd + Sigma_U dub/dpd) of every row
+        constexpr bool BPD = XQ > 0 && BOUNDS_PD;
         CPDP_SHARED double s_V[NX * NXS], s_W[NX * NPS], s_G[NX * DCS], s_Y[NX * DCS], s_Q[NZ * DCS], s_K[NU * DCS];
         CPDP_SHARED double s_hxx[NX * NX], s_hxe[NX * NP], s_L[NU * NU];
+        CPDP_SHARED double s_db[BPD ? 2 * NZ * XQ : 1], s_sg[BPD ? 2 * NZ : 1];   // [dlb/dpd | dub/dpd] (NZ x NQ), [Sigma_L | Sigma_U]
         CPDP_SHARED int s_flag;
+        const double* pdb0 = pdata_of(a, b);       // the bounds' constants (never the time slot)
         if (lane == 0) {
             PdBuf pdb;
-            const double* pd = pd_at(pdata_of(a, b), grid_time(a.T, N, N), pdb);
+            const double* pd = pd_at(pdb0, grid_time(a.T, N, N), pdb);
             Model::term2(a.X + ((size_t)b * (N + 1) + N) * NX, theta_of(a, b), pd, s_hxx, s_hxe);
             if constexpr (XQ > 0) PM::term2_pd(a.X + ((size_t)b * (N + 1) + N) * NX, theta_of(a, b), pd, s_G);     // hxp, parked in G
+            if constexpr (BPD) PM::dbounds(pdb0, s_db, s_db + NZ * XQ);        // once per problem: the bounds do not vary by node
             s_flag = 0;
         }
         NWT_SYNC();
@@ -245,14 +250,24 @@ CPDP_GLOBAL void __launch_bounds__(DISC_THREADS) k_aux_discrete(AuxArgs x, Solve
                 if (i == c) {
                     const size_t o = ((size_t)b * (N + 1) + N) * NZ + i;
                     double sg, bg;
-                    bnd_terms(i, a.X[((size_t)b * (N + 1) + N) * NX + i], a.zL[o], a.zU[o], 0.0, sg, bg);
+                    bnd_terms(i, pdb0, a.X[((size_t)b * (N + 1) + N) * NX + i], a.zL[o], a.zU[o], 0.0, sg, bg);
                     s_V[i * NXS + c] += sg;
                 }
             }
         }
         for (int q = lane; q < NX * NP; q += DISC_THREADS) s_W[(q / NP) * NPS + q % NP] = s_hxe[q];
         if constexpr (XQ > 0) {
-            for (int q = lane; q < NX * XQ; q += DISC_THREADS) s_W[(q / XQ) * NPS + NP + q % XQ] = s_G[q];     // W^pd starts at hxp
+            for (int q = lane; q < NX * XQ; q += DISC_THREADS) {
+                double v = s_G[q];                                                  // W^pd starts at hxp
+                if constexpr (BPD) {                                                // - Sigma_L dlb/dpd - Sigma_U dub/dpd of x_N
+                    const int i = q / XQ;
+                    const size_t o = ((size_t)b * (N + 1) + N) * NZ + i;
+                    double sgl, sgu;
+                    bnd_sigmas(i, pdb0, a.X[((size_t)b * (N + 1) + N) * NX + i], a.zL[o], a.zU[o], sgl, sgu);
+                    v -= sgl * s_db[q] + sgu * s_db[NZ * XQ + q];
+                }
+                s_W[(q / XQ) * NPS + NP + q % XQ] = v;
+            }
         }
         NWT_SYNC();
         for (int k = N - 1; k >= 0; --k) {
@@ -265,6 +280,13 @@ CPDP_GLOBAL void __launch_bounds__(DISC_THREADS) k_aux_discrete(AuxArgs x, Solve
             for (int c = lane; c < DCOL; c += DISC_THREADS) {
                 NWT_UNROLL for (int e = 0; e < NX; ++e)
                     s_G[e * DCS + c] = (c < NZ) ? ABg[e * NZ + c] : (c < NZ + NP) ? Eg[e * NP + c - NZ] : Epg[e * XQ + c - NZ - NP];
+                if constexpr (BPD) {
+                    if (c < NZ) {                          // the two parts of Sigma_k of row c, for the pdata columns below
+                        const size_t o = ((size_t)b * (N + 1) + k) * NZ + c;
+                        const double w = (c < NX) ? a.X[((size_t)b * (N + 1) + k) * NX + c] : a.U[((size_t)b * (N + 1) + k) * NU + c - NX];
+                        bnd_sigmas(c, pdb0, w, a.zL[o], a.zU[o], s_sg[c], s_sg[NZ + c]);
+                    }
+                }
             }
             NWT_SYNC();
             for (int c = lane; c < DCOL; c += DISC_THREADS) {
@@ -280,8 +302,15 @@ CPDP_GLOBAL void __launch_bounds__(DISC_THREADS) k_aux_discrete(AuxArgs x, Solve
                         const size_t o = ((size_t)b * (N + 1) + k) * NZ + c;
                         const double w = (c < NX) ? a.X[((size_t)b * (N + 1) + k) * NX + c] : a.U[((size_t)b * (N + 1) + k) * NU + c - NX];
                         double sg, bg;
-                        bnd_terms(c, w, a.zL[o], a.zU[o], 0.0, sg, bg);
+                        bnd_terms(c, pdb0, w, a.zL[o], a.zU[o], 0.0, sg, bg);
                         NWT_UNROLL for (int r_ = 0; r_ < NZ; ++r_) if (r_ == c) q[r_] += sg;
+                    }
+                }
+                if constexpr (BPD) {
+                    if (c >= NZ + NP) {                    // pdata column: - Sigma_L dlb/dpd - Sigma_U dub/dpd (DESIGN.md §3.12)
+                        const int qc = c - NZ - NP;
+                        NWT_UNROLL for (int r_ = 0; r_ < NZ; ++r_)
+                            q[r_] -= s_sg[r_] * s_db[r_ * XQ + qc] + s_sg[NZ + r_] * s_db[NZ * XQ + r_ * XQ + qc];
                     }
                 }
                 nwt_mac<NZ>(s_G, DCS, s_Y + c, DCS, NX, q);                    // (my own column of Y: no barrier needed)

@@ -27,14 +27,23 @@ constexpr int FILTER_CAP = 256;        // filter entries per problem (one is add
 enum Status { ST_RUNNING = 0, ST_CONVERGED = 1, ST_MAXITER = 2, ST_LINESEARCH = 3, ST_NUMERIC = 4, ST_INFEASIBLE = 5 };
 
 // Box bounds on the states and controls (DESIGN.md §3.8).  A model header defines HAS_BOUNDS and XLB / XUB / ULB / UUB only when
-// some bound is finite; every other model takes the unbounded code path unchanged.
+// some bound is finite; every other model takes the unbounded code path unchanged.  A model with BOUNDS_PD = 1 (DESIGN.md §3.12)
+// has bounds that are expressions of its per-problem constants: XLB(i, pd) ...; every call site passes its problem's constants pd
+// (the user constants, never the time slot), which lo(j, pd) / hi(j, pd) of a constant-bound model ignore.
+template <class M, class = void> struct ModelBoundsPd { static constexpr int PD = 0; };
+template <class M> struct ModelBoundsPd<M, std::void_t<decltype(M::BOUNDS_PD)>> { static constexpr int PD = M::BOUNDS_PD; };
+
 template <class M, class = void> struct ModelBounds {
     static constexpr int HAS = 0;
+    static constexpr int PD = 0;
     CPDP_HD static double lo(int) { return -1e20; }
     CPDP_HD static double hi(int) { return 1e20; }
+    CPDP_HD static double lo(int, const double*) { return -1e20; }
+    CPDP_HD static double hi(int, const double*) { return 1e20; }
 };
 template <class M> struct ModelBounds<M, std::void_t<decltype(M::HAS_BOUNDS)>> {
     static constexpr int HAS = M::HAS_BOUNDS;
+    static constexpr int PD = ModelBoundsPd<M>::PD;
     // bound of component j of z = [x; u] (a chain of selects: no local-memory table for a lane-dependent j)
     CPDP_HD static double lo(int j) {
         double v = 0.0;
@@ -48,24 +57,53 @@ template <class M> struct ModelBounds<M, std::void_t<decltype(M::HAS_BOUNDS)>> {
         CPDP_PRAGMA_UNROLL(NU) for (int i = 0; i < NU; ++i) if (NX + i == j) v = M::UUB(i);
         return v;
     }
+    // the bound of problem constants pd (the same select chain over the model's expressions of pd)
+    CPDP_HD static double lo(int j, const double* pd) {
+        if constexpr (!PD) {
+            return lo(j);
+        } else {
+            double v = 0.0;
+            CPDP_PRAGMA_UNROLL(NX) for (int i = 0; i < NX; ++i) if (i == j) v = M::XLB(i, pd);
+            CPDP_PRAGMA_UNROLL(NU) for (int i = 0; i < NU; ++i) if (NX + i == j) v = M::ULB(i, pd);
+            return v;
+        }
+    }
+    CPDP_HD static double hi(int j, const double* pd) {
+        if constexpr (!PD) {
+            return hi(j);
+        } else {
+            double v = 0.0;
+            CPDP_PRAGMA_UNROLL(NX) for (int i = 0; i < NX; ++i) if (i == j) v = M::XUB(i, pd);
+            CPDP_PRAGMA_UNROLL(NU) for (int i = 0; i < NU; ++i) if (NX + i == j) v = M::UUB(i, pd);
+            return v;
+        }
+    }
 };
 constexpr int HAS_BOUNDS = ModelBounds<Model>::HAS;
+constexpr int BOUNDS_PD = ModelBounds<Model>::PD;      // bounds that depend on the per-problem constants
 CPDP_HD bool bnd_finite(double v) { return fabs(v) < 1e19; }
 
 // Barrier terms of component j (value w, multipliers zl, zu of its lower / upper bound, barrier parameter mu):
-// sig = zl/sl + zu/su (the diagonal Sigma), bg = -mu/sl + mu/su (the barrier's gradient), sl = w - lb, su = ub - w.
-CPDP_HD void bnd_terms(int j, double w, double zl, double zu, double mu, double& sig, double& bg) {
-    const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+// sig = zl/sl + zu/su (the diagonal Sigma), bg = -mu/sl + mu/su (the barrier's gradient), sl = w - lb, su = ub - w; pd: the
+// problem's constants.
+CPDP_HD void bnd_terms(int j, const double* pd, double w, double zl, double zu, double mu, double& sig, double& bg) {
+    const double lb = ModelBounds<Model>::lo(j, pd), ub = ModelBounds<Model>::hi(j, pd);
     sig = 0.0; bg = 0.0;
     if (bnd_finite(lb)) { const double s = w - lb; sig += zl / s; bg -= mu / s; }
     if (bnd_finite(ub)) { const double s = ub - w; sig += zu / s; bg += mu / s; }
+}
+// The two parts of bnd_terms' Sigma: sgl = zl/sl of the lower bound, sgu = zu/su of the upper one (0 for no finite bound).
+CPDP_HD void bnd_sigmas(int j, const double* pd, double w, double zl, double zu, double& sgl, double& sgu) {
+    const double lb = ModelBounds<Model>::lo(j, pd), ub = ModelBounds<Model>::hi(j, pd);
+    sgl = bnd_finite(lb) ? zl / (w - lb) : 0.0;
+    sgu = bnd_finite(ub) ? zu / (ub - w) : 0.0;
 }
 
 // Newton step of a bound multiplier z with slack s whose step is ds:  dz = mu/s - z - (z/s) ds.
 CPDP_HD double bnd_dz(double s, double z, double mu, double ds) { return mu / s - z - (z / s) * ds; }
 // ln of the slacks of component j at value w (the barrier's log terms; 0 for no finite bound)
-CPDP_HD double bnd_log(int j, double w) {
-    const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+CPDP_HD double bnd_log(int j, const double* pd, double w) {
+    const double lb = ModelBounds<Model>::lo(j, pd), ub = ModelBounds<Model>::hi(j, pd);
     double v = 0.0;
     if (bnd_finite(lb)) v += log(w - lb);
     if (bnd_finite(ub)) v += log(ub - w);
@@ -640,7 +678,7 @@ CPDP_D void newton_step_problem(const SolveArgs& a, const int b) {
             const int k = idx / NZ, j = idx % NZ;
             if (k == N && j >= NX) continue;
             const double w = (j < NX) ? X[(size_t)k * NX + j] : U[(size_t)k * NU + j - NX];
-            const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+            const double lb = ModelBounds<Model>::lo(j, pd0), ub = ModelBounds<Model>::hi(j, pd0);
             if (bnd_finite(lb)) { const double sl = w - lb, p = sl * zL[idx]; szmax = fmax(szmax, p); nszmin = fmax(nszmin, -p); lg += log(sl); }
             if (bnd_finite(ub)) { const double su = ub - w, p = su * zU[idx]; szmax = fmax(szmax, p); nszmin = fmax(nszmin, -p); lg += log(su); }
         }
@@ -674,7 +712,7 @@ CPDP_D void newton_step_problem(const SolveArgs& a, const int b) {
     // barrier terms of the final state (lane i: component i)
     double sgN = 0.0, bgN = 0.0;
     if constexpr (HAS_BOUNDS) {
-        if (isX) bnd_terms(jx, X[(size_t)N * NX + jx], zL[(size_t)N * NZ + jx], zU[(size_t)N * NZ + jx], mu, sgN, bgN);
+        if (isX) bnd_terms(jx, pd0, X[(size_t)N * NX + jx], zL[(size_t)N * NZ + jx], zU[(size_t)N * NZ + jx], mu, sgN, bgN);
     }
 
     // ---- Riccati factorisation with inertia correction (IPOPT Alg. IC)
@@ -710,7 +748,7 @@ CPDP_D void newton_step_problem(const SolveArgs& a, const int b) {
             const double gl = isZ ? gLg[jz] : 0.0;
             double sgk = 0.0, bgk = 0.0;                 // barrier terms of my component of z_k
             if constexpr (HAS_BOUNDS) {
-                if (isZ) bnd_terms(jz, jz < NX ? X[(size_t)k * NX + jz] : U[(size_t)k * NU + jz - NX], zL[(size_t)k * NZ + jz],
+                if (isZ) bnd_terms(jz, pd0, jz < NX ? X[(size_t)k * NX + jz] : U[(size_t)k * NU + jz - NX], zL[(size_t)k * NZ + jz],
                                    zU[(size_t)k * NZ + jz], mu, sgk, bgk);
             }
             if (isX) { s_dk[jx] = dk1[jx]; s_lk[jx] = lk1[jx]; }
@@ -885,7 +923,7 @@ CPDP_D void newton_step_problem(const SolveArgs& a, const int b) {
             if (k == N && j >= NX) continue;
             const double w = (j < NX) ? X[(size_t)k * NX + j] : U[(size_t)k * NU + j - NX];
             const double dw = (j < NX) ? dX[(size_t)k * NX + j] : dU[(size_t)k * NU + j - NX];
-            const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+            const double lb = ModelBounds<Model>::lo(j, pd0), ub = ModelBounds<Model>::hi(j, pd0);
             if (bnd_finite(lb)) {
                 const double sl = w - lb, dz = bnd_dz(sl, zL[idx], mu, dw);
                 if (dw < 0.0) na = fmax(na, tau * sl / dw);
@@ -925,11 +963,11 @@ CPDP_D void newton_step_problem(const SolveArgs& a, const int b) {
             PdBuf pdb;
             const double* pd = pd_at(pd0, grid_time(a.T, N, k), pdb);
             for (int i = 0; i < NX; ++i) xk[i] = X[(size_t)k * NX + i] + alpha * dX[(size_t)k * NX + i];
-            if constexpr (HAS_BOUNDS) { NWT_UNROLL for (int i = 0; i < NX; ++i) lt += bnd_log(i, xk[i]); }
+            if constexpr (HAS_BOUNDS) { NWT_UNROLL for (int i = 0; i < NX; ++i) lt += bnd_log(i, pd0, xk[i]); }
             if (k < N) {
                 double uk[NU], xe[NX], q;
                 for (int i = 0; i < NU; ++i) uk[i] = U[(size_t)k * NU + i] + alpha * dU[(size_t)k * NU + i];
-                if constexpr (HAS_BOUNDS) { NWT_UNROLL for (int i = 0; i < NU; ++i) lt += bnd_log(NX + i, uk[i]); }
+                if constexpr (HAS_BOUNDS) { NWT_UNROLL for (int i = 0; i < NU; ++i) lt += bnd_log(NX + i, pd0, uk[i]); }
                 rk4_interval(xk, uk, th, pd, DT, a.S, xe, q);
                 Jt += q;
                 for (int i = 0; i < NX; ++i)
@@ -979,7 +1017,7 @@ CPDP_D void newton_step_problem(const SolveArgs& a, const int b) {
             const double w = (j < NX) ? X[(size_t)k * NX + j] : U[(size_t)k * NU + j - NX];
             const double dw = (j < NX) ? dX[(size_t)k * NX + j] : dU[(size_t)k * NU + j - NX];
             const double wn = w + alpha * dw;
-            const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+            const double lb = ModelBounds<Model>::lo(j, pd0), ub = ModelBounds<Model>::hi(j, pd0);
             if (bnd_finite(lb)) {
                 const double z = zL[idx] + az * bnd_dz(w - lb, zL[idx], mu, dw), sn = wn - lb;
                 zL[idx] = fmax(fmin(z, 1e10 * mu / sn), mu / (1e10 * sn));
@@ -1034,19 +1072,25 @@ CPDP_HD double bnd_push(double lb, double ub, bool fl, bool fu, double w, double
 // Cold seed of component j of z = [x; u] in a row where it is a variable (var; row N holds the final state only): the zero seed
 // (CPDP.py:139,155,167) pushed into the interior by bound_push = bound_frac = 1e-2, and z = 1 for every finite bound (0 else).
 // k_solve_init spells out the same three statements: routing its stores through this helper changes its generated code.
-CPDP_HD void cold_seed(int j, bool var, double& w, double& zl, double& zu) {
-    const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+CPDP_HD void cold_seed(int j, const double* pd, bool var, double& w, double& zl, double& zu) {
+    const double lb = ModelBounds<Model>::lo(j, pd), ub = ModelBounds<Model>::hi(j, pd);
     const bool fl = var && bnd_finite(lb), fu = var && bnd_finite(ub);
     w = bnd_push(lb, ub, fl, fu, 0.0, COLD_PUSH);
     zl = fl ? 1.0 : 0.0;
     zu = fu ? 1.0 : 0.0;
 }
 
-// x0 outside a finite state bound cannot be reached: status CPDP_INFEASIBLE (both starts).
+// x0 outside a finite state bound cannot be reached: status CPDP_INFEASIBLE (both starts).  Bounds that depend on the problem's
+// constants: also a component whose lb(pd) >= ub(pd) (or NaN), an empty box for that problem.
 CPDP_HD void check_x0(const SolveArgs& a, size_t i) {
+    const double* pd = pdata_of(a, (int)i);
     for (int j = 0; j < NX; ++j) {
-        const double v = a.x0[i * NX + j], lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+        const double v = a.x0[i * NX + j], lb = ModelBounds<Model>::lo(j, pd), ub = ModelBounds<Model>::hi(j, pd);
         if ((bnd_finite(lb) && !(v > lb)) || (bnd_finite(ub) && !(v < ub))) a.status[i] = ST_INFEASIBLE;
+    }
+    if constexpr (BOUNDS_PD) {
+        for (int j = 0; j < NZ; ++j)
+            if (!(ModelBounds<Model>::lo(j, pd) < ModelBounds<Model>::hi(j, pd))) a.status[i] = ST_INFEASIBLE;
     }
 }
 
@@ -1067,7 +1111,8 @@ CPDP_GLOBAL void k_solve_init(SolveArgs a) {
             const int j = (int)(i % NZ);
             const size_t k = i / NZ;
             const bool var = (k % (a.N + 1)) < (size_t)a.N || j < NX;           // (row N holds the final state only)
-            const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+            const double* pd = pdata_of(a, (int)(k / (a.N + 1)));
+            const double lb = ModelBounds<Model>::lo(j, pd), ub = ModelBounds<Model>::hi(j, pd);
             const bool fl = var && bnd_finite(lb), fu = var && bnd_finite(ub);
             const double w = bnd_push(lb, ub, fl, fu, 0.0, COLD_PUSH);
             if (j < NX) a.X[k * NX + j] = w; else a.U[k * NU + j - NX] = w;

@@ -36,11 +36,12 @@ constexpr double WARM_MULT_PUSH = 1e-3;   // IPOPT's warm_start_mult_bound_push
 constexpr int WARM_THREADS = 32;
 
 // Starting value of component j in row k for a warm-started problem (bounded models: pushed, z from the guess or mu_init / s).
-CPDP_D void warm_value(const WarmArgs& g, int j, bool var, double v, double zlg, double zug, double& w, double& zl, double& zu) {
+CPDP_D void warm_value(const WarmArgs& g, int j, const double* pd, bool var, double v, double zlg, double zug, double& w, double& zl,
+                       double& zu) {
     if constexpr (!HAS_BOUNDS) {
         w = v; zl = 0.0; zu = 0.0;
     } else {
-        const double lb = ModelBounds<Model>::lo(j), ub = ModelBounds<Model>::hi(j);
+        const double lb = ModelBounds<Model>::lo(j, pd), ub = ModelBounds<Model>::hi(j, pd);
         const bool fl = var && bnd_finite(lb), fu = var && bnd_finite(ub);
         w = bnd_push(lb, ub, fl, fu, v, WARM_PUSH);
         if (g.Zlg) { zl = fl ? fmax(zlg, WARM_MULT_PUSH) : 0.0; zu = fu ? fmax(zug, WARM_MULT_PUSH) : 0.0; }
@@ -54,6 +55,7 @@ CPDP_GLOBAL void __launch_bounds__(WARM_THREADS) k_solve_init_warm(SolveArgs a, 
     const bool cold = g.init_status && g.init_status[b] != ST_CONVERGED;
     NWT_SYNC();                                        // every lane has read init_status[b] before lane 0 writes status[b]
     const size_t rx = (size_t)b * (N + 1) * NX, ru = (size_t)b * (N + 1) * NU, rz = (size_t)b * (N + 1) * NZ;
+    const double* pd = pdata_of(a, b);
     for (int j = lane; j < NZ; j += WARM_THREADS) {
         const bool isx = j < NX;
         const int c = isx ? j : j - NX, nc = isx ? NX : NU;
@@ -67,12 +69,12 @@ CPDP_GLOBAL void __launch_bounds__(WARM_THREADS) k_solve_init_warm(SolveArgs a, 
             const int ks = (k + g.shift < last) ? k + g.shift : last;
             double lam = 0.0;
             if (cold) {
-                cold_seed(j, var, w, zl, zu);
+                cold_seed(j, pd, var, w, zl, zu);
             } else if (var) {
                 const double v = (isx && k == 0) ? a.x0[(size_t)b * NX + c] : src[r0 + (size_t)ks * nc + c];
                 const double zlg = g.Zlg ? g.Zlg[rz + (size_t)ks * NZ + j] : 0.0, zug = g.Zug ? g.Zug[rz + (size_t)ks * NZ + j] : 0.0;
                 if (isx) lam = g.Lg[rx + (size_t)ks * NX + c];
-                warm_value(g, j, true, v, zlg, zug, w, zl, zu);
+                warm_value(g, j, pd, true, v, zlg, zug, w, zl, zu);
             } else {
                 zl = 0.0; zu = 0.0;                    // U_N = U_{N-1}: w keeps row N-1's value
             }

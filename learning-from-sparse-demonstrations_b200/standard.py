@@ -201,6 +201,53 @@ def quadrotor_bounded_oc(n_grid=25):
 BOUNDED = {"pendulum_bounded": pendulum_bounded_oc, "robotarm_bounded": robotarm_bounded_oc,
            "quadrotor_bounded": quadrotor_bounded_oc}
 
+# ---- the same limits as expressions of per-problem constants (DESIGN.md §3.12): one library serves every limit value ------------
+def pendulum_pdbounded_oc(n_grid=10):
+    """pendulum_bounded_oc with the torque limit per problem, |u| <= umax (pdata = [umax])."""
+    oc = pendulum_oc(n_grid)
+    umax = SX.sym('umax')
+    oc.setProblemVariable(umax)
+    oc.setControlVariable(oc.env.U, [-umax], [umax])
+    oc.lib_name = "pendulum_pdbounded"
+    return oc
+
+
+def pendulum_pdbounded_ab_oc(n_grid=10):
+    """pendulum_bounded_oc with nonlinear limits of two constants (pdata = [a, b]): -a (1 + b^2) <= u <= a + b^2, i.e. |u| <= 5 at
+    a = 1, b = 2."""
+    oc = pendulum_oc(n_grid)
+    a, b = SX.sym('a'), SX.sym('b')
+    oc.setProblemVariable(vertcat(a, b))
+    oc.setControlVariable(oc.env.U, [-a * (1 + b ** 2)], [a + b ** 2])
+    oc.lib_name = "pendulum_pdbounded_ab"
+    return oc
+
+
+def robotarm_pdbounded_oc(n_grid=30):
+    """robotarm_bounded_oc with the joint-speed limit per problem, |dq2| <= vmax (pdata = [vmax]); |u_i| <= 3 stays constant."""
+    oc = robotarm_oc(n_grid)
+    vmax = SX.sym('vmax')
+    oc.setProblemVariable(vmax)
+    oc.setStateVariable(oc.env.X, [-1e20, -1e20, -1e20, -vmax], [1e20, 1e20, 1e20, vmax])
+    oc.setControlVariable(oc.env.U, [-3.0, -3.0], [3.0, 3.0])
+    oc.lib_name = "robotarm_pdbounded"
+    return oc
+
+
+def quadrotor_pdbounded_oc(n_grid=25):
+    """quadrotor_bounded_oc with the thrust limit per problem, 1 <= f_i <= f_max (pdata = [goal position (3), f_max])."""
+    oc = quadrotor_oc(n_grid)
+    fmax = SX.sym('f_max')
+    oc.setProblemVariable(vertcat(oc.pvar, fmax))
+    oc.setControlVariable(oc.env.U, [1.0] * 4, [fmax] * 4)
+    oc.lib_name = "quadrotor_pdbounded"
+    return oc
+
+
+# not part of build_all: built on first use
+PD_BOUNDED = {"pendulum_pdbounded": pendulum_pdbounded_oc, "pendulum_pdbounded_ab": pendulum_pdbounded_ab_oc,
+              "robotarm_pdbounded": robotarm_pdbounded_oc, "quadrotor_pdbounded": quadrotor_pdbounded_oc}
+
 STANDARD = {"pendulum": pendulum_oc, "pendulum_tw2": pendulum_timewarp_oc, "robotarm": robotarm_oc, "rocket": rocket_oc, "quadrotor": quadrotor_oc,
             "cartpole": cartpole_oc}
 
